@@ -1,11 +1,18 @@
-"""Writes one translation unit per register-tiled solver instantiation plus the dispatch table.
+"""Writes one translation unit per register-tiled solver variant plus the dispatch table.
 
-    python gen_fast_instances.py        (run from pybold_b200/csrc; outputs are committed)
+    python gen_fast_instances.py OUTDIR        (the Makefile runs it with OUTDIR = build/gen)
 
-Each row: (real, R, KMAX, CIRC).  R = samples per lane (32 R >= T), KMAX = unrolled tap count
+Each unit defines one Variant (pb_fast_registry.h) from its family's factory; pb_fast_table.inc
+lists them per dtype for pb_fast_registry.cu.  Nothing it writes is committed: the lists below are
+the record of the variants and of why each exists.  Files whose content is unchanged are left alone,
+so that editing one row recompiles that unit and the table only.  Prints the units' paths.
+
+Warp rows: (real, R, KMAX, CIRC, ...).  R = samples per lane (32 R >= T), KMAX = unrolled tap count
 (>= K), CIRC = wrap-around variant (T % R == 0 and idle lanes >= halo, see pb_fast.cuh).
-The table is searched in order, so cheaper variants come first.
 """
+import os
+import sys
+
 VARIANTS = [
     # (real, R, KMAX, CIRC, warps per CTA, min CTAs per SM) -- launch bounds picked by the sweep
     # in tools/exp_bd.cu on a B200 (profiles/r01_launch_bounds_sweep.txt)
@@ -112,118 +119,51 @@ CVARIANTS = [
 ]
 
 
-def ctag(real, R, K, NW):
-    return "%s_r%d_k%d_w%d" % ("f32" if real == "float" else "f64", R, K, NW)
+DTYPE = {"float": "f32", "double": "f64"}
 
 
-def gtag(real, R, K, G, tail):
-    return "%s_r%d_k%d_g%d_t%d" % ("f32" if real == "float" else "f64", R, K, G, tail)
-
-
-def tag(real, R, K, circ):
-    return "%s_r%d_k%d_%s" % ("f32" if real == "float" else "f64", R, K, "circ" if circ else "lin")
-
-
-def main():
-    rows = []
-    for real, R, K, circ, W, M in VARIANTS:
-        t = tag(real, R, K, circ)
-        c = "true" if circ else "false"
-        with open("pb_fast_inst_%s.cu" % t, "w") as f:
-            f.write('// GENERATED by gen_fast_instances.py -- do not edit.\n')
-            f.write('#include "pb_fast.cuh"\n\nnamespace pb {\n')
-            f.write('bool fast_ok_%s(int T, int K) { return fast_shape_ok<%s, %d, %d, %s>(T, K); }\n'
-                    % (t, real, R, K, c))
-            f.write('int fast_deconv_%s(const DeconvArgs<%s> &a, cudaStream_t s) {\n'
-                    '    return fast_deconv_launch<%s, %d, %d, %s, %d, %d>(a, s);\n}\n' % (t, real, real, R, K, c, W, M))
-            f.write('int fast_bd_%s(const BdArgs<%s> &a, cudaStream_t s) {\n'
-                    '    return fast_bd_launch<%s, %d, %d, %s, %d, %d>(a, s);\n}\n' % (t, real, real, R, K, c, W, M))
-            f.write('}  // namespace pb\n')
-        rows.append((real, R, K, circ, t))
-    grows = []
-    for real, R, K, G, tail, W, M in GVARIANTS:
-        t = gtag(real, R, K, G, tail)
-        with open("pb_fast_inst_%s.cu" % t, "w") as f:
-            f.write('// GENERATED by gen_fast_instances.py -- do not edit.\n')
-            f.write('#include "pb_fastg.cuh"\n\nnamespace pb {\n')
-            f.write('bool fastg_ok_%s(int T, int K) { return fastg_shape_ok<%d, %d, %d, %d>(T, K); }\n'
-                    % (t, R, K, G, tail))
-            f.write('int fastg_bd_%s(const BdArgs<%s> &a, cudaStream_t s) {\n'
-                    '    return fast_bdg_launch<%s, %d, %d, %d, %d, %d, %d>(a, s);\n}\n'
-                    % (t, real, real, R, K, G, tail, W, M))
-            f.write('int fastg_deconv_%s(const DeconvArgs<%s> &a, cudaStream_t s) {\n'
-                    '    return fast_deconvg_launch<%s, %d, %d, %d, %d, %d, %d>(a, s);\n}\n'
-                    % (t, real, real, R, K, G, tail, W, M))
-            f.write('int fastg_wave_%s(int nb_iter) { return fast_bdg_wave<%s, %d, %d, %d, %d, %d, %d>(nb_iter); }\n'
-                    % (t, real, R, K, G, tail, W, M))
-            f.write('int fastg_bd_es_%s(const BdArgs<%s> &a, cudaStream_t s) {\n'
-                    '    return fast_bdg_launch<%s, %d, %d, %d, %d, %d, %d, 0, 0, true>(a, s);\n}\n'
-                    % (t, real, real, R, K, G, tail, W, M))
-            f.write('}  // namespace pb\n')
-        grows.append((real, R, K, G, tail, t))
-    crows = []
+def rows():
+    """(real, tag, family header, factory call) per variant, in the order the dispatcher searches them:
+    CTA rows, then group rows, then warp rows (ties go to the first row)."""
     for real, R, K, NW, M in CVARIANTS:
-        t = ctag(real, R, K, NW)
-        with open("pb_fast_inst_%s.cu" % t, "w") as f:
-            f.write('// GENERATED by gen_fast_instances.py -- do not edit.\n')
-            f.write('#include "pb_fastc.cuh"\n\nnamespace pb {\n')
-            f.write('bool fastc_ok_%s(int T, int K) { return fastc_shape_ok<%d, %d, %d>(T, K); }\n' % (t, R, K, NW))
-            f.write('int fastc_bd_%s(const BdArgs<%s> &a, cudaStream_t s) {\n'
-                    '    return fast_bdc_launch<%s, %d, %d, %d, %d>(a, s);\n}\n' % (t, real, real, R, K, NW, M))
-            f.write('int fastc_wave_%s(int nb_iter) { return fast_bdc_wave<%s, %d, %d, %d, %d>(nb_iter); }\n'
-                    % (t, real, R, K, NW, M))
-            f.write('}  // namespace pb\n')
-        crows.append((real, R, K, NW, t))
-    with open("pb_fast_table.inc", "w") as f:
-        f.write('// GENERATED by gen_fast_instances.py -- do not edit.\n')
-        for real, R, K, NW, t in crows:
-            f.write('bool fastc_ok_%s(int, int);\n' % t)
-            f.write('int fastc_bd_%s(const BdArgs<%s> &, cudaStream_t);\n' % (t, real))
-            f.write('int fastc_wave_%s(int);\n' % t)
-        for real in ("float", "double"):
-            f.write('template <> const FastGEntry<%s> *fastc_table<%s>(int *n) {\n' % (real, real))
-            f.write('    static const FastGEntry<%s> table[] = {\n' % real)
-            cnt = 0
-            for r2, R, K, NW, t in crows:
-                if r2 != real:
-                    continue
-                f.write('        {%d, %d, %d, 0, fastc_ok_%s, fastc_bd_%s, fastc_wave_%s, nullptr, nullptr},\n' % (R, K, 32 * NW, t, t, t))
-                cnt += 1
-            f.write('        {0, 0, 0, 0, nullptr, nullptr, nullptr, nullptr, nullptr},\n')
-            f.write('    };\n    *n = %d;\n    return table;\n}\n' % cnt)
-        for real, R, K, G, tail, t in grows:
-            f.write('bool fastg_ok_%s(int, int);\n' % t)
-            f.write('int fastg_bd_%s(const BdArgs<%s> &, cudaStream_t);\n' % (t, real))
-            f.write('int fastg_wave_%s(int);\n' % t)
-            f.write('int fastg_deconv_%s(const DeconvArgs<%s> &, cudaStream_t);\n' % (t, real))
-            f.write('int fastg_bd_es_%s(const BdArgs<%s> &, cudaStream_t);\n' % (t, real))
-        for real in ("float", "double"):
-            f.write('template <> const FastGEntry<%s> *fastg_table<%s>(int *n) {\n' % (real, real))
-            f.write('    static const FastGEntry<%s> table[] = {\n' % real)
-            cnt = 0
-            for r2, R, K, G, tail, t in grows:
-                if r2 != real:
-                    continue
-                f.write('        {%d, %d, %d, %d, fastg_ok_%s, fastg_bd_%s, fastg_wave_%s, fastg_deconv_%s, fastg_bd_es_%s},\n' % (R, K, G, tail, t, t, t, t, t))
-                cnt += 1
-            f.write('        {0, 0, 0, 0, nullptr, nullptr, nullptr, nullptr},\n')
-            f.write('    };\n    *n = %d;\n    return table;\n}\n' % cnt)
-        for real, R, K, circ, t in rows:
-            f.write('bool fast_ok_%s(int, int);\n' % t)
-            f.write('int fast_deconv_%s(const DeconvArgs<%s> &, cudaStream_t);\n' % (t, real))
-            f.write('int fast_bd_%s(const BdArgs<%s> &, cudaStream_t);\n' % (t, real))
-        for real in ("float", "double"):
-            f.write('template <> const FastEntry<%s> *fast_table<%s>(int *n) {\n' % (real, real))
-            f.write('    static const FastEntry<%s> table[] = {\n' % real)
-            cnt = 0
-            for r2, R, K, circ, t in rows:
-                if r2 != real:
-                    continue
-                f.write('        {%d, %d, %s, fast_ok_%s, fast_deconv_%s, fast_bd_%s},\n'
-                        % (R, K, "true" if circ else "false", t, t, t))
-                cnt += 1
-            f.write('    };\n    *n = %d;\n    return table;\n}\n' % cnt)
+        yield (real, "%s_r%d_k%d_w%d" % (DTYPE[real], R, K, NW), "pb_fastc.cuh",
+               "cta_variant<%s, %d, %d, %d, %d>" % (real, R, K, NW, M))
+    for real, R, K, G, tail, W, M in GVARIANTS:
+        yield (real, "%s_r%d_k%d_g%d_t%d" % (DTYPE[real], R, K, G, tail), "pb_fastg.cuh",
+               "group_variant<%s, %d, %d, %d, %d, %d, %d>" % (real, R, K, G, tail, W, M))
+    for real, R, K, circ, W, M in VARIANTS:
+        yield (real, "%s_r%d_k%d_%s" % (DTYPE[real], R, K, "circ" if circ else "lin"), "pb_fast.cuh",
+               "warp_variant<%s, %d, %d, %s, %d, %d>" % (real, R, K, "true" if circ else "false", W, M))
+
+
+def write(path, text):
+    """Writes text unless the file already holds it, so that make recompiles only what changed."""
+    if os.path.exists(path):
+        with open(path) as f:
+            if f.read() == text:
+                return
+    with open(path, "w") as f:
+        f.write(text)
+
+
+HEAD = "// GENERATED by gen_fast_instances.py -- do not edit.\n"
+
+
+def main(out):
+    os.makedirs(out, exist_ok=True)
+    decls, table, srcs = [], {real: [] for real in DTYPE}, []
+    for real, tag, header, factory in rows():
+        src = os.path.join(out, "pb_fast_inst_%s.cu" % tag)
+        write(src, HEAD + '#include "%s"\n\nnamespace pb {\nextern const Variant<%s> variant_%s = %s();\n}\n'
+              % (header, real, tag, factory))
+        srcs.append(src)
+        decls.append("extern const Variant<%s> variant_%s;\n" % (real, tag))
+        table[real].append("    &variant_%s,\n" % tag)
+    arrays = ["static const Variant<%s> *const variants_%s[] = {\n%s};\n" % (real, DTYPE[real], "".join(table[real]))
+              for real in DTYPE]
+    write(os.path.join(out, "pb_fast_table.inc"), HEAD + "".join(decls) + "".join(arrays))
+    print(" ".join(srcs))
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1])

@@ -415,7 +415,8 @@ int run_bd(pb::BdArgs<real> a, double t_r, double hrf_dur, pb_stream_t stream) {
     if (a.T > PB_MAX_T || a.K > PB_MAX_K || a.nb_iter > PB_MAX_ITER) return PB_ERR_UNSUPPORTED;
     if (a.V == 0) return PB_OK;
     // group / CTA kernels pull their tasks from it (static stride if null; PB_NO_QUEUE=1: developer A/B switch)
-    a.queue = getenv("PB_NO_QUEUE") ? nullptr : queue_slot();
+    static const bool no_queue = getenv("PB_NO_QUEUE") != nullptr;
+    a.queue = no_queue ? nullptr : queue_slot();
     int rc = pb::fast_bd_dispatch(a, (cudaStream_t)stream);
     if (rc != pb::FAST_NO_MATCH) return rc;
     DeviceInfo d = device_info();

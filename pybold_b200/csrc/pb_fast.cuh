@@ -510,7 +510,7 @@ fast_bd_kernel(BdArgs<real> p) {
 }
 
 // ------------------------------------------------------------------------------------------------
-// host-side launchers (one instantiation per translation unit, see pb_fast_inst_*.cu)
+// host-side launchers (one variant per translation unit, see gen_fast_instances.py)
 // ------------------------------------------------------------------------------------------------
 template <typename real, int R, int KMAX, bool CIRC>
 bool fast_shape_ok(int T, int K) {
@@ -519,55 +519,30 @@ bool fast_shape_ok(int T, int K) {
     return true;
 }
 
-template <typename Kern>
-int fast_launch(Kern kern, size_t smem, int warps, int64_t V, cudaStream_t stream,
-                int *grid_out) {
-    int dev = 0, sms = 0, max_smem = 0;
-    cudaError_t e = cudaGetDevice(&dev);
-    if (e != cudaSuccess) return (int)e;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-    if (smem > (size_t)max_smem) return -2;
-    e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return (int)e;
-    int occ = 0;
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, warps * 32, smem);
-    if (e != cudaSuccess) return (int)e;
-    if (occ < 1) return -2;
-    int64_t need = (V + warps - 1) / warps;
-    int64_t cap = (int64_t)sms * occ;
-    *grid_out = (int)(need < cap ? need : cap);
-    return 0;
-}
-
+// FAST_NO_MATCH when the ring does not fit: the generic kernel decides
 template <typename real, int R, int KMAX, bool CIRC, int WARPS, int MINB>
 int fast_deconv_launch(const DeconvArgs<real> &a, cudaStream_t stream) {
     const bool es = a.early_stopping && a.wind >= 2;
     const int ring_rows = es ? a.wind - 1 : 0;
     const size_t beta_bytes = ((size_t)a.nb_iter * sizeof(real) + 15) & ~(size_t)15;
     const size_t smem = beta_bytes + (size_t)WARPS * ring_rows * R * 32 * sizeof(real);
-    auto kern = fast_deconv_kernel<real, R, KMAX, CIRC, WARPS, MINB>;
-    int grid = 0;
-    int rc = fast_launch(kern, smem, WARPS, a.V, stream, &grid);
-    if (rc == -2) return FAST_NO_MATCH;   // ring does not fit: let the generic kernel decide
-    if (rc) return rc;
-    kern<<<grid, WARPS * 32, smem, stream>>>(a, ring_rows);
-    cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? 0 : (int)e;
+    return launch_persistent(fast_deconv_kernel<real, R, KMAX, CIRC, WARPS, MINB>, WARPS * 32, smem, WARPS,
+                             a.V, nullptr, stream, a, ring_rows);
 }
 
 template <typename real, int R, int KMAX, bool CIRC, int WARPS, int MINB>
 int fast_bd_launch(const BdArgs<real> &a, cudaStream_t stream) {
     const size_t beta_bytes = ((size_t)a.nb_iter * sizeof(real) + 15) & ~(size_t)15;
     const size_t smem = beta_bytes + (size_t)WARPS * pb_scratch_doubles(KMAX) * sizeof(double);
-    auto kern = fast_bd_kernel<real, R, KMAX, CIRC, WARPS, MINB>;
-    int grid = 0;
-    int rc = fast_launch(kern, smem, WARPS, a.V, stream, &grid);
-    if (rc == -2) return FAST_NO_MATCH;
-    if (rc) return rc;
-    kern<<<grid, WARPS * 32, smem, stream>>>(a);
-    cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? 0 : (int)e;
+    return launch_persistent(fast_bd_kernel<real, R, KMAX, CIRC, WARPS, MINB>, WARPS * 32, smem, WARPS, a.V,
+                             nullptr, stream, a);
+}
+
+template <typename real, int R, int KMAX, bool CIRC, int WARPS, int MINB>
+constexpr Variant<real> warp_variant() {
+    return {TIER_WARP, 32, R, KMAX, 0, CIRC, fast_shape_ok<real, R, KMAX, CIRC>,
+            fast_bd_launch<real, R, KMAX, CIRC, WARPS, MINB>, nullptr,
+            fast_deconv_launch<real, R, KMAX, CIRC, WARPS, MINB>, nullptr};
 }
 
 }  // namespace pb

@@ -1,119 +1,93 @@
-// Dispatch over the register-tiled instantiations listed in pb_fast_table.inc.
+// Dispatch over the register-tiled variants listed in the generated pb_fast_table.inc.
 #include <cstdlib>
 
 #include "pb_fast_registry.h"
 
 namespace pb {
 
-template <typename real>
-struct FastEntry {
-    int R, KMAX;
-    bool circ;
-    bool (*ok)(int T, int K);
-    int (*deconv)(const DeconvArgs<real> &, cudaStream_t);
-    int (*bd)(const BdArgs<real> &, cudaStream_t);
-};
-
-template <typename real>
-const FastEntry<real> *fast_table(int *n);
-
-// group variants (pb_fastg.cuh): several voxels per warp, bd without early stopping only
-template <typename real>
-struct FastGEntry {
-    int R, KMAX, G, TAIL;
-    bool (*ok)(int T, int K);
-    int (*bd)(const BdArgs<real> &, cudaStream_t);
-    int (*wave)(int nb_iter);
-    int (*deconv)(const DeconvArgs<real> &, cudaStream_t);   // null for CTA variants
-    int (*bd_es)(const BdArgs<real> &, cudaStream_t);        // bd with early stopping (Q6 / Q7); null for CTA variants
-};
-
-template <typename real>
-const FastGEntry<real> *fastg_table(int *n);
-// CTA variants (pb_fastc.cuh): NW warps per voxel; same entry type, G = 32 * NW
-template <typename real>
-const FastGEntry<real> *fastc_table(int *n);
-
+// variants_f32[], variants_f64[]: CTA rows, then group rows, then warp rows
 #include "pb_fast_table.inc"
 
+static const auto &variants(float) { return variants_f32; }
+static const auto &variants(double) { return variants_f64; }
+
 template <typename real>
-static const FastEntry<real> *pick(int T, int K) {
-    int n = 0;
-    const FastEntry<real> *t = fast_table<real>(&n);
-    // cheapest matching variant: unrolled work per iteration ~ R * KMAX (the CIRC variants skip
-    // the halo / tail selects, hence the small bonus)
-    const FastEntry<real> *best = nullptr;
-    int best_cost = 0;
-    for (int i = 0; i < n; ++i) {
-        if (!t[i].ok(T, K)) continue;
-        const int cost = t[i].R * t[i].KMAX * (t[i].circ ? 19 : 20);
-        if (!best || cost < best_cost) {
-            best = &t[i];
-            best_cost = cost;
-        }
-    }
-    return best;
+static long cost(const Variant<real> &v) {
+    // warp tier: unrolled work per iteration ~ R * KMAX (the CIRC variants skip the halo / tail selects,
+    // hence the small bonus)
+    if (v.tier == TIER_WARP) return (long)v.R * v.KMAX * (v.circ ? 19 : 20);
+    // tier 0: slots per voxel (lanes x samples per lane) x unrolled taps, ties broken by the tail-select count
+    long c = (long)v.R * v.KMAX * v.lanes * 64 + v.TAIL;
+    // one warp per voxel with 64 taps runs four warps per SM (shared-memory scratch), two warps per
+    // voxel run eight: prefer the latter up to 1.3 x the slots (measured: T = 405..512 2.5 x faster on two
+    // warps of R = 8 than on one of R = 16; T = 300 5 % slower than on one warp of R = 12)
+    if (v.KMAX == 64 && v.lanes == 32) c += c * 3 / 10;
+    return c;
 }
 
-// cheapest matching group / CTA variant: slots per voxel (lanes x samples per lane) x unrolled taps,
-// ties broken by the tail-select count
-template <typename real>
-static const FastGEntry<real> *pick_group(int T, int K, bool es = false) {
-    const FastGEntry<real> *best = nullptr;
+// cheapest variant of `tier` that serves (T, K) and has the entry point `need`; ties go to the first
+// row (strict <), so CTA rows win ties against group rows
+template <typename real, typename Fn>
+static const Variant<real> *pick(int tier, int T, int K, Fn Variant<real>::*need) {
+    const Variant<real> *best = nullptr;
     long best_cost = 0;
-    for (int which = 0; which < 2; ++which) {
-        int n = 0;
-        const FastGEntry<real> *t = which == 0 ? fastc_table<real>(&n) : fastg_table<real>(&n);
-        for (int i = 0; i < n; ++i) {
-            if (!t[i].ok(T, K) || (es && !t[i].bd_es)) continue;
-            long cost = (long)t[i].R * t[i].KMAX * t[i].G * 64 + t[i].TAIL;
-            // one warp per voxel with 64 taps runs four warps per SM (shared-memory scratch), two warps per
-            // voxel run eight: prefer the latter up to 1.3 x the slots (measured: T = 405..512 2.5 x faster on two
-            // warps of R = 8 than on one of R = 16; T = 300 5 % slower than on one warp of R = 12)
-            if (t[i].KMAX == 64 && t[i].G == 32) cost += cost * 3 / 10;
-            if (!best || cost < best_cost) {
-                best = &t[i];
-                best_cost = cost;
-            }
+    for (const Variant<real> *v : variants(real())) {
+        if (v->tier != tier || !(v->*need) || !v->ok(T, K)) continue;
+        const long c = cost(*v);
+        if (!best || c < best_cost) {
+            best = v;
+            best_cost = c;
         }
     }
     return best;
 }
 
+// PB_DISABLE_GROUP=1: developer switch for A/B timing of tier 0 against the warp-per-voxel kernels
+static bool tier0_disabled() {
+    static const bool disabled = getenv("PB_DISABLE_GROUP") != nullptr;
+    return disabled;
+}
+
+// The warp tier runs only when the one tier-0 candidate returns FAST_NO_MATCH (its shared memory
+// does not fit); no second tier-0 candidate is tried.
 template <typename real>
 static int bd_dispatch(const BdArgs<real> &a, cudaStream_t s) {
-    // PB_DISABLE_GROUP=1: developer switch for A/B timing of the two register-tiled kernels
-    static const bool no_group = getenv("PB_DISABLE_GROUP") != nullptr;
-    if (!no_group) {
-        const FastGEntry<real> *ge = pick_group<real>(a.T, a.K, a.early_stopping != 0);
-        if (ge) {
-            const int rc = a.early_stopping ? ge->bd_es(a, s) : ge->bd(a, s);
+    // early stopping: only the rows with bd_es (the group variants) are candidates
+    const auto need = a.early_stopping ? &Variant<real>::bd_es : &Variant<real>::bd;
+    if (!tier0_disabled())
+        if (const Variant<real> *v = pick<real>(TIER_GROUP_CTA, a.T, a.K, need)) {
+            const int rc = (v->*need)(a, s);
             if (rc != FAST_NO_MATCH) return rc;
         }
-    }
-    const FastEntry<real> *e = pick<real>(a.T, a.K);
-    return e ? e->bd(a, s) : FAST_NO_MATCH;
+    const Variant<real> *v = pick<real>(TIER_WARP, a.T, a.K, &Variant<real>::bd);
+    return v ? v->bd(a, s) : FAST_NO_MATCH;
 }
 
 template <typename real>
 static int deconv_dispatch(const DeconvArgs<real> &a, cudaStream_t s) {
-    static const bool no_group = getenv("PB_DISABLE_GROUP") != nullptr;
-    // early stopping runs on the group layout too when a work-queue counter was provided (a.queue)
-    if ((!(a.early_stopping && a.wind >= 2) || a.queue) && !no_group) {
-        int n = 0;
-        const FastGEntry<real> *t = fastg_table<real>(&n);
-        const FastGEntry<real> *best = nullptr;
-        for (int i = 0; i < n; ++i)
-            if (t[i].deconv && t[i].ok(a.T, a.K) &&
-                (!best || t[i].R * t[i].KMAX * t[i].G * 64 + t[i].TAIL < best->R * best->KMAX * best->G * 64 + best->TAIL))
-                best = &t[i];
-        if (best) {
-            const int rc = best->deconv(a, s);
+    // tier 0 is the group rows only (the CTA rows have no deconv); early stopping runs there only when a
+    // work-queue counter was provided (a.queue)
+    if ((!(a.early_stopping && a.wind >= 2) || a.queue) && !tier0_disabled())
+        if (const Variant<real> *v = pick<real>(TIER_GROUP_CTA, a.T, a.K, &Variant<real>::deconv)) {
+            const int rc = v->deconv(a, s);
             if (rc != FAST_NO_MATCH) return rc;
         }
-    }
-    const FastEntry<real> *e = pick<real>(a.T, a.K);
-    return e ? e->deconv(a, s) : FAST_NO_MATCH;
+    const Variant<real> *v = pick<real>(TIER_WARP, a.T, a.K, &Variant<real>::deconv);
+    return v ? v->deconv(a, s) : FAST_NO_MATCH;
+}
+
+// the queries describe bd without early stopping and ignore PB_DISABLE_GROUP
+template <typename real>
+static int variant_id(int T, int K) {
+    const Variant<real> *v = pick<real>(TIER_GROUP_CTA, T, K, &Variant<real>::bd);
+    if (!v) v = pick<real>(TIER_WARP, T, K, &Variant<real>::bd);
+    return v ? v->lanes * 1000000 + v->R * 1000 + v->KMAX : 0;
+}
+
+template <typename real>
+static int bd_wave_voxels(int T, int K, int nb_iter) {
+    const Variant<real> *v = pick<real>(TIER_GROUP_CTA, T, K, &Variant<real>::wave);
+    return v ? v->wave(nb_iter) : 0;
 }
 
 int fast_deconv_dispatch(const DeconvArgs<float> &a, cudaStream_t s) { return deconv_dispatch<float>(a, s); }
@@ -122,25 +96,11 @@ int fast_bd_dispatch(const BdArgs<float> &a, cudaStream_t s) { return bd_dispatc
 int fast_bd_dispatch(const BdArgs<double> &a, cudaStream_t s) { return bd_dispatch<double>(a, s); }
 
 int fast_bd_wave_voxels(int T, int K, bool is_f64, int nb_iter) {
-    if (is_f64) {
-        const FastGEntry<double> *g = pick_group<double>(T, K);
-        return g ? g->wave(nb_iter) : 0;
-    }
-    const FastGEntry<float> *g = pick_group<float>(T, K);
-    return g ? g->wave(nb_iter) : 0;
+    return is_f64 ? bd_wave_voxels<double>(T, K, nb_iter) : bd_wave_voxels<float>(T, K, nb_iter);
 }
 
-// id of the kernel a bd call without early stopping uses: G * 1000000 + R * 1000 + KMAX (G = lanes
-// per voxel), 0 = generic kernel
 int fast_variant_id(int T, int K, bool is_f64) {
-    if (is_f64) {
-        if (const FastGEntry<double> *g = pick_group<double>(T, K)) return g->G * 1000000 + g->R * 1000 + g->KMAX;
-        const FastEntry<double> *e = pick<double>(T, K);
-        return e ? 32 * 1000000 + e->R * 1000 + e->KMAX : 0;
-    }
-    if (const FastGEntry<float> *g = pick_group<float>(T, K)) return g->G * 1000000 + g->R * 1000 + g->KMAX;
-    const FastEntry<float> *e = pick<float>(T, K);
-    return e ? 32 * 1000000 + e->R * 1000 + e->KMAX : 0;
+    return is_f64 ? variant_id<double>(T, K) : variant_id<float>(T, K);
 }
 
 }  // namespace pb

@@ -1,6 +1,7 @@
-// Dispatch table of the register-tiled warp solver instantiations (pb_fast.cuh).  Each
-// instantiation lives in its own translation unit (pb_fast_inst_*.cu) so that they compile in
-// parallel; pb_fast_registry.cu picks one from (T, K, dtype).
+// Register-tiled solver variants (pb_fast.cuh, pb_fastg.cuh, pb_fastc.cuh) and their dispatch.
+// gen_fast_instances.py writes one translation unit per variant into build/gen/ at build time, so
+// that they compile in parallel, each defining one Variant, plus the table pb_fast_registry.cu
+// picks from by (T, K, dtype).
 #pragma once
 #include <cuda_runtime.h>
 
@@ -14,10 +15,72 @@ int fast_deconv_dispatch(const DeconvArgs<float> &a, cudaStream_t stream);
 int fast_deconv_dispatch(const DeconvArgs<double> &a, cudaStream_t stream);
 int fast_bd_dispatch(const BdArgs<float> &a, cudaStream_t stream);
 int fast_bd_dispatch(const BdArgs<double> &a, cudaStream_t stream);
-// 0 = generic kernel, else R * 1000 + KMAX
+// 0 = generic kernel, else lanes per voxel * 1000000 + R * 1000 + KMAX
 int fast_variant_id(int T, int K, bool is_f64);
 // voxels per full wave of the persistent bd grid (0 when unknown): batch sizes that are multiples
 // of it waste no tail
 int fast_bd_wave_voxels(int T, int K, bool is_f64, int nb_iter);
+
+// A call runs the cheapest matching variant of tier 0 (group and CTA variants) and falls back to
+// the cheapest warp-per-voxel variant only when that launch returns FAST_NO_MATCH.
+enum VariantTier { TIER_GROUP_CTA = 0, TIER_WARP = 1 };
+
+template <typename real>
+struct Variant {
+    int tier;
+    int lanes;          // lanes per voxel: G (group), 32 NW (CTA), 32 (warp)
+    int R, KMAX, TAIL;  // samples per lane, unrolled taps, maskable tail slots (group)
+    bool circ;          // wrap-around warp variant
+    // entry points; null: the variant has none
+    bool (*ok)(int T, int K);
+    int (*bd)(const BdArgs<real> &, cudaStream_t);
+    int (*bd_es)(const BdArgs<real> &, cudaStream_t);  // bd with early stopping (Q6 / Q7)
+    int (*deconv)(const DeconvArgs<real> &, cudaStream_t);
+    int (*wave)(int nb_iter);
+};
+
+// Launches a persistent kernel of `threads` threads and `smem` bytes of dynamic shared memory per
+// CTA: as many CTAs as fit on the device at once, at most one per `voxels_per_cta` voxels.  Returns
+// FAST_NO_MATCH when the kernel does not fit (shared memory beyond the opt-in limit, or no resident
+// CTA), else 0 or the CUDA error.  A work-queue counter, when given, is zeroed on the stream first.
+template <typename Kern, typename... Args>
+int launch_persistent(Kern kern, int threads, size_t smem, int voxels_per_cta, int64_t V,
+                      unsigned int *queue, cudaStream_t stream, const Args &...args) {
+    int dev = 0, sms = 0, max_smem = 0, occ = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess) return (int)e;
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+    if (smem > (size_t)max_smem) return FAST_NO_MATCH;
+    e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return (int)e;
+    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, threads, smem);
+    if (e != cudaSuccess) return (int)e;
+    if (occ < 1) return FAST_NO_MATCH;
+    if (queue) {
+        e = cudaMemsetAsync(queue, 0, sizeof(unsigned int), stream);
+        if (e != cudaSuccess) return (int)e;
+    }
+    const int64_t need = (V + voxels_per_cta - 1) / voxels_per_cta;
+    const int64_t cap = (int64_t)sms * occ;
+    kern<<<(int)(need < cap ? need : cap), threads, smem, stream>>>(args...);
+    e = cudaGetLastError();
+    return e == cudaSuccess ? 0 : (int)e;
+}
+
+// voxels one full wave of the persistent grid holds (SMs x resident CTAs x voxels per CTA); 0 on
+// any failure, with the error cleared
+template <typename Kern>
+int wave_voxels(Kern kern, int threads, size_t smem, int voxels_per_cta) {
+    int dev = 0, sms = 0, occ = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess ||
+        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess ||
+        cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess ||
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, threads, smem) != cudaSuccess) {
+        cudaGetLastError();
+        return 0;
+    }
+    return sms * occ * voxels_per_cta;
+}
 
 }  // namespace pb

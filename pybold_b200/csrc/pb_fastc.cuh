@@ -427,45 +427,20 @@ bool fastc_shape_ok(int T, int K) {
 template <typename real, int R, int KMAX, int NW, int MINB>
 int fast_bdc_launch(const BdArgs<real> &a, cudaStream_t stream) {
     using L = CtaLayout<real, R, KMAX, NW>;
-    const size_t smem = L::bytes(a.nb_iter);
-    auto kern = fast_bdc_kernel<real, R, KMAX, NW, MINB>;
-    int dev = 0, sms = 0, max_smem = 0;
-    cudaError_t e = cudaGetDevice(&dev);
-    if (e != cudaSuccess) return (int)e;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-    if (smem > (size_t)max_smem) return FAST_NO_MATCH;
-    e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return (int)e;
-    int occ = 0;
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, NW * 32, smem);
-    if (e != cudaSuccess) return (int)e;
-    if (occ < 1) return FAST_NO_MATCH;
-    const int64_t cap = (int64_t)sms * occ;
-    const int grid = (int)(a.V < cap ? a.V : cap);
-    if (a.queue) {
-        e = cudaMemsetAsync(a.queue, 0, sizeof(unsigned int), stream);
-        if (e != cudaSuccess) return (int)e;
-    }
-    kern<<<grid, NW * 32, smem, stream>>>(a);
-    e = cudaGetLastError();
-    return e == cudaSuccess ? 0 : (int)e;
+    return launch_persistent(fast_bdc_kernel<real, R, KMAX, NW, MINB>, NW * 32, L::bytes(a.nb_iter), 1, a.V,
+                             a.queue, stream, a);
 }
 
 template <typename real, int R, int KMAX, int NW, int MINB>
 int fast_bdc_wave(int nb_iter) {
     using L = CtaLayout<real, R, KMAX, NW>;
-    int dev = 0, sms = 0, occ = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) return 0;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    auto kern = fast_bdc_kernel<real, R, KMAX, NW, MINB>;
-    const size_t smem = L::bytes(nb_iter);
-    if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess ||
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, NW * 32, smem) != cudaSuccess) {
-        cudaGetLastError();
-        return 0;
-    }
-    return sms * occ;
+    return wave_voxels(fast_bdc_kernel<real, R, KMAX, NW, MINB>, NW * 32, L::bytes(nb_iter), 1);
+}
+
+template <typename real, int R, int KMAX, int NW, int MINB>
+constexpr Variant<real> cta_variant() {
+    return {TIER_GROUP_CTA, 32 * NW, R, KMAX, 0, false, fastc_shape_ok<R, KMAX, NW>,
+            fast_bdc_launch<real, R, KMAX, NW, MINB>, nullptr, nullptr, fast_bdc_wave<real, R, KMAX, NW, MINB>};
 }
 
 }  // namespace pb

@@ -749,30 +749,13 @@ fast_bdg_kernel(BdArgs<real> p) {
     }
 }
 
-// voxels one full wave of the persistent grid holds (SMs x resident CTAs x voxels per CTA)
-template <typename Kern>
-int fast_wave_voxels(Kern kern, int threads, size_t smem, int voxels_per_cta) {
-    int dev = 0, sms = 0, occ = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) return 0;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
-        cudaGetLastError();
-        return 0;
-    }
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, threads, smem) != cudaSuccess) {
-        cudaGetLastError();
-        return 0;
-    }
-    return sms * occ * voxels_per_cta;
-}
-
 template <typename real, int R, int KMAX, int G, int TAIL, int WARPS, int MINB, int LEAN = 0,
           int SMH = 0>
 int fast_bdg_wave(int nb_iter) {
     const size_t beta_bytes = ((size_t)nb_iter * sizeof(real) + 15) & ~(size_t)15;
     const size_t smem = beta_bytes + (size_t)WARPS * fastg_warp_bytes<real, R, KMAX, G, LEAN, SMH>();
-    return fast_wave_voxels(fast_bdg_kernel<real, R, KMAX, G, TAIL, WARPS, MINB, LEAN, SMH>, WARPS * 32,
-                            smem, WARPS * (32 / G));
+    return wave_voxels(fast_bdg_kernel<real, R, KMAX, G, TAIL, WARPS, MINB, LEAN, SMH>, WARPS * 32, smem,
+                       WARPS * (32 / G));
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1039,49 +1022,16 @@ fast_deconvg_es_kernel(DeconvArgs<real> p, int ring_rows) {
 template <typename real, int R, int KMAX, int G, int TAIL, int WARPS, int MINB>
 int fast_deconvg_launch(const DeconvArgs<real> &a, cudaStream_t stream) {
     constexpr int VPW = 32 / G;
+    const size_t beta_bytes = ((size_t)a.nb_iter * sizeof(real) + 15) & ~(size_t)15;
     if (a.early_stopping && a.wind >= 2) {
         if (!a.queue) return FAST_NO_MATCH;
         const int ring_rows = a.wind - 1;
-        const size_t beta_bytes = ((size_t)a.nb_iter * sizeof(real) + 15) & ~(size_t)15;
-        const size_t smem_es = beta_bytes + (size_t)WARPS * ring_rows * 32 * fastg_block_floats<R>() * sizeof(real);
-        auto kes = fast_deconvg_es_kernel<real, R, KMAX, G, TAIL, WARPS, MINB>;
-        int dev = 0, sms = 0, occ = 0, max_smem = 0;
-        cudaError_t e = cudaGetDevice(&dev);
-        if (e != cudaSuccess) return (int)e;
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-        if (smem_es > (size_t)max_smem) return FAST_NO_MATCH;
-        e = cudaFuncSetAttribute(kes, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_es);
-        if (e != cudaSuccess) return (int)e;
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kes, WARPS * 32, smem_es);
-        if (e != cudaSuccess) return (int)e;
-        if (occ < 1) return FAST_NO_MATCH;
-        e = cudaMemsetAsync(a.queue, 0, sizeof(unsigned int), stream);
-        if (e != cudaSuccess) return (int)e;
-        const int64_t per_cta = (int64_t)WARPS * VPW;
-        const int64_t need = (a.V + per_cta - 1) / per_cta;
-        const int64_t cap = (int64_t)sms * occ;
-        kes<<<(int)(need < cap ? need : cap), WARPS * 32, smem_es, stream>>>(a, ring_rows);
-        e = cudaGetLastError();
-        return e == cudaSuccess ? 0 : (int)e;
+        const size_t smem = beta_bytes + (size_t)WARPS * ring_rows * 32 * fastg_block_floats<R>() * sizeof(real);
+        return launch_persistent(fast_deconvg_es_kernel<real, R, KMAX, G, TAIL, WARPS, MINB>, WARPS * 32, smem,
+                                 WARPS * VPW, a.V, a.queue, stream, a, ring_rows);
     }
-    const size_t smem = ((size_t)a.nb_iter * sizeof(real) + 15) & ~(size_t)15;
-    auto kern = fast_deconvg_kernel<real, R, KMAX, G, TAIL, WARPS, MINB>;
-    int dev = 0, sms = 0, occ = 0;
-    cudaError_t e = cudaGetDevice(&dev);
-    if (e != cudaSuccess) return (int)e;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return (int)e;
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, WARPS * 32, smem);
-    if (e != cudaSuccess) return (int)e;
-    if (occ < 1) return FAST_NO_MATCH;
-    const int64_t per_cta = (int64_t)WARPS * VPW;
-    const int64_t need = (a.V + per_cta - 1) / per_cta;
-    const int64_t cap = (int64_t)sms * occ;
-    kern<<<(int)(need < cap ? need : cap), WARPS * 32, smem, stream>>>(a);
-    e = cudaGetLastError();
-    return e == cudaSuccess ? 0 : (int)e;
+    return launch_persistent(fast_deconvg_kernel<real, R, KMAX, G, TAIL, WARPS, MINB>, WARPS * 32, beta_bytes,
+                             WARPS * VPW, a.V, nullptr, stream, a);
 }
 
 template <int R, int KMAX, int G, int TAIL>
@@ -1095,33 +1045,19 @@ bool fastg_shape_ok(int T, int K) {
 template <typename real, int R, int KMAX, int G, int TAIL, int WARPS, int MINB, int LEAN = 0,
           int SMH = 0, bool ES = false>
 int fast_bdg_launch(const BdArgs<real> &a, cudaStream_t stream) {
-    constexpr int VPW = 32 / G;
     const size_t beta_bytes = ((size_t)a.nb_iter * sizeof(real) + 15) & ~(size_t)15;
     const size_t smem = beta_bytes + (size_t)WARPS * fastg_warp_bytes<real, R, KMAX, G, LEAN, SMH>();
-    auto kern = fast_bdg_kernel<real, R, KMAX, G, TAIL, WARPS, MINB, LEAN, SMH, ES>;
-    int dev = 0, sms = 0, max_smem = 0;
-    cudaError_t e = cudaGetDevice(&dev);
-    if (e != cudaSuccess) return (int)e;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-    if (smem > (size_t)max_smem) return FAST_NO_MATCH;
-    e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return (int)e;
-    int occ = 0;
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, WARPS * 32, smem);
-    if (e != cudaSuccess) return (int)e;
-    if (occ < 1) return FAST_NO_MATCH;
-    const int64_t per_cta = (int64_t)WARPS * VPW;
-    const int64_t need = (a.V + per_cta - 1) / per_cta;
-    const int64_t cap = (int64_t)sms * occ;
-    const int grid = (int)(need < cap ? need : cap);
-    if (a.queue) {
-        e = cudaMemsetAsync(a.queue, 0, sizeof(unsigned int), stream);
-        if (e != cudaSuccess) return (int)e;
-    }
-    kern<<<grid, WARPS * 32, smem, stream>>>(a);
-    e = cudaGetLastError();
-    return e == cudaSuccess ? 0 : (int)e;
+    return launch_persistent(fast_bdg_kernel<real, R, KMAX, G, TAIL, WARPS, MINB, LEAN, SMH, ES>, WARPS * 32, smem,
+                             WARPS * (32 / G), a.V, a.queue, stream, a);
+}
+
+template <typename real, int R, int KMAX, int G, int TAIL, int WARPS, int MINB>
+constexpr Variant<real> group_variant() {
+    return {TIER_GROUP_CTA, G, R, KMAX, TAIL, false, fastg_shape_ok<R, KMAX, G, TAIL>,
+            fast_bdg_launch<real, R, KMAX, G, TAIL, WARPS, MINB>,
+            fast_bdg_launch<real, R, KMAX, G, TAIL, WARPS, MINB, 0, 0, true>,
+            fast_deconvg_launch<real, R, KMAX, G, TAIL, WARPS, MINB>,
+            fast_bdg_wave<real, R, KMAX, G, TAIL, WARPS, MINB>};
 }
 
 }  // namespace pb

@@ -188,6 +188,25 @@ int pb_deconv_lbda_path_f64(const double *y, const double *h, const double *L, c
                             int n_lbda, int nb_iter, double *out_x, double *out_z, double *out_dz,
                             double *out_J, int32_t *out_niter, int64_t V, int T, int K, pb_stream_t stream);
 
+/* Same path with per-voxel HRFs, the reference's early stop and the cost terms of every problem -- a loop of
+ * `deconv(y, t_r, h, lbda=l, early_stopping=..., tol=..., wind=...)` over lbdas, in one launch.
+ *   h[v*h_stride + k], L[v*L_stride]   taps and Lipschitz constant of voxel v (strides 0: shared)
+ *   early_stopping, wind, tol          as in pb_deconv_*: out_niter[l*V + v] = iterations done, out_J rows are
+ *                                      written up to it (the caller fills the tail, e.g. with NaN)
+ *   out_r, out_g [n_lbda * V]          terms of the final cost J = 0.5 R + lambda G of each problem:
+ *                                      R = ||x - y||^2, G = ||diff_z||_1, in the working precision
+ * out_J, out_r and out_g may be NULL (not written).  out_x, out_z, out_dz are always written; a caller that
+ * only wants the cost terms cuts V into ranges and reuses the same solution buffers range after range. */
+int pb_deconv_lbda_path_ex_f32(const float *y, const float *h, int64_t h_stride, const float *L, int64_t L_stride,
+                               const float *lbdas, int n_lbda, int nb_iter, int early_stopping, int wind,
+                               double tol, float *out_x, float *out_z, float *out_dz, float *out_J, float *out_r,
+                               float *out_g, int32_t *out_niter, int64_t V, int T, int K, pb_stream_t stream);
+int pb_deconv_lbda_path_ex_f64(const double *y, const double *h, int64_t h_stride, const double *L,
+                               int64_t L_stride, const double *lbdas, int n_lbda, int nb_iter, int early_stopping,
+                               int wind, double tol, double *out_x, double *out_z, double *out_dz, double *out_J,
+                               double *out_r, double *out_g, int32_t *out_niter, int64_t V, int T, int K,
+                               pb_stream_t stream);
+
 /* ---- A10: the theta step alone / hrf_estim (pybold/bold_signal.py:217-239, :329-334) --
  * theta[v] <- bounded local minimiser of 0.5||y_v - h(theta)*z_v||^2 from theta0;
  * out_h [V,K] = non-normalised taps at the minimiser; out_cost [V] = the cost there. */

@@ -137,43 +137,133 @@ def deconv(y, t_r, hrf, lbda=None, early_stopping=True, tol=1.0e-6,  # noqa
     return (like_input(x, y), like_input(z, y), like_input(dz, y), like_input(Jn, y), None, None)
 
 
-def deconv_lbda_path(y, t_r, hrf, lbdas, nb_iter=200, x0=None, dtype=None, max_problems=1 << 21):
-    """Regularisation path: ``deconv`` (fixed lambda, no early stopping) for every lambda of ``lbdas``
-    and every voxel of ``y[V, T]`` -- the grid search of examples/icassp_2019/validation.py batched
-    over (lambda, voxel) instead of looping (BASELINE.json configs[4]).
+# deconv_lbda_path_fit keeps no solution: each launch writes its (x, z, diff_z) into one scratch of at most this
+# many bytes, reused voxel range after voxel range.  4 GiB holds about 290 000 (lambda, voxel) problems at 1200
+# scans in FP32 (580 000 at 600): tens of waves of the persistent grid per launch, so the partly idle end of each
+# launch (early-stopped problems finish at different times) costs a few per cent at most, while the scratch stays
+# small beside the 180 GB of the card and a whole-brain y (1.1 GB at 230 000 x 1200 in FP32).
+FIT_SCRATCH_BYTES = 4 << 30
 
-    Returns ``(x, z, diff_z, J)`` with a leading lambda axis: ``[n_lbda, V, T]`` and
-    ``[n_lbda, V, nb_iter]`` (J normalised by its first entry like ``deconv``).  Every (lambda, voxel)
-    pair is an independent problem of ONE persistent launch (``pb_deconv_lbda_path_*``) that reads the
-    rows of ``y`` in place -- nothing is replicated per lambda -- and writes straight into the results;
-    more than ``max_problems`` pairs are cut into launches of whole lambdas.
-    """
+
+def _path_problem(y, hrf, lbdas, x0, dtype):
+    """Device inputs of the regularisation path: the rows of ``y``, the taps (``[K]`` shared or ``[V, K]``), the
+    Lipschitz constants ``0.9 x spectral_radius_est`` from ``x0`` -- per voxel with ``[V, K]`` taps, the constants
+    ``deconv(y, t_r, hrf, x0=x0)`` uses -- and the lambdas, with the element strides of the C ABI."""
     dtype = pick_dtype(y, hrf, dtype=dtype)
     yb, _ = _as_batch(y, dtype)
     yb = yb.contiguous()
     V, T = yb.shape
-    hd = to_device(hrf, dtype).reshape(-1).contiguous()
-    K = hd.numel()
+    hd = to_device(hrf, dtype)
+    if hd.dim() > 2 or (hd.dim() == 2 and hd.shape[0] not in (1, V)):
+        raise ValueError("hrf must be [K] (shared) or [V, K] with V = %d voxels, got %s"
+                         % (V, tuple(hd.shape)))
+    if hd.dim() == 2 and hd.shape[0] == 1:
+        hd = hd[0]
+    hd = hd.contiguous()
+    h_stride = hd.shape[-1] if hd.dim() == 2 else 0
     lb = upload(np.asarray(lbdas, dtype=np.float64).reshape(-1), dtype, yb.device)
-    n_l = lb.numel()
     if x0 is None:
         x0 = np.random.randn(T)
     est = spectral_radius_est(ConvAndLinear(DiscretInteg(), hd, dim_in=T), (T,), x0=to_device(x0, dtype))
-    lipschitz = per_voxel(_lipschitz_cst(est, dtype), 1, dtype, yb.device, "lipschitz")[0]
-    outs = [torch.empty((n_l, V, T), dtype=dtype, device=yb.device) for _ in range(3)]
-    J = torch.empty((n_l, V, nb_iter), dtype=dtype, device=yb.device)
-    n_iter = torch.empty(n_l * V, dtype=torch.int32, device=yb.device)
-    per = max(1, min(n_l, max_problems // max(V, 1)))
+    Lc, L_stride = per_voxel(_lipschitz_cst(est, dtype), V, dtype, yb.device, "lipschitz")
+    return yb, hd, h_stride, Lc, L_stride, lb
+
+
+def _path_launch(yb, hd, h_stride, Lc, L_stride, lb, nb_iter, early_stopping, wind, tol, sol, J, r, g, n_iter):
+    """One ``pb_deconv_lbda_path_ex`` launch: every lambda of ``lb`` x every row of ``yb``, problem (l, v) at
+    flat index l * V + v of the outputs.  ``sol`` = (x, z, diff_z) buffers of n_lbda * V * T elements; ``J``
+    (n_lbda * V * nb_iter), ``r`` and ``g`` may be None; ``n_iter`` holds n_lbda * V int32."""
+    V, T = yb.shape
     with torch.cuda.device(yb.device):
-        for l0 in range(0, n_l, per):
-            l1 = min(l0 + per, n_l)
-            rc = _lib.fn("pb_deconv_lbda_path", dtype)(
-                ptr(yb), ptr(hd), ptr(lipschitz), ptr(lb[l0:l1]), l1 - l0, int(nb_iter),
-                ptr(outs[0][l0:l1]), ptr(outs[1][l0:l1]), ptr(outs[2][l0:l1]), ptr(J[l0:l1]),
-                ptr(n_iter[l0 * V:l1 * V]), V, T, K, stream_ptr())
-            _lib.check(rc, "pb_deconv_lbda_path")
+        rc = _lib.fn("pb_deconv_lbda_path_ex", yb.dtype)(
+            ptr(yb), ptr(hd), h_stride, ptr(Lc), L_stride, ptr(lb), lb.numel(), int(nb_iter),
+            int(bool(early_stopping)), int(wind), float(tol), ptr(sol[0]), ptr(sol[1]), ptr(sol[2]),
+            ptr(J), ptr(r), ptr(g), ptr(n_iter), V, T, hd.shape[-1], stream_ptr())
+    _lib.check(rc, "pb_deconv_lbda_path_ex")
+
+
+def deconv_lbda_path(y, t_r, hrf, lbdas, nb_iter=200, x0=None, dtype=None, max_problems=1 << 21,
+                     early_stopping=False, tol=1.0e-6, wind=6):
+    """Regularisation path: ``deconv(y, t_r, hrf, lbda=l, nb_iter=nb_iter, x0=x0, early_stopping=...,
+    tol=..., wind=...)`` for every lambda of ``lbdas`` and every voxel of ``y[V, T]`` -- the grid search of
+    examples/icassp_2019/validation.py batched over (lambda, voxel) instead of looping (BASELINE.json configs[4]).
+
+    ``hrf`` is ``[K]`` (shared) or ``[V, K]`` (one HRF per voxel, e.g. from ``bd``); with ``[V, K]`` the
+    Lipschitz constants are per voxel, from the same ``x0``.  Early stopping is off by default (the cfg5 grid
+    runs every iteration); with ``early_stopping=True`` each problem stops like the reference's ``deconv``.
+
+    Returns ``(x, z, diff_z, J)`` with a leading lambda axis: ``[n_lbda, V, T]`` and
+    ``[n_lbda, V, nb_iter]`` (J normalised by its first entry like ``deconv``, NaN past a problem's stop
+    iteration).  Every (lambda, voxel) pair is an independent problem of ONE persistent launch
+    (``pb_deconv_lbda_path_ex_*``) that reads the rows of ``y`` in place -- nothing is replicated per lambda --
+    and writes straight into the results; more than ``max_problems`` pairs are cut into launches of whole
+    lambdas.  The solutions take ``3 n_lbda V T`` elements on the device: to choose lambda at whole-brain size,
+    use :func:`deconv_lbda_path_fit`.
+    """
+    yb, hd, h_stride, Lc, L_stride, lb = _path_problem(y, hrf, lbdas, x0, dtype)
+    V, T = yb.shape
+    n_l = lb.numel()
+    outs = [torch.empty((n_l, V, T), dtype=yb.dtype, device=yb.device) for _ in range(3)]
+    if early_stopping:
+        J = torch.full((n_l, V, nb_iter), float("nan"), dtype=yb.dtype, device=yb.device)
+    else:                                                         # every entry is written
+        J = torch.empty((n_l, V, nb_iter), dtype=yb.dtype, device=yb.device)
+    n_iter = torch.empty((n_l, V), dtype=torch.int32, device=yb.device)
+    per = max(1, min(n_l, max_problems // max(V, 1)))
+    for l0 in range(0, n_l, per):
+        l1 = min(l0 + per, n_l)
+        _path_launch(yb, hd, h_stride, Lc, L_stride, lb[l0:l1], nb_iter, early_stopping, wind, tol,
+                     [o[l0:l1] for o in outs], J[l0:l1], None, None, n_iter[l0:l1])
     J /= (J[:, :, :1] + 1.0e-30)                                   # bold_signal.py:97, in place
     return tuple(like_input(t, y) for t in outs) + (like_input(J, y),)
+
+
+def deconv_lbda_path_fit(y, t_r, hrf, lbdas, nb_iter=200, early_stopping=False, tol=1.0e-6, wind=6, x0=None,
+                         dtype=None):
+    """Data-fit and penalty terms of every (lambda, voxel) problem of :func:`deconv_lbda_path`, without
+    keeping the solutions: what choosing lambda needs, at any number of voxels.
+
+    Returns ``(R, G, n_iter)``, each ``[n_lbda, V]``: ``R = ||x - y||^2`` and ``G = ||diff_z||_1`` of the
+    solution ``deconv(y, t_r, hrf, lbda=l, ...)`` returns (the reference's own ``R`` and ``G``,
+    bold_signal.py:139-145; its cost is ``0.5 R + l G``), in the working precision, and the number of
+    iterations each problem ran.  Arguments as in :func:`deconv_lbda_path`.
+
+    The batch is cut into voxel ranges; one launch solves every lambda of a range, so the rows of ``y`` are
+    still read once per voxel, and its solutions go to one scratch of at most ``FIT_SCRATCH_BYTES`` reused
+    from range to range.  Device memory is ``y``, ``hrf``, the three ``[n_lbda, V]`` results and that scratch,
+    whatever V is.  The library does not choose lambda; a two-stage use, picking per voxel the lambda whose
+    data fit is nearest the noise level (the target the reference's ``lbda=None`` loop steers toward), then
+    solving once at it -- the same kernel, so the rows equal the path's rows at the chosen lambdas::
+
+        R, G, n_iter = deconv_lbda_path_fit(y, t_r, h, lbdas, nb_iter=200, early_stopping=True, x0=x0)
+        sigma = mad_daub_noise_est(y)                              # [V]
+        lbda_v = np.asarray(lbdas)[np.argmin(np.abs(R - y.shape[1] * sigma ** 2), axis=0)]
+        x, z, diff_z, J, _, _ = deconv(y, t_r, h, lbda=lbda_v, nb_iter=200, early_stopping=True, x0=x0)
+    """
+    yb, hd, h_stride, Lc, L_stride, lb = _path_problem(y, hrf, lbdas, x0, dtype)
+    V, T = yb.shape
+    n_l = lb.numel()
+    dev = yb.device
+    R = torch.empty((n_l, V), dtype=yb.dtype, device=dev)
+    G = torch.empty((n_l, V), dtype=yb.dtype, device=dev)
+    n_iter = torch.empty((n_l, V), dtype=torch.int32, device=dev)
+    if V == 0 or n_l == 0:
+        return like_input(R, y), like_input(G, y), like_input(n_iter, y)
+    # voxels per launch: three solution planes [n_lbda, vc, T] within the scratch budget
+    vc = max(1, min(V, FIT_SCRATCH_BYTES // (3 * n_l * T * yb.element_size())))
+    scratch = torch.empty((3, n_l * vc * T), dtype=yb.dtype, device=dev)
+    r = torch.empty(n_l * vc, dtype=yb.dtype, device=dev)
+    g = torch.empty_like(r)
+    n_it = torch.empty(n_l * vc, dtype=torch.int32, device=dev)
+    for v0 in range(0, V, vc):
+        v1 = min(v0 + vc, V)
+        n = v1 - v0
+        _path_launch(yb[v0:v1], hd[v0:v1] if h_stride else hd, h_stride, Lc[v0:v1] if L_stride else Lc,
+                     L_stride, lb, nb_iter, early_stopping, wind, tol, scratch, None, r, g, n_it)
+        R[:, v0:v1] = r[:n_l * n].view(n_l, n)
+        G[:, v0:v1] = g[:n_l * n].view(n_l, n)
+        n_iter[:, v0:v1] = n_it[:n_l * n].view(n_l, n)
+    return like_input(R, y), like_input(G, y), like_input(n_iter, y)
 
 
 def bd_alloc(V, T, K, nb_iter, dtype, dev):

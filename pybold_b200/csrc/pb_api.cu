@@ -682,18 +682,29 @@ int pb_hrf_len_ex(double t_r, double dur, double dt) {
         a.T = T; a.K = K; a.active = active;                                                           \
         return run_deconv<REAL>(a, s);                                                                 \
     }                                                                                                  \
+    int pb_deconv_lbda_path_ex_##SUF(const REAL *y, const REAL *h, int64_t h_stride, const REAL *L,    \
+                                     int64_t L_stride, const REAL *lbdas, int n_lbda, int nb_iter,     \
+                                     int early_stopping, int wind, double tol, REAL *out_x,            \
+                                     REAL *out_z, REAL *out_dz, REAL *out_J, REAL *out_r,              \
+                                     REAL *out_g, int32_t *out_niter, int64_t V, int T, int K,         \
+                                     pb_stream_t s) {                                                  \
+        if (n_lbda < 0 || V < 0 || h_stride < 0 || L_stride < 0) return PB_ERR_INVALID_ARG;          \
+        pb::DeconvArgs<REAL> a;                                                                        \
+        a.y = y; a.h = h; a.h_stride = h_stride; a.L = L; a.L_stride = L_stride; a.lbda = lbdas;       \
+        a.lbda_stride = 0; a.w0 = nullptr; a.nb_iter = nb_iter; a.early_stopping = early_stopping;     \
+        a.wind = wind; a.tol = tol; a.out_x = out_x; a.out_z = out_z; a.out_dz = out_dz;               \
+        a.out_J = out_J; a.out_r = out_r; a.out_g = out_g; a.out_niter = out_niter;                    \
+        a.V = (int64_t)n_lbda * V; a.T = T; a.K = K;                                                   \
+        a.y_mod = V; a.lbda_div = V;                                                                   \
+        return run_deconv<REAL>(a, s);                                                                 \
+    }                                                                                                  \
     int pb_deconv_lbda_path_##SUF(const REAL *y, const REAL *h, const REAL *L, const REAL *lbdas,      \
                                   int n_lbda, int nb_iter, REAL *out_x, REAL *out_z, REAL *out_dz,     \
                                   REAL *out_J, int32_t *out_niter, int64_t V, int T, int K,            \
                                   pb_stream_t s) {                                                     \
-        if (n_lbda < 0 || V < 0) return PB_ERR_INVALID_ARG;                                            \
-        pb::DeconvArgs<REAL> a;                                                                        \
-        a.y = y; a.h = h; a.h_stride = 0; a.L = L; a.L_stride = 0; a.lbda = lbdas;                     \
-        a.lbda_stride = 0; a.w0 = nullptr; a.nb_iter = nb_iter; a.early_stopping = 0; a.wind = 0;      \
-        a.tol = 0.0; a.out_x = out_x; a.out_z = out_z; a.out_dz = out_dz; a.out_J = out_J;             \
-        a.out_niter = out_niter; a.V = (int64_t)n_lbda * V; a.T = T; a.K = K;                          \
-        a.y_mod = V; a.lbda_div = V;                                                                   \
-        return run_deconv<REAL>(a, s);                                                                 \
+        return pb_deconv_lbda_path_ex_##SUF(y, h, 0, L, 0, lbdas, n_lbda, nb_iter, 0, 0, 0.0, out_x,   \
+                                            out_z, out_dz, out_J, nullptr, nullptr, out_niter, V, T,   \
+                                            K, s);                                                     \
     }                                                                                                  \
     int pb_bd_##SUF(const REAL *y, double t_r, double hrf_dur, const REAL *lbda, int64_t lbda_stride,  \
                     const REAL *theta0, int64_t theta0_stride, const REAL *z0, double theta_lo,        \

@@ -269,7 +269,7 @@ fast_deconv_kernel(DeconvArgs<real> p, int ring_rows) {
     for (int64_t v = (int64_t)blockIdx.x * WARPS + warp; v < p.V; v += (int64_t)gridDim.x * WARPS) {
         if (!p.is_active(v)) continue;
         const real *yv = p.y_row(v);
-        const real *hv = p.h + v * p.h_stride;
+        const real *hv = p.h_row(v);
         vx.set_dy(yv, T);
 #pragma unroll
         for (int j = 0; j < KMAX; ++j) vx.h[j] = (j < K && vx.nvalid > 0) ? hv[j] : real(0);
@@ -278,7 +278,7 @@ fast_deconv_kernel(DeconvArgs<real> p, int ring_rows) {
             const int i = lane * R + r;
             vx.w[r] = (p.w0 && i < T) ? p.w0[v * T + i] : real(0);
         }
-        const double Lc = (double)p.L[v * p.L_stride];
+        const double Lc = p.L_of(v);
         const double lam = p.lam_of(v);
         const real step = (real)(1.0 / Lc), th = (real)(lam / Lc);
         real *Jv = p.out_J + v * (int64_t)p.nb_iter;
@@ -337,9 +337,14 @@ fast_deconv_kernel(DeconvArgs<real> p, int ring_rows) {
         }
         vx.forward(res);
         if (n_done > 0) {
-            const double J = 0.5 * warp_sum((double)vx.partial_sumsq(res)) +
-                             lam * warp_sum((double)vx.partial_sumabs(vx.w));
-            if (lane == 0 && p.out_J) Jv[n_done - 1] = (real)J;
+            const double rr = warp_sum((double)vx.partial_sumsq(res));
+            const double gg = warp_sum((double)vx.partial_sumabs(vx.w));
+            const double J = 0.5 * rr + lam * gg;
+            if (lane == 0) {
+                if (p.out_J) Jv[n_done - 1] = (real)J;
+                if (p.out_r) p.out_r[v] = (real)rr;
+                if (p.out_g) p.out_g[v] = (real)gg;
+            }
         }
         real y[R], z[R];
         vx.load_y(yv, T, y);

@@ -782,7 +782,7 @@ fast_deconvg_kernel(DeconvArgs<real> p) {
         if (!__any_sync(PB_FULL, on)) continue;
         const int64_t v = on ? v0 + grp : p.V - 1;
         const real *yv = p.y_row(v);
-        const real *hv = p.h + v * p.h_stride;
+        const real *hv = p.h_row(v);
         vx.set_dy(yv, T);
 #pragma unroll
         for (int j = 0; j < KMAX; ++j) vx.h[j] = j < K ? hv[j] : real(0);
@@ -791,7 +791,7 @@ fast_deconvg_kernel(DeconvArgs<real> p) {
             const int i = q * R + r;
             vx.w[r] = (p.w0 && i < T) ? p.w0[v * T + i] : real(0);
         }
-        const double Lc = (double)p.L[v * p.L_stride];
+        const double Lc = p.L_of(v);
         const double lam = p.lam_of(v);
         const real step = (real)(1.0 / Lc), th = (real)(lam / Lc);
         real *Jv = p.out_J + v * (int64_t)p.nb_iter;
@@ -811,9 +811,12 @@ fast_deconvg_kernel(DeconvArgs<real> p) {
         }
         vx.forward(res);
         {
-            const double J = 0.5 * (double)Seg<real, G>::sum(vx.partial_sumsq(res)) +
-                             lam * (double)Seg<real, G>::sum(vx.partial_sumabs(vx.w));
+            const double rr = (double)Seg<real, G>::sum(vx.partial_sumsq(res));
+            const double gg = (double)Seg<real, G>::sum(vx.partial_sumabs(vx.w));
+            const double J = 0.5 * rr + lam * gg;
             if (tracer) Jv[p.nb_iter - 1] = (real)J;
+            if (writer && p.out_r) p.out_r[v] = (real)rr;
+            if (writer && p.out_g) p.out_g[v] = (real)gg;
         }
         real y[R], z[R];
         vx.load_y(yv, T, y);
@@ -887,7 +890,7 @@ fast_deconvg_es_kernel(DeconvArgs<real> p, int ring_rows) {
                 active = (int64_t)idx < p.V;
                 if (active) {
                     v = idx;
-                    const real *hv = p.h + v * p.h_stride;
+                    const real *hv = p.h_row(v);
                     vx.set_dy(p.y_row(v), T);
 #pragma unroll
                     for (int j = 0; j < KMAX; ++j) vx.h[j] = j < K ? hv[j] : real(0);
@@ -896,7 +899,7 @@ fast_deconvg_es_kernel(DeconvArgs<real> p, int ring_rows) {
                         const int i = q * R + r;
                         vx.w[r] = (p.w0 && i < T) ? p.w0[v * T + i] : real(0);
                     }
-                    const double Lc = (double)p.L[v * p.L_stride];
+                    const double Lc = p.L_of(v);
                     lam = p.lam_of(v);
                     step = (real)(1.0 / Lc);
                     th = (real)(lam / Lc);
@@ -978,8 +981,17 @@ fast_deconvg_es_kernel(DeconvArgs<real> p, int ring_rows) {
 #pragma unroll
             for (int r = 0; r < R; ++r) z[r] = vx.w[r];
             vx.scan_fwd(z);
+            // the two terms of the last cost, summed again like above (same values) rather than carried
+            // through every turn in registers
+            double rr = 0.0, gg = 0.0;
+            if (p.out_r || p.out_g) {
+                rr = (double)Seg<real, G>::sum(vx.partial_sumsq(res));
+                gg = (double)Seg<real, G>::sum(vx.partial_sumabs(vx.w));
+            }
             if (closing) {
                 if (q == 0) p.out_niter[v] = k;
+                if (q == 0 && p.out_r) p.out_r[v] = (real)rr;
+                if (q == 0 && p.out_g) p.out_g[v] = (real)gg;
                 real y[R];
                 vx.load_y(p.y_row(v), T, y);
 #pragma unroll

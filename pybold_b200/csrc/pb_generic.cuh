@@ -219,9 +219,13 @@ struct DeconvArgs {
     int32_t *out_niter;
     int64_t V;
     int T, K;
+    // optional [V] terms of the final cost J = 0.5 R + lambda G of the returned iterate w (null: not written):
+    // R = ||x - y||^2 = ||A w - y||^2, G = ||w||_1
+    real *out_r = nullptr, *out_g = nullptr;
     // regularisation path (cfg5): problem p = l * y_mod + v solves voxel v with lambda l.  y_mod > 0 makes
-    // the problems share the y rows (row p % y_mod) instead of a replicated copy, lbda_div > 0 takes
-    // lbda[p / lbda_div].  Both 0: one y row and one lbda (element stride lbda_stride) per problem.
+    // the problems share the voxel's y row, taps row and Lipschitz constant (voxel p % y_mod) instead of a
+    // replicated copy, lbda_div > 0 takes lbda[p / lbda_div].  Both 0: one voxel and one lbda (element
+    // stride lbda_stride) per problem.
     int64_t y_mod = 0, lbda_div = 0;
     // early-stopping group kernel: device counter (zeroed on the launch stream) the groups pull voxels from
     unsigned int *queue = nullptr;
@@ -229,7 +233,11 @@ struct DeconvArgs {
     // of deconv(lbda=None) keeps calling with fewer and fewer live voxels); out_J may be null (no cost trace)
     const unsigned char *active = nullptr;
     __device__ __forceinline__ bool is_active(int64_t v) const { return !active || active[v] != 0; }
-    __device__ __forceinline__ const real *y_row(int64_t v) const { return y + (y_mod ? v % y_mod : v) * T; }
+    __device__ __forceinline__ int64_t voxel_of(int64_t v) const { return y_mod ? v % y_mod : v; }
+    __device__ __forceinline__ const real *y_row(int64_t v) const { return y + voxel_of(v) * T; }
+    // taps row and Lipschitz constant of the problem's voxel (h_stride / L_stride 0: shared)
+    __device__ __forceinline__ const real *h_row(int64_t v) const { return h + voxel_of(v) * h_stride; }
+    __device__ __forceinline__ double L_of(int64_t v) const { return (double)L[voxel_of(v) * L_stride]; }
     __device__ __forceinline__ double lam_of(int64_t v) const {
         return (double)lbda[lbda_div ? v / lbda_div : v * lbda_stride];
     }
@@ -252,14 +260,14 @@ __global__ void generic_deconv_kernel(DeconvArgs<real> p, GenLayout lay) {
     for (int64_t v = (int64_t)blockIdx.x * nwarp + warp; v < p.V; v += (int64_t)gridDim.x * nwarp) {
         if (!p.is_active(v)) continue;
         const real *yv = p.y_row(v);
-        const real *hv = p.h + v * p.h_stride;
+        const real *hv = p.h_row(v);
         for (int i = lane; i < T; i += 32) {
             g.ys[i] = yv[i];
             g.ws[i] = p.w0 ? p.w0[v * T + i] : real(0);
         }
         for (int a = lane; a < K; a += 32) g.hr[a] = hv[a];
         __syncwarp();
-        const double Lc = (double)p.L[v * p.L_stride];
+        const double Lc = p.L_of(v);
         const double lam = p.lam_of(v);
         const real step = (real)(1.0 / Lc), th = (real)(lam / Lc);
         real *Jv = p.out_J + v * (int64_t)p.nb_iter;
@@ -305,8 +313,13 @@ __global__ void generic_deconv_kernel(DeconvArgs<real> p, GenLayout lay) {
         }
         g.forward();
         if (n_done > 0) {
-            const double J = 0.5 * g.sumsq(g.bs) + lam * g.sumabs(g.ws);
-            if (lane == 0 && p.out_J) Jv[n_done - 1] = (real)J;
+            const double rr = g.sumsq(g.bs), gg = g.sumabs(g.ws);
+            const double J = 0.5 * rr + lam * gg;
+            if (lane == 0) {
+                if (p.out_J) Jv[n_done - 1] = (real)J;
+                if (p.out_r) p.out_r[v] = (real)rr;
+                if (p.out_g) p.out_g[v] = (real)gg;
+            }
         }
         for (int i = lane; i < T; i += 32) {
             p.out_x[v * T + i] = g.bs[i] + g.ys[i];

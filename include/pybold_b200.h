@@ -176,6 +176,29 @@ int pb_deconv_masked_f64(const double *y, const double *h, int64_t h_stride, con
                          double *out_dz, double *out_J, int32_t *out_niter, int64_t V, int T, int K,
                          pb_stream_t stream);
 
+/* ---- N1: `deconv(lbda=None)`, the noise-constrained lambda (pybold/bold_signal.py:99-214), in ONE launch: every
+ * voxel runs its outer loop inside the deconv kernel -- alpha = 1, lbda = 1 / (2 alpha); per outer iteration an
+ * inner pass of at most nb_sub_iter prox-gradient iterations (warm start, Q5 early stop), then
+ * alpha += 1e-4 (||x - y||^2 - T sigma^2), lbda = 1 / (2 alpha) and the alpha-window stop (`early_stopping`, `wind`,
+ * `tol`); then one final inner pass with the last lambda.  Asynchronous on `stream`.
+ *   h[v*h_stride + k], L[v*L_stride], sigma[v*sigma_stride]   taps, Lipschitz constant, noise level (strides 0: shared)
+ *   nb_iter >= 1            outer iterations at most; nb_sub_iter <= pb_max_iter() inner iterations per pass
+ *   out_x, out_z, out_dz    [V,T] from the final pass
+ *   out_J, out_R, out_G     [V, nb_iter]: 0.5 R + lbda G (with the updated lbda), ||x - y||^2, ||diff_z||_1 of every
+ *                           outer iteration, NaN past the voxel's outer count
+ *   out_lbda [V]            the lambda of the final pass;  out_nouter [V]  outer iterations done
+ * out_J, out_R, out_G, out_lbda and out_nouter may be NULL (not written). */
+int pb_deconv_auto_f32(const float *y, const float *h, int64_t h_stride, const float *L, int64_t L_stride,
+                       const float *sigma, int64_t sigma_stride, int nb_iter, int nb_sub_iter, int early_stopping,
+                       int wind, double tol, float *out_x, float *out_z, float *out_dz, float *out_J, float *out_R,
+                       float *out_G, float *out_lbda, int32_t *out_nouter, int64_t V, int T, int K,
+                       pb_stream_t stream);
+int pb_deconv_auto_f64(const double *y, const double *h, int64_t h_stride, const double *L, int64_t L_stride,
+                       const double *sigma, int64_t sigma_stride, int nb_iter, int nb_sub_iter, int early_stopping,
+                       int wind, double tol, double *out_x, double *out_z, double *out_dz, double *out_J,
+                       double *out_R, double *out_G, double *out_lbda, int32_t *out_nouter, int64_t V, int T,
+                       int K, pb_stream_t stream);
+
 /* ---- cfg5: regularisation path, `deconv` (fixed lambda, no early stopping, pybold/bold_signal.py:49-97)
  * for every lambda of lbdas[n_lbda] and every voxel of y[V,T] in one launch -- the lambda grid search of
  * examples/icassp_2019/validation.py batched over (lambda, voxel).  Problem (l, v) reads row v of y (the

@@ -53,6 +53,8 @@ _OPS = {
                   _P, _P, _P, _P, _P, c_int64, c_int, c_int, _P],
     "pb_deconv_masked": [_P, _P, c_int64, _P, c_int64, _P, c_int64, _P, _P, c_int, c_int, c_int, c_double,
                          _P, _P, _P, _P, _P, c_int64, c_int, c_int, _P],
+    "pb_deconv_auto": [_P, _P, c_int64, _P, c_int64, _P, c_int64, c_int, c_int, c_int, c_int, c_double,
+                       _P, _P, _P, _P, _P, _P, _P, _P, c_int64, c_int, c_int, _P],
     "pb_deconv_lbda_path": [_P, _P, _P, _P, c_int, c_int, _P, _P, _P, _P, _P, c_int64, c_int, c_int, _P],
     "pb_deconv_lbda_path_ex": [_P, _P, c_int64, _P, c_int64, _P, c_int, c_int, c_int, c_int, c_double,
                                _P, _P, _P, _P, _P, _P, _P, c_int64, c_int, c_int, _P],

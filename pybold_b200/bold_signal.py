@@ -91,6 +91,44 @@ def deconv_batch(y, hrf, lbda, lipschitz, w0=None, early_stopping=True, tol=1.0e
     return x, z, dz, J, n_iter
 
 
+def deconv_auto_batch(y, hrf, sigma, lipschitz, nb_iter=1000, nb_sub_iter=1000, early_stopping=True, tol=1.0e-6,
+                      wind=6):
+    """Device entry point of ``deconv(lbda=None)`` (pybold/bold_signal.py:99-214): tensors in, dict of tensors out.
+
+    ``y`` is ``[V, T]`` on the device, ``hrf`` ``[K]`` (shared) or ``[V, K]``, ``sigma`` (noise level) and
+    ``lipschitz`` scalars or ``[V]``.  Every voxel runs its whole outer loop -- at most ``nb_iter`` outer iterations
+    of at most ``nb_sub_iter`` inner ones, then the final inner pass -- inside ONE persistent kernel launch
+    (``pb_deconv_auto_*``); with every input already on the device the call makes no host synchronisation.
+
+    Returns ``{x, z, diff_z}`` (``[V, T]``, final pass), ``{J, R, G}`` (``[V, nb_iter]``, one entry per outer
+    iteration, NaN past the voxel's outer count), ``lbda`` (``[V]``, the lambda of the final pass) and
+    ``n_outer`` (``[V]`` int32, outer iterations done).
+    """
+    V, T = y.shape
+    dtype, dev = y.dtype, y.device
+    hrf = hrf.to(device=dev, dtype=dtype).contiguous()
+    K = hrf.shape[-1]
+    if hrf.dim() > 2 or (hrf.dim() == 2 and hrf.shape[0] not in (1, V)):
+        raise ValueError("hrf must be [K] (shared) or [V, K] with V = %d voxels, got %s"
+                         % (V, tuple(hrf.shape)))
+    h_stride = 0 if hrf.dim() == 1 or hrf.shape[0] == 1 else K
+    y = y.contiguous()
+    sg, sg_stride = per_voxel(sigma, V, dtype, dev, "sigma")
+    Lc, L_stride = per_voxel(lipschitz, V, dtype, dev, "lipschitz")
+    out = {k: torch.empty((V, T), dtype=dtype, device=dev) for k in ("x", "z", "diff_z")}
+    out.update({k: torch.empty((V, nb_iter), dtype=dtype, device=dev) for k in ("J", "R", "G")})
+    out["lbda"] = torch.empty(V, dtype=dtype, device=dev)
+    out["n_outer"] = torch.empty(V, dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        rc = _lib.fn("pb_deconv_auto", dtype)(
+            ptr(y), ptr(hrf), h_stride, ptr(Lc), L_stride, ptr(sg), sg_stride, int(nb_iter), int(nb_sub_iter),
+            int(bool(early_stopping)), int(wind), float(tol), ptr(out["x"]), ptr(out["z"]), ptr(out["diff_z"]),
+            ptr(out["J"]), ptr(out["R"]), ptr(out["G"]), ptr(out["lbda"]), ptr(out["n_outer"]), V, T, K,
+            stream_ptr())
+    _lib.check(rc, "pb_deconv_auto")
+    return out
+
+
 def _lipschitz_cst(est, dtype):
     """``0.9 * spectral_radius_est`` (bold_signal.py:52), the product taken in double like the reference does
     and rounded once to the build's type: the same constant on every path that solves the same problem."""

@@ -374,6 +374,32 @@ int run_toeplitz(const real *k, int klen, real *out, int64_t dim_out, int64_t di
     return last_error();
 }
 
+// the register-tiled variant the picker chooses, else the generic kernel; a.nb_outer > 0 selects the
+// deconv(lbda=None) instances
+template <typename real>
+int launch_deconv(const pb::DeconvArgs<real> &a, pb_stream_t stream) {
+    int rc = pb::fast_deconv_dispatch(a, (cudaStream_t)stream);
+    if (rc != pb::FAST_NO_MATCH) return rc;
+    DeviceInfo d = device_info();
+    if (d.err) return d.err;
+    const bool es = a.early_stopping && a.wind >= 2;
+    pb::GenLayout lay = pb::GenLayout::make(a.T, a.K, es ? a.wind - 1 : 0, false);
+    if (a.nb_outer > 0 && lay.doubles < (size_t)a.wind) lay.doubles = (size_t)a.wind;   // the window of alphas
+    const size_t beta_bytes = ((size_t)a.nb_iter * sizeof(real) + 15) & ~(size_t)15;
+    // long series in double with the early-stopping ring: rows that do not fit move to the output rows
+    while (beta_bytes + lay.warp_bytes(sizeof(real)) > (size_t)d.max_smem_optin && lay.spill_ring_row()) {
+    }
+    LaunchPlan p = plan_launch(d, beta_bytes, lay.warp_bytes(sizeof(real)), a.V, 8);
+    if (!p.warps) return PB_ERR_UNSUPPORTED;
+    auto go = [&](auto kern) {
+        int e = set_smem(kern, p.smem);
+        if (e) return e;
+        kern<<<p.grid, p.warps * 32, p.smem, (cudaStream_t)stream>>>(a, lay);
+        return last_error();
+    };
+    return a.nb_outer > 0 ? go(pb::generic_deconv_kernel<real, true>) : go(pb::generic_deconv_kernel<real, false>);
+}
+
 template <typename real>
 int run_deconv(pb::DeconvArgs<real> a, pb_stream_t stream) {
     if (a.V == 0) return PB_OK;
@@ -383,23 +409,27 @@ int run_deconv(pb::DeconvArgs<real> a, pb_stream_t stream) {
     if (a.T > PB_MAX_T || a.K > PB_MAX_K || a.nb_iter > PB_MAX_ITER) return PB_ERR_UNSUPPORTED;
     if (a.V == 0) return PB_OK;
     if (a.early_stopping && a.wind >= 2) a.queue = queue_slot();
-    int rc = pb::fast_deconv_dispatch(a, (cudaStream_t)stream);
-    if (rc != pb::FAST_NO_MATCH) return rc;
-    DeviceInfo d = device_info();
-    if (d.err) return d.err;
-    const bool es = a.early_stopping && a.wind >= 2;
-    pb::GenLayout lay = pb::GenLayout::make(a.T, a.K, es ? a.wind - 1 : 0, false);
-    const size_t beta_bytes = ((size_t)a.nb_iter * sizeof(real) + 15) & ~(size_t)15;
-    // long series in double with the early-stopping ring: rows that do not fit move to the output rows
-    while (beta_bytes + lay.warp_bytes(sizeof(real)) > (size_t)d.max_smem_optin && lay.spill_ring_row()) {
+    return launch_deconv(a, stream);
+}
+
+// deconv(lbda=None): the noise loop runs inside the kernel, nb_outer outer iterations at most, nb_iter inner
+// ones per pass
+template <typename real>
+int run_deconv_auto(pb::DeconvArgs<real> a, pb_stream_t stream) {
+    if (a.V == 0) return PB_OK;
+    if (!a.y || !a.h || !a.L || !a.sigma || !a.out_x || !a.out_z || !a.out_dz || a.V < 0 || a.T <= 0 ||
+        a.K <= 0 || a.nb_iter < 1 || a.nb_outer < 1 || a.wind < 0 || a.h_stride < 0 || a.L_stride < 0 ||
+        a.sigma_stride < 0)
+        return PB_ERR_INVALID_ARG;
+    if (a.T > PB_MAX_T || a.K > PB_MAX_K || a.nb_iter > PB_MAX_ITER) return PB_ERR_UNSUPPORTED;
+    // without early stopping (or with wind < 2, which has no window) the window length does not matter; 2 keeps
+    // the group kernel's ring of u's one row long
+    if (!(a.early_stopping && a.wind >= 2)) {
+        a.early_stopping = 0;
+        a.wind = 2;
     }
-    LaunchPlan p = plan_launch(d, beta_bytes, lay.warp_bytes(sizeof(real)), a.V, 8);
-    if (!p.warps) return PB_ERR_UNSUPPORTED;
-    auto kern = pb::generic_deconv_kernel<real>;
-    int e = set_smem(kern, p.smem);
-    if (e) return e;
-    kern<<<p.grid, p.warps * 32, p.smem, (cudaStream_t)stream>>>(a, lay);
-    return last_error();
+    a.queue = queue_slot();
+    return launch_deconv(a, stream);
 }
 
 template <typename real>
@@ -681,6 +711,21 @@ int pb_hrf_len_ex(double t_r, double dur, double dt) {
         a.out_z = out_z; a.out_dz = out_dz; a.out_J = out_J; a.out_niter = out_niter; a.V = V;         \
         a.T = T; a.K = K; a.active = active;                                                           \
         return run_deconv<REAL>(a, s);                                                                 \
+    }                                                                                                  \
+    int pb_deconv_auto_##SUF(const REAL *y, const REAL *h, int64_t h_stride, const REAL *L,            \
+                             int64_t L_stride, const REAL *sigma, int64_t sigma_stride, int nb_iter,     \
+                             int nb_sub_iter, int early_stopping, int wind, double tol, REAL *out_x,     \
+                             REAL *out_z, REAL *out_dz, REAL *out_J, REAL *out_R, REAL *out_G,           \
+                             REAL *out_lbda, int32_t *out_nouter, int64_t V, int T, int K,               \
+                             pb_stream_t s) {                                                            \
+        pb::DeconvArgs<REAL> a;                                                                        \
+        a.y = y; a.h = h; a.h_stride = h_stride; a.L = L; a.L_stride = L_stride; a.lbda = nullptr;     \
+        a.lbda_stride = 0; a.w0 = nullptr; a.nb_iter = nb_sub_iter; a.early_stopping = early_stopping; \
+        a.wind = wind; a.tol = tol; a.out_x = out_x; a.out_z = out_z; a.out_dz = out_dz;               \
+        a.out_J = out_J; a.out_niter = nullptr; a.V = V; a.T = T; a.K = K;                             \
+        a.sigma = sigma; a.sigma_stride = sigma_stride; a.nb_outer = nb_iter; a.out_R = out_R;         \
+        a.out_G = out_G; a.out_lbda = out_lbda; a.out_nouter = out_nouter;                             \
+        return run_deconv_auto<REAL>(a, s);                                                            \
     }                                                                                                  \
     int pb_deconv_lbda_path_ex_##SUF(const REAL *y, const REAL *h, int64_t h_stride, const REAL *L,    \
                                      int64_t L_stride, const REAL *lbdas, int n_lbda, int nb_iter,     \

@@ -250,7 +250,9 @@ struct WarpVoxel {
 // ------------------------------------------------------------------------------------------------
 // deconv, fixed lambda (pybold/bold_signal.py:49-97)
 // ------------------------------------------------------------------------------------------------
-template <typename real, int R, int KMAX, bool CIRC, int WARPS, int MINB>
+// AUTO: deconv(lbda=None), one inner pass per outer iteration of the noise loop (pb_noise_loop.cuh), then the
+// final pass; the window of alphas (wind doubles per warp) follows the rings in shared memory
+template <typename real, int R, int KMAX, bool CIRC, int WARPS, int MINB, bool AUTO = false>
 __global__ void __launch_bounds__(WARPS * 32, MINB)
 fast_deconv_kernel(DeconvArgs<real> p, int ring_rows) {
     extern __shared__ __align__(16) unsigned char smem[];
@@ -279,72 +281,91 @@ fast_deconv_kernel(DeconvArgs<real> p, int ring_rows) {
             vx.w[r] = (p.w0 && i < T) ? p.w0[v * T + i] : real(0);
         }
         const double Lc = p.L_of(v);
-        const double lam = p.lam_of(v);
-        const real step = (real)(1.0 / Lc), th = (real)(lam / Lc);
+        NoiseLoop nl;
+        if (AUTO) {
+            const size_t ring_bytes = (size_t)WARPS * ring_rows * R * 32 * sizeof(real);
+            nl.start(reinterpret_cast<double *>(smem + beta_bytes + ring_bytes) + (size_t)warp * p.wind);
+        }
+        double lam = AUTO ? nl.lbda : p.lam_of(v);
+        const real step = (real)(1.0 / Lc);
+        real th = (real)(lam / Lc);
         real *Jv = p.out_J + v * (int64_t)p.nb_iter;
         int n_done = 0, ring_pos = 0;
         real res[R];
-        for (int k = 0; k < p.nb_iter; ++k) {
-            vx.forward(res);
-            if (k > 0) {   // cost of the previous iterate: its residual has just been formed
-                const double J = 0.5 * warp_sum((double)vx.partial_sumsq(res)) +
-                                 lam * warp_sum((double)vx.partial_sumabs(vx.w));
-                if (lane == 0 && p.out_J) Jv[k - 1] = (real)J;
-            }
-            real g[R], u[R], pc, pw;
-            vx.adjoint(res, g);
-            if (es) {
-                vx.template update<true, false>(g, step, th, beta[k], u, pc, pw);
-                real *slot = ring + (size_t)ring_pos * R * 32;         // ring_pos = k % nring
-#pragma unroll
-                for (int r = 0; r < R; ++r) slot[r * 32 + lane] = u[r];
-            } else {
-                vx.template update<false, false>(g, step, th, beta[k], u, pc, pw);
-            }
-            n_done = k + 1;
-            if (es && k > p.wind) {
-                // xx = [u_{k-wind+2}, ..., u_k, w_k]; old = mean(first wind-sub), new = mean(last sub)
-                const real inv_old = real(1) / real(p.wind - sub), inv_new = real(1) / real(sub);
-                real so[R], sn[R];
-#pragma unroll
-                for (int r = 0; r < R; ++r) {
-                    so[r] = 0;
-                    sn[r] = vx.w[r];
+        for (;;) {   // one pass (AUTO: one per outer iteration)
+            n_done = 0;
+            ring_pos = 0;
+            for (int k = 0; k < p.nb_iter; ++k) {
+                vx.forward(res);
+                if (!AUTO && k > 0) {   // cost of the previous iterate: its residual has just been formed
+                    const double J = 0.5 * warp_sum((double)vx.partial_sumsq(res)) +
+                                     lam * warp_sum((double)vx.partial_sumabs(vx.w));
+                    if (lane == 0 && p.out_J) Jv[k - 1] = (real)J;
                 }
-                int pos = ring_pos + 1 == nring ? 0 : ring_pos + 1;     // (k - wind + 2) % nring: oldest u
-                for (int m = 0; m < p.wind - 1; ++m) {
-                    const real *slot = ring + (size_t)pos * R * 32;
-                    pos = pos + 1 == nring ? 0 : pos + 1;
-                    const bool is_old = m < p.wind - sub;
+                real g[R], u[R], pc, pw;
+                vx.adjoint(res, g);
+                if (es) {
+                    vx.template update<true, false>(g, step, th, beta[k], u, pc, pw);
+                    real *slot = ring + (size_t)ring_pos * R * 32;         // ring_pos = k % nring
+#pragma unroll
+                    for (int r = 0; r < R; ++r) slot[r * 32 + lane] = u[r];
+                } else {
+                    vx.template update<false, false>(g, step, th, beta[k], u, pc, pw);
+                }
+                n_done = k + 1;
+                if (es && k > p.wind) {
+                    // xx = [u_{k-wind+2}, ..., u_k, w_k]; old = mean(first wind-sub), new = mean(last sub)
+                    const real inv_old = real(1) / real(p.wind - sub), inv_new = real(1) / real(sub);
+                    real so[R], sn[R];
 #pragma unroll
                     for (int r = 0; r < R; ++r) {
-                        const real uu = slot[r * 32 + lane];
-                        if (is_old) so[r] += uu; else sn[r] += uu;
+                        so[r] = 0;
+                        sn[r] = vx.w[r];
                     }
-                }
-                real qn = 0, qd = 0;                  // lane partials in `real`, warp sums in double
+                    int pos = ring_pos + 1 == nring ? 0 : ring_pos + 1;     // (k - wind + 2) % nring: oldest u
+                    for (int m = 0; m < p.wind - 1; ++m) {
+                        const real *slot = ring + (size_t)pos * R * 32;
+                        pos = pos + 1 == nring ? 0 : pos + 1;
+                        const bool is_old = m < p.wind - sub;
 #pragma unroll
-                for (int r = 0; r < R; ++r) {
-                    const real mo = so[r] * inv_old, mn = sn[r] * inv_new;
-                    qn = fma(mn - mo, mn - mo, qn);
-                    qd = fma(mn, mn, qd);
+                        for (int r = 0; r < R; ++r) {
+                            const real uu = slot[r * 32 + lane];
+                            if (is_old) so[r] += uu; else sn[r] += uu;
+                        }
+                    }
+                    real qn = 0, qd = 0;                  // lane partials in `real`, warp sums in double
+#pragma unroll
+                    for (int r = 0; r < R; ++r) {
+                        const real mo = so[r] * inv_old, mn = sn[r] * inv_new;
+                        qn = fma(mn - mo, mn - mo, qn);
+                        qd = fma(mn, mn, qd);
+                    }
+                    const double pn = warp_sum((double)qn);
+                    const double pd = warp_sum((double)qd);
+                    if (sqrt(pn) / (sqrt(pd) + 1.0e-10) < p.tol) break;
                 }
-                const double pn = warp_sum((double)qn);
-                const double pd = warp_sum((double)qd);
-                if (sqrt(pn) / (sqrt(pd) + 1.0e-10) < p.tol) break;
+                if (es) ring_pos = ring_pos + 1 == nring ? 0 : ring_pos + 1;
             }
-            if (es) ring_pos = ring_pos + 1 == nring ? 0 : ring_pos + 1;
-        }
-        vx.forward(res);
-        if (n_done > 0) {
-            const double rr = warp_sum((double)vx.partial_sumsq(res));
-            const double gg = warp_sum((double)vx.partial_sumabs(vx.w));
-            const double J = 0.5 * rr + lam * gg;
-            if (lane == 0) {
-                if (p.out_J) Jv[n_done - 1] = (real)J;
-                if (p.out_r) p.out_r[v] = (real)rr;
-                if (p.out_g) p.out_g[v] = (real)gg;
+            vx.forward(res);
+            if (AUTO) {
+                const double rr = warp_sum((double)vx.partial_sumsq(res));
+                const double gg = warp_sum((double)vx.partial_sumabs(vx.w));
+                if (!nl.pass_done(p, v, rr, gg, lane == 0, lane, 32)) {
+                    lam = nl.lbda;
+                    th = (real)(lam / Lc);
+                    continue;
+                }
+            } else if (n_done > 0) {
+                const double rr = warp_sum((double)vx.partial_sumsq(res));
+                const double gg = warp_sum((double)vx.partial_sumabs(vx.w));
+                const double J = 0.5 * rr + lam * gg;
+                if (lane == 0) {
+                    if (p.out_J) Jv[n_done - 1] = (real)J;
+                    if (p.out_r) p.out_r[v] = (real)rr;
+                    if (p.out_g) p.out_g[v] = (real)gg;
+                }
             }
+            break;
         }
         real y[R], z[R];
         vx.load_y(yv, T, y);
@@ -357,7 +378,7 @@ fast_deconv_kernel(DeconvArgs<real> p, int ring_rows) {
         vx.store(p.out_x + v * T, y, T);
         vx.store(p.out_z + v * T, z, T);
         vx.store(p.out_dz + v * T, vx.w, T);
-        if (lane == 0) p.out_niter[v] = n_done;
+        if (lane == 0 && !AUTO) p.out_niter[v] = n_done;
         __syncwarp();
     }
 }
@@ -525,13 +546,14 @@ bool fast_shape_ok(int T, int K) {
 }
 
 // FAST_NO_MATCH when the ring does not fit: the generic kernel decides
-template <typename real, int R, int KMAX, bool CIRC, int WARPS, int MINB>
+template <typename real, int R, int KMAX, bool CIRC, int WARPS, int MINB, bool AUTO = false>
 int fast_deconv_launch(const DeconvArgs<real> &a, cudaStream_t stream) {
     const bool es = a.early_stopping && a.wind >= 2;
     const int ring_rows = es ? a.wind - 1 : 0;
     const size_t beta_bytes = ((size_t)a.nb_iter * sizeof(real) + 15) & ~(size_t)15;
-    const size_t smem = beta_bytes + (size_t)WARPS * ring_rows * R * 32 * sizeof(real);
-    return launch_persistent(fast_deconv_kernel<real, R, KMAX, CIRC, WARPS, MINB>, WARPS * 32, smem, WARPS,
+    const size_t smem = beta_bytes + (size_t)WARPS * ring_rows * R * 32 * sizeof(real) +
+                        (AUTO ? (size_t)WARPS * a.wind * sizeof(double) : 0);
+    return launch_persistent(fast_deconv_kernel<real, R, KMAX, CIRC, WARPS, MINB, AUTO>, WARPS * 32, smem, WARPS,
                              a.V, nullptr, stream, a, ring_rows);
 }
 
@@ -547,7 +569,8 @@ template <typename real, int R, int KMAX, bool CIRC, int WARPS, int MINB>
 constexpr Variant<real> warp_variant() {
     return {TIER_WARP, 32, R, KMAX, 0, CIRC, fast_shape_ok<real, R, KMAX, CIRC>,
             fast_bd_launch<real, R, KMAX, CIRC, WARPS, MINB>, nullptr,
-            fast_deconv_launch<real, R, KMAX, CIRC, WARPS, MINB>, nullptr};
+            fast_deconv_launch<real, R, KMAX, CIRC, WARPS, MINB>, nullptr,
+            fast_deconv_launch<real, R, KMAX, CIRC, WARPS, MINB, true>};
 }
 
 }  // namespace pb

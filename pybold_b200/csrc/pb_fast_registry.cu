@@ -65,15 +65,17 @@ static int bd_dispatch(const BdArgs<real> &a, cudaStream_t s) {
 
 template <typename real>
 static int deconv_dispatch(const DeconvArgs<real> &a, cudaStream_t s) {
+    // deconv(lbda=None) (nb_outer > 0) takes the same rows through their deconv_auto entry points
+    const auto need = a.nb_outer > 0 ? &Variant<real>::deconv_auto : &Variant<real>::deconv;
     // tier 0 is the group rows only (the CTA rows have no deconv); early stopping runs there only when a
     // work-queue counter was provided (a.queue)
     if ((!(a.early_stopping && a.wind >= 2) || a.queue) && !tier0_disabled())
-        if (const Variant<real> *v = pick<real>(TIER_GROUP_CTA, a.T, a.K, &Variant<real>::deconv)) {
-            const int rc = v->deconv(a, s);
+        if (const Variant<real> *v = pick<real>(TIER_GROUP_CTA, a.T, a.K, need)) {
+            const int rc = (v->*need)(a, s);
             if (rc != FAST_NO_MATCH) return rc;
         }
-    const Variant<real> *v = pick<real>(TIER_WARP, a.T, a.K, &Variant<real>::deconv);
-    return v ? v->deconv(a, s) : FAST_NO_MATCH;
+    const Variant<real> *v = pick<real>(TIER_WARP, a.T, a.K, need);
+    return v ? (v->*need)(a, s) : FAST_NO_MATCH;
 }
 
 // the queries describe bd without early stopping and ignore PB_DISABLE_GROUP

@@ -37,6 +37,8 @@ struct Variant {
     int (*bd_es)(const BdArgs<real> &, cudaStream_t);  // bd with early stopping (Q6 / Q7)
     int (*deconv)(const DeconvArgs<real> &, cudaStream_t);
     int (*wave)(int nb_iter);
+    // deconv(lbda=None): DeconvArgs::nb_outer > 0, the noise loop inside the kernel (pb_noise_loop.cuh)
+    int (*deconv_auto)(const DeconvArgs<real> &, cudaStream_t);
 };
 
 // Launches a persistent kernel of `threads` threads and `smem` bytes of dynamic shared memory per

@@ -845,8 +845,12 @@ fast_deconvg_kernel(DeconvArgs<real> p) {
 // voxel only involves its own G lanes, in the same lane order.
 // Ring of the past u's (Q5 window): [slot][lane][RP] in shared memory, every lane reads and writes its
 // own 16-byte aligned block with vector accesses (RP / 4 odd: conflict free).
+// AUTO: deconv(lbda=None).  A group keeps its voxel through every outer iteration of the noise loop
+// (pb_noise_loop.cuh): where an inner pass ends, it updates lambda and starts the next pass in the same turn
+// from the residual just formed, so only the final pass of a voxel costs the neighbour group a turn.  The
+// windows of alphas (wind doubles per group) follow the rings in shared memory.
 // ------------------------------------------------------------------------------------------------
-template <typename real, int R, int KMAX, int G, int TAIL, int WARPS, int MINB>
+template <typename real, int R, int KMAX, int G, int TAIL, int WARPS, int MINB, bool AUTO = false>
 __global__ void __launch_bounds__(WARPS * 32, MINB)
 fast_deconvg_es_kernel(DeconvArgs<real> p, int ring_rows) {
     using GV = GroupVoxel<real, R, KMAX, G, TAIL, 0>;
@@ -876,6 +880,7 @@ fast_deconvg_es_kernel(DeconvArgs<real> p, int ring_rows) {
     bool active = false, want = true;
     double lam = 0.0;
     real step = 0, th = 0;
+    NoiseLoop nl;
     for (;;) {
         if (__any_sync(PB_FULL, want)) {
             unsigned int idx = 0xffffffffu;
@@ -900,7 +905,14 @@ fast_deconvg_es_kernel(DeconvArgs<real> p, int ring_rows) {
                         vx.w[r] = (p.w0 && i < T) ? p.w0[v * T + i] : real(0);
                     }
                     const double Lc = p.L_of(v);
-                    lam = p.lam_of(v);
+                    if constexpr (AUTO) {
+                        nl.start(reinterpret_cast<double *>(smem + beta_bytes + (size_t)WARPS * ring_rows * 32 * RP *
+                                                                                    sizeof(real)) +
+                                 (size_t)(warp * (32 / G) + lane / G) * p.wind);
+                        lam = nl.lbda;
+                    } else {
+                        lam = p.lam_of(v);
+                    }
                     step = (real)(1.0 / Lc);
                     th = (real)(lam / Lc);
                     k = 0;
@@ -966,13 +978,26 @@ fast_deconvg_es_kernel(DeconvArgs<real> p, int ring_rows) {
             const double rhs = p.tol * (sqrt_refined(pd) + 1.0e-10);
             stop = es_on && k - 1 > p.wind && pn < rhs * rhs;
         }
-        {   // cost of the previous iterate: its residual has just been formed.  For a closing voxel k is the
-            // number of iterations done and this is its last cost.
+        if constexpr (!AUTO) {   // cost of the previous iterate: its residual has just been formed.  For a
+                                 // closing voxel k is the number of iterations done and this is its last cost.
             const double J = 0.5 * (double)Seg<real, G>::sum(vx.partial_sumsq(res)) +
                              lam * (double)Seg<real, G>::sum(vx.partial_sumabs(vx.w));
             if (active && q == 0 && k > 0 && p.out_J) Jv[k - 1] = (real)J;
         }
-        const bool closing = active && k > 0 && (stop || k == p.nb_iter);
+        bool closing = active && k > 0 && (stop || k == p.nb_iter);
+        if constexpr (AUTO) if (__any_sync(PB_FULL, closing)) {
+            // an inner pass has ended; unless it was the voxel's final pass, the next one starts here: the
+            // residual just formed is that of its starting iterate (iteration 0 below)
+            const double rr = (double)Seg<real, G>::sum(vx.partial_sumsq(res));
+            const double gg = (double)Seg<real, G>::sum(vx.partial_sumabs(vx.w));
+            if (closing && !nl.pass_done(p, v, rr, gg, q == 0, q, G)) {
+                closing = false;
+                lam = nl.lbda;
+                th = (real)(lam / p.L_of(v));
+                k = 0;
+                ring_pos = 0;
+            }
+        }
         if (__any_sync(PB_FULL, closing)) {
             // The iterate in registers is final for this voxel and the residual just formed is its own: store
             // it and hand the group back to the queue; the neighbour group loses this turn's forward pass
@@ -989,7 +1014,7 @@ fast_deconvg_es_kernel(DeconvArgs<real> p, int ring_rows) {
                 gg = (double)Seg<real, G>::sum(vx.partial_sumabs(vx.w));
             }
             if (closing) {
-                if (q == 0) p.out_niter[v] = k;
+                if constexpr (!AUTO) if (q == 0) p.out_niter[v] = k;
                 if (q == 0 && p.out_r) p.out_r[v] = (real)rr;
                 if (q == 0 && p.out_g) p.out_g[v] = (real)gg;
                 real y[R];
@@ -1031,16 +1056,18 @@ fast_deconvg_es_kernel(DeconvArgs<real> p, int ring_rows) {
     }
 }
 
-template <typename real, int R, int KMAX, int G, int TAIL, int WARPS, int MINB>
+// AUTO (deconv(lbda=None)) always runs the early-stopping kernel: its launcher sets wind >= 2
+template <typename real, int R, int KMAX, int G, int TAIL, int WARPS, int MINB, bool AUTO = false>
 int fast_deconvg_launch(const DeconvArgs<real> &a, cudaStream_t stream) {
     constexpr int VPW = 32 / G;
     const size_t beta_bytes = ((size_t)a.nb_iter * sizeof(real) + 15) & ~(size_t)15;
-    if (a.early_stopping && a.wind >= 2) {
+    if (AUTO || (a.early_stopping && a.wind >= 2)) {
         if (!a.queue) return FAST_NO_MATCH;
         const int ring_rows = a.wind - 1;
-        const size_t smem = beta_bytes + (size_t)WARPS * ring_rows * 32 * fastg_block_floats<R>() * sizeof(real);
-        return launch_persistent(fast_deconvg_es_kernel<real, R, KMAX, G, TAIL, WARPS, MINB>, WARPS * 32, smem,
-                                 WARPS * VPW, a.V, a.queue, stream, a, ring_rows);
+        const size_t smem = beta_bytes + (size_t)WARPS * ring_rows * 32 * fastg_block_floats<R>() * sizeof(real) +
+                            (AUTO ? (size_t)WARPS * VPW * a.wind * sizeof(double) : 0);
+        return launch_persistent(fast_deconvg_es_kernel<real, R, KMAX, G, TAIL, WARPS, MINB, AUTO>, WARPS * 32,
+                                 smem, WARPS * VPW, a.V, a.queue, stream, a, ring_rows);
     }
     return launch_persistent(fast_deconvg_kernel<real, R, KMAX, G, TAIL, WARPS, MINB>, WARPS * 32, beta_bytes,
                              WARPS * VPW, a.V, nullptr, stream, a);
@@ -1069,7 +1096,8 @@ constexpr Variant<real> group_variant() {
             fast_bdg_launch<real, R, KMAX, G, TAIL, WARPS, MINB>,
             fast_bdg_launch<real, R, KMAX, G, TAIL, WARPS, MINB, 0, 0, true>,
             fast_deconvg_launch<real, R, KMAX, G, TAIL, WARPS, MINB>,
-            fast_bdg_wave<real, R, KMAX, G, TAIL, WARPS, MINB>};
+            fast_bdg_wave<real, R, KMAX, G, TAIL, WARPS, MINB>,
+            fast_deconvg_launch<real, R, KMAX, G, TAIL, WARPS, MINB, true>};
 }
 
 }  // namespace pb

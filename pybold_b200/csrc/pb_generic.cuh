@@ -8,6 +8,7 @@
 // :281-382 (bd); quirks Q1-Q9 of SURVEY.md section 8 are reproduced on purpose.
 #pragma once
 #include "pb_device.cuh"
+#include "pb_noise_loop.cuh"
 
 namespace pb {
 
@@ -232,6 +233,15 @@ struct DeconvArgs {
     // optional mask: problems with active[v] == 0 are skipped, their outputs stay untouched (the outer loop
     // of deconv(lbda=None) keeps calling with fewer and fewer live voxels); out_J may be null (no cost trace)
     const unsigned char *active = nullptr;
+    // deconv(lbda=None) (nb_outer > 0, kernels instantiated with AUTO): lambda follows the noise level
+    // sigma[v * sigma_stride] through at most nb_outer outer iterations (pb_noise_loop.cuh) instead of coming from
+    // lbda; nb_iter stays the inner count.  out_J, out_R, out_G are [V, nb_outer] (NaN past the voxel's outer
+    // count), out_lbda [V] the last lambda, out_nouter [V] the outer count; each may be null.
+    const real *sigma = nullptr;
+    int64_t sigma_stride = 0;
+    int nb_outer = 0;
+    real *out_R = nullptr, *out_G = nullptr, *out_lbda = nullptr;
+    int32_t *out_nouter = nullptr;
     __device__ __forceinline__ bool is_active(int64_t v) const { return !active || active[v] != 0; }
     __device__ __forceinline__ int64_t voxel_of(int64_t v) const { return y_mod ? v % y_mod : v; }
     __device__ __forceinline__ const real *y_row(int64_t v) const { return y + voxel_of(v) * T; }
@@ -243,7 +253,9 @@ struct DeconvArgs {
     }
 };
 
-template <typename real>
+// AUTO: deconv(lbda=None), one inner pass per outer iteration of the noise loop, then the final pass; the
+// window of alphas lives in the warp's scratch doubles
+template <typename real, bool AUTO = false>
 __global__ void generic_deconv_kernel(DeconvArgs<real> p, GenLayout lay) {
     extern __shared__ __align__(16) unsigned char smem[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = blockDim.x >> 5;
@@ -268,8 +280,11 @@ __global__ void generic_deconv_kernel(DeconvArgs<real> p, GenLayout lay) {
         for (int a = lane; a < K; a += 32) g.hr[a] = hv[a];
         __syncwarp();
         const double Lc = p.L_of(v);
-        const double lam = p.lam_of(v);
-        const real step = (real)(1.0 / Lc), th = (real)(lam / Lc);
+        NoiseLoop nl;
+        if (AUTO) nl.start(scratch);
+        double lam = AUTO ? nl.lbda : p.lam_of(v);
+        const real step = (real)(1.0 / Lc);
+        real th = (real)(lam / Lc);
         real *Jv = p.out_J + v * (int64_t)p.nb_iter;
         // ring row r: shared memory, or (long series in double) this voxel's output rows until the final store;
         // a lane only ever reads back the elements it wrote itself
@@ -279,54 +294,64 @@ __global__ void generic_deconv_kernel(DeconvArgs<real> p, GenLayout lay) {
             return (o == 0 ? p.out_x : (o == 1 ? p.out_z : p.out_dz)) + v * T;
         };
         int n_done = 0;
-        for (int k = 0; k < p.nb_iter; ++k) {
-            g.forward();
-            if (k > 0) {
-                const double J = 0.5 * g.sumsq(g.bs) + lam * g.sumabs(g.ws);
-                if (lane == 0 && p.out_J) Jv[k - 1] = (real)J;
-            }
-            g.adjoint();
-            double d0, d1;
-            real *uslot = es ? ring_row(k % nring) : nullptr;
-            g.update(step, th, beta[k], uslot, false, d0, d1);
-            n_done = k + 1;
-            if (es && k > p.wind) {
-                // xx = [u_{k-wind+2}, ..., u_k, w_k]; old = mean(first wind-sub), new = mean(last sub)
-                double pn = 0.0, pd = 0.0;
-                const real inv_old = real(1) / real(p.wind - sub), inv_new = real(1) / real(sub);
-                for (int i = lane; i < T; i += 32) {
-                    real so = 0, sn = 0;
-                    for (int m = 0; m < p.wind - 1; ++m) {
-                        const int j = k - p.wind + 2 + m;
-                        const real u = ring_row(j % nring)[i];
-                        if (m < p.wind - sub) so += u; else sn += u;
-                    }
-                    sn += g.ws[i];
-                    const real mo = so * inv_old, mn = sn * inv_new;
-                    pn += (double)(mn - mo) * (double)(mn - mo);
-                    pd += (double)mn * (double)mn;
+        for (;;) {   // one pass (AUTO: one per outer iteration)
+            n_done = 0;
+            for (int k = 0; k < p.nb_iter; ++k) {
+                g.forward();
+                if (!AUTO && k > 0) {
+                    const double J = 0.5 * g.sumsq(g.bs) + lam * g.sumabs(g.ws);
+                    if (lane == 0 && p.out_J) Jv[k - 1] = (real)J;
                 }
-                pn = warp_sum(pn);
-                pd = warp_sum(pd);
-                if (sqrt(pn) / (sqrt(pd) + 1.0e-10) < p.tol) break;
+                g.adjoint();
+                double d0, d1;
+                real *uslot = es ? ring_row(k % nring) : nullptr;
+                g.update(step, th, beta[k], uslot, false, d0, d1);
+                n_done = k + 1;
+                if (es && k > p.wind) {
+                    // xx = [u_{k-wind+2}, ..., u_k, w_k]; old = mean(first wind-sub), new = mean(last sub)
+                    double pn = 0.0, pd = 0.0;
+                    const real inv_old = real(1) / real(p.wind - sub), inv_new = real(1) / real(sub);
+                    for (int i = lane; i < T; i += 32) {
+                        real so = 0, sn = 0;
+                        for (int m = 0; m < p.wind - 1; ++m) {
+                            const int j = k - p.wind + 2 + m;
+                            const real u = ring_row(j % nring)[i];
+                            if (m < p.wind - sub) so += u; else sn += u;
+                        }
+                        sn += g.ws[i];
+                        const real mo = so * inv_old, mn = sn * inv_new;
+                        pn += (double)(mn - mo) * (double)(mn - mo);
+                        pd += (double)mn * (double)mn;
+                    }
+                    pn = warp_sum(pn);
+                    pd = warp_sum(pd);
+                    if (sqrt(pn) / (sqrt(pd) + 1.0e-10) < p.tol) break;
+                }
             }
-        }
-        g.forward();
-        if (n_done > 0) {
-            const double rr = g.sumsq(g.bs), gg = g.sumabs(g.ws);
-            const double J = 0.5 * rr + lam * gg;
-            if (lane == 0) {
-                if (p.out_J) Jv[n_done - 1] = (real)J;
-                if (p.out_r) p.out_r[v] = (real)rr;
-                if (p.out_g) p.out_g[v] = (real)gg;
+            g.forward();
+            if (AUTO) {
+                if (!nl.pass_done(p, v, g.sumsq(g.bs), g.sumabs(g.ws), lane == 0, lane, 32)) {
+                    lam = nl.lbda;
+                    th = (real)(lam / Lc);
+                    continue;
+                }
+            } else if (n_done > 0) {
+                const double rr = g.sumsq(g.bs), gg = g.sumabs(g.ws);
+                const double J = 0.5 * rr + lam * gg;
+                if (lane == 0) {
+                    if (p.out_J) Jv[n_done - 1] = (real)J;
+                    if (p.out_r) p.out_r[v] = (real)rr;
+                    if (p.out_g) p.out_g[v] = (real)gg;
+                }
             }
+            break;
         }
         for (int i = lane; i < T; i += 32) {
             p.out_x[v * T + i] = g.bs[i] + g.ys[i];
             p.out_z[v * T + i] = g.as[i];
             p.out_dz[v * T + i] = g.ws[i];
         }
-        if (lane == 0) p.out_niter[v] = n_done;
+        if (lane == 0 && !AUTO) p.out_niter[v] = n_done;
         __syncwarp();
     }
 }

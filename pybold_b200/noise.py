@@ -1,8 +1,8 @@
 """``deconv(lbda=None)``: noise-constrained regularisation (pybold/bold_signal.py:99-214).
 
-Row N1 of SURVEY.md 8(f).  The inner prox-gradient loops run in the persistent ``pb_deconv``
-kernel (warm-started through ``w0``); the outer loop -- one scalar update of alpha / lambda per
-voxel and per outer iteration -- is driven from the host with O(V) tensor arithmetic.
+Row N1 of SURVEY.md 8(f).  The whole loop -- inner prox-gradient passes and the scalar alpha / lambda update of
+every outer iteration -- runs per voxel inside the persistent deconv kernels (``pb_deconv_auto``,
+csrc/pb_noise_loop.cuh): one launch per call.
 
 The noise level sigma is the MAD of the level-1 db3 detail coefficients in the reference
 (pybold/utils.py:10-25, PyWavelets); here one kernel (``pb_mad_daub_noise_est_*``).  The loop itself
@@ -65,16 +65,14 @@ def mad_daub_noise_est(x, c=0.6744):
 
 def deconv_auto_lbda(y_in, yb, one_d, hrf, lipschitz, sigma, early_stopping, tol, wind,
                      nb_iter, nb_sub_iter):
-    """Outer loop of ``deconv(lbda=None)`` (pybold/bold_signal.py:99-214) for a batch.
-
-    Every outer iteration is two launches: the inner prox-gradient loops of the voxels that are still
-    running (``pb_deconv_masked``: warm start, no cost trace, finished voxels skipped) and the fused
-    residual / alpha / lambda update (``pb_noise_step``).  The alpha-window stop of every voxel is
-    evaluated on the device; the host only looks at "is anything still running" every few iterations.
+    """``deconv(lbda=None)`` (pybold/bold_signal.py:99-214) for a batch: the noise level (given, or estimated
+    like the reference does), then the whole noise-constrained loop of every voxel in ONE persistent kernel
+    launch (:func:`~pybold_b200.bold_signal.deconv_auto_batch`): outer iterations, alpha / lambda updates, the
+    alpha-window stop and the final inner pass all run on the device, nothing goes through the host between
+    outer iterations.  Returns the reference's tuple (x, z, diff_z, J, R, G): lists for one voxel, rows cut at
+    the largest outer count (NaN past each voxel's own) for a batch.
     """
-    from .bold_signal import deconv_batch
-    V, T = yb.shape
-    dtype, dev = yb.dtype, yb.device
+    from .bold_signal import deconv_auto_batch
     if sigma is None:
         # bold_signal.py:103.  The wavelet convention of this estimate could not be compared with PyWavelets
         # itself (see mad_daub_noise_est): say so once, `sigma=` makes the run independent of it
@@ -86,56 +84,13 @@ def deconv_auto_lbda(y_in, yb, one_d, hrf, lipschitz, sigma, early_stopping, tol
                           "a run that does not depend on it", UserWarning, stacklevel=3)
             _warned_sigma = True
         sigma = mad_daub_noise_est(yb)
-    sigma = torch.as_tensor(sigma, dtype=dtype, device=dev).reshape(-1).expand(V).clone()
-    alpha = torch.ones(V, dtype=dtype, device=dev)                  # bold_signal.py:104
-    lbda = 1.0 / (2.0 * alpha)
-    mu = 1.0e-4
-    w = torch.zeros_like(yb)
-    x = torch.zeros_like(yb)
-    z = torch.zeros_like(yb)
-    scratch = (torch.empty_like(yb), torch.empty_like(yb), torch.empty_like(yb),
-               torch.zeros(V, dtype=torch.int32, device=dev))
-    active = torch.ones(V, dtype=torch.uint8, device=dev)
-    n_outer = torch.full((V,), nb_iter, dtype=torch.int64, device=dev)   # outer iterations each voxel runs
-    sub = int(wind / 2)
-    hist = []
-    J = torch.full((V, nb_iter), float("nan"), dtype=dtype, device=dev)
-    R = torch.full((V, nb_iter), float("nan"), dtype=dtype, device=dev)
-    G = torch.full((V, nb_iter), float("nan"), dtype=dtype, device=dev)
-    step = _lib.fn("pb_noise_step", dtype)
-    check_every = 1 if V == 1 else 4
-    for i in range(nb_iter):
-        x_n, z_n, w_n, _, _ = deconv_batch(yb, hrf, lbda, lipschitz, w, early_stopping, tol, wind,
-                                           nb_sub_iter, active=active, out=scratch, trace=False)
-        r = torch.empty(V, dtype=dtype, device=dev)
-        g = torch.empty(V, dtype=dtype, device=dev)
-        # bold_signal.py:139-145: keep the result of the active voxels, r, g, alpha and lambda updates
-        with torch.cuda.device(dev):
-            rc = step(ptr(x_n), ptr(z_n), ptr(w_n), ptr(yb), ptr(sigma), ptr(active), mu, ptr(x), ptr(z), ptr(w),
-                      ptr(alpha), ptr(lbda), ptr(r), ptr(g), V, T, stream_ptr())
-        _lib.check(rc, "pb_noise_step")
-        hist.append(alpha.clone())
-        if len(hist) > wind:
-            hist = hist[1:]
-        live = active.bool()
-        R[:, i] = torch.where(live, r, R[:, i])
-        G[:, i] = torch.where(live, g, G[:, i])
-        J[:, i] = torch.where(live, 0.5 * r + lbda * g, J[:, i])
-        if early_stopping and i > wind and sub > 0:                 # bold_signal.py:164-178
-            old_it = torch.stack(hist[:-sub]).mean(dim=0)
-            new_it = torch.stack(hist[-sub:]).mean(dim=0)
-            stop = ((new_it - old_it).abs() / new_it.abs() < tol) & live
-            n_outer = torch.where(stop, torch.full_like(n_outer, i + 1), n_outer)
-            active = active & (~stop).to(torch.uint8)
-            if (i % check_every == 0 or i == nb_iter - 1) and not bool(active.any()):
-                break
-    # bold_signal.py:180-212: last deconvolution with the final lambda, every voxel
-    x, z, w, _, _ = deconv_batch(yb, hrf, lbda, lipschitz, w, early_stopping, tol, wind, nb_sub_iter, trace=False)
+    out = deconv_auto_batch(yb, hrf, sigma, lipschitz, nb_iter, nb_sub_iter, early_stopping, tol, wind)
+    x, z, w, J, R, G = (out[k] for k in ("x", "z", "diff_z", "J", "R", "G"))
     if one_d:
-        n = int(n_outer[0])
+        n = int(out["n_outer"][0])
         conv = lambda t: like_input(t[0], y_in)  # noqa: E731
         return (conv(x), conv(z), conv(w), [float(v) for v in J[0, :n]], [float(v) for v in R[0, :n]],
                 [float(v) for v in G[0, :n]])
-    n_max = int(n_outer.max())
+    n_max = int(out["n_outer"].max())
     conv = lambda t: like_input(t, y_in)  # noqa: E731
     return conv(x), conv(z), conv(w), conv(J[:, :n_max]), conv(R[:, :n_max]), conv(G[:, :n_max])

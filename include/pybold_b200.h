@@ -50,6 +50,14 @@ int pb_solver_variant(int T, int K, int is_f64);
  * shape runs on a kernel without that notion).  Hosts that stream a large batch in chunks should
  * cut it at multiples of this number. */
 int pb_bd_wave_voxels(int T, int K, int is_f64, int nb_iter);
+/* Which kernel a deconvolution with this shape runs on the current device: pb_deconv / pb_deconv_masked /
+ * pb_deconv_lbda_path(_ex) with (nb_iter, early_stopping, wind), or pb_deconv_auto (is_auto != 0, nb_iter the
+ * inner count nb_sub_iter).  Returns the variant in the encoding of pb_solver_variant (0 = generic kernel) and
+ * the family in *family: 0 generic, 1 group, 2 warp per voxel, 3 CTA per voxel (a one-warp CTA and a warp
+ * variant can share an id).  The choice is the launch's own, shared-memory and occupancy checks included.
+ * Negative PB_ERR_* on bad arguments, shapes beyond the limits, or PB_ERR_NO_DEVICE. */
+int pb_deconv_variant(int T, int K, int is_f64, int nb_iter, int early_stopping, int wind, int is_auto,
+                      int *family);
 
 /* ---- A1: DiscretInteg.op / .adj (pybold/linear.py:15-28, :30-43) -------------------- */
 int pb_integ_op_f32(const float *x, float *out, int64_t V, int T, pb_stream_t stream);

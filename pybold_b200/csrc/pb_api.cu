@@ -374,11 +374,12 @@ int run_toeplitz(const real *k, int klen, real *out, int64_t dim_out, int64_t di
     return last_error();
 }
 
-// the register-tiled variant the picker chooses, else the generic kernel; a.nb_outer > 0 selects the
-// deconv(lbda=None) instances
+// the register-tiled variant the dispatch chooses (pb_fast_registry.cu), else the generic kernel; a.nb_outer > 0
+// selects the deconv(lbda=None) instances.  V == 0 launches nothing: *id / *family report the kernel a launch
+// would run (pb_deconv_variant).
 template <typename real>
-int launch_deconv(const pb::DeconvArgs<real> &a, pb_stream_t stream) {
-    int rc = pb::fast_deconv_dispatch(a, (cudaStream_t)stream);
+int launch_deconv(const pb::DeconvArgs<real> &a, pb_stream_t stream, int *id = nullptr, int *family = nullptr) {
+    int rc = pb::fast_deconv_dispatch(a, (cudaStream_t)stream, id, family);
     if (rc != pb::FAST_NO_MATCH) return rc;
     DeviceInfo d = device_info();
     if (d.err) return d.err;
@@ -391,6 +392,7 @@ int launch_deconv(const pb::DeconvArgs<real> &a, pb_stream_t stream) {
     }
     LaunchPlan p = plan_launch(d, beta_bytes, lay.warp_bytes(sizeof(real)), a.V, 8);
     if (!p.warps) return PB_ERR_UNSUPPORTED;
+    if (a.V == 0) return PB_OK;
     auto go = [&](auto kern) {
         int e = set_smem(kern, p.smem);
         if (e) return e;
@@ -398,6 +400,19 @@ int launch_deconv(const pb::DeconvArgs<real> &a, pb_stream_t stream) {
         return last_error();
     };
     return a.nb_outer > 0 ? go(pb::generic_deconv_kernel<real, true>) : go(pb::generic_deconv_kernel<real, false>);
+}
+
+// What the deconv entry points set before the dispatch: for deconv(lbda=None) without early stopping (or with
+// wind < 2, which has no window) wind = 2 -- the window length does not matter then, and 2 keeps the group kernel's
+// ring of u's one row long -- and the work-queue counter of the early-stopping and deconv(lbda=None) kernels, taken
+// from `queue` (queue_slot for a launch).
+template <typename real>
+void set_routing(pb::DeconvArgs<real> &a, unsigned int *(*queue)()) {
+    if (a.nb_outer > 0 && !(a.early_stopping && a.wind >= 2)) {
+        a.early_stopping = 0;
+        a.wind = 2;
+    }
+    if (a.nb_outer > 0 || (a.early_stopping && a.wind >= 2)) a.queue = queue();
 }
 
 template <typename real>
@@ -408,7 +423,7 @@ int run_deconv(pb::DeconvArgs<real> a, pb_stream_t stream) {
         return PB_ERR_INVALID_ARG;
     if (a.T > PB_MAX_T || a.K > PB_MAX_K || a.nb_iter > PB_MAX_ITER) return PB_ERR_UNSUPPORTED;
     if (a.V == 0) return PB_OK;
-    if (a.early_stopping && a.wind >= 2) a.queue = queue_slot();
+    set_routing(a, queue_slot);
     return launch_deconv(a, stream);
 }
 
@@ -422,14 +437,36 @@ int run_deconv_auto(pb::DeconvArgs<real> a, pb_stream_t stream) {
         a.sigma_stride < 0)
         return PB_ERR_INVALID_ARG;
     if (a.T > PB_MAX_T || a.K > PB_MAX_K || a.nb_iter > PB_MAX_ITER) return PB_ERR_UNSUPPORTED;
-    // without early stopping (or with wind < 2, which has no window) the window length does not matter; 2 keeps
-    // the group kernel's ring of u's one row long
-    if (!(a.early_stopping && a.wind >= 2)) {
-        a.early_stopping = 0;
-        a.wind = 2;
-    }
-    a.queue = queue_slot();
+    set_routing(a, queue_slot);
     return launch_deconv(a, stream);
+}
+
+// pb_deconv_variant: the routing of a deconv call with V = 0 (nothing is launched)
+template <typename real>
+int deconv_variant(int T, int K, int nb_iter, int early_stopping, int wind, int is_auto, int *family) {
+    if (!family || T <= 0 || K <= 0 || nb_iter < 1 || wind < 0) return PB_ERR_INVALID_ARG;
+    if (T > PB_MAX_T || K > PB_MAX_K || nb_iter > PB_MAX_ITER) return PB_ERR_UNSUPPORTED;
+    pb::DeconvArgs<real> a{};
+    a.T = T;
+    a.K = K;
+    a.nb_iter = nb_iter;
+    a.early_stopping = early_stopping;
+    a.wind = wind;
+    a.nb_outer = is_auto ? 1 : 0;
+    a.V = 0;
+    // a placeholder counter: the routing sees a work queue exactly when a call would, and a launch with V = 0
+    // neither zeroes nor reads it, so the query takes no slot of the pool
+    set_routing(a, +[]() -> unsigned int * {
+        static unsigned int placeholder;
+        return &placeholder;
+    });
+    int id = 0;
+    const int rc = launch_deconv(a, nullptr, &id, family);
+    if (rc > 0) {               // a CUDA error
+        cudaGetLastError();
+        return PB_ERR_NO_DEVICE;
+    }
+    return rc < 0 ? rc : id;
 }
 
 template <typename real>
@@ -630,6 +667,12 @@ const char *pb_error_string(int code) {
 }
 
 int pb_solver_variant(int T, int K, int is_f64) { return pb::fast_variant_id(T, K, is_f64 != 0); }
+
+int pb_deconv_variant(int T, int K, int is_f64, int nb_iter, int early_stopping, int wind, int is_auto,
+                      int *family) {
+    return is_f64 ? deconv_variant<double>(T, K, nb_iter, early_stopping, wind, is_auto, family)
+                  : deconv_variant<float>(T, K, nb_iter, early_stopping, wind, is_auto, family);
+}
 
 int pb_bd_wave_voxels(int T, int K, int is_f64, int nb_iter) {
     if (T <= 0 || K <= 0 || nb_iter < 1) return 0;

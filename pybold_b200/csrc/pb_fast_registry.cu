@@ -25,14 +25,23 @@ static long cost(const Variant<real> &v) {
     return c;
 }
 
-// cheapest variant of `tier` that serves (T, K) and has the entry point `need`; ties go to the first
-// row (strict <), so CTA rows win ties against group rows
+// the family of a row: warp tier, or tier 0 with fewer lanes than a warp (group) or a whole number of warps (CTA)
+template <typename real>
+static int family(const Variant<real> &v) {
+    return v.tier == TIER_WARP ? FAMILY_WARP : (v.lanes < 32 ? FAMILY_GROUP : FAMILY_CTA);
+}
+
+constexpr unsigned bit(int family) { return 1u << family; }
+constexpr unsigned TIER0 = bit(FAMILY_GROUP) | bit(FAMILY_CTA);
+
+// cheapest variant of the families in the mask `families` that serves (T, K) and has the entry point `need`;
+// ties go to the first row (strict <), so CTA rows win ties against group rows
 template <typename real, typename Fn>
-static const Variant<real> *pick(int tier, int T, int K, Fn Variant<real>::*need) {
+static const Variant<real> *pick(unsigned families, int T, int K, Fn Variant<real>::*need) {
     const Variant<real> *best = nullptr;
     long best_cost = 0;
     for (const Variant<real> *v : variants(real())) {
-        if (v->tier != tier || !(v->*need) || !v->ok(T, K)) continue;
+        if (!(families & bit(family(*v))) || !(v->*need) || !v->ok(T, K)) continue;
         const long c = cost(*v);
         if (!best || c < best_cost) {
             best = v;
@@ -55,45 +64,62 @@ static int bd_dispatch(const BdArgs<real> &a, cudaStream_t s) {
     // early stopping: only the rows with bd_es (the group variants) are candidates
     const auto need = a.early_stopping ? &Variant<real>::bd_es : &Variant<real>::bd;
     if (!tier0_disabled())
-        if (const Variant<real> *v = pick<real>(TIER_GROUP_CTA, a.T, a.K, need)) {
+        if (const Variant<real> *v = pick<real>(TIER0, a.T, a.K, need)) {
             const int rc = (v->*need)(a, s);
             if (rc != FAST_NO_MATCH) return rc;
         }
-    const Variant<real> *v = pick<real>(TIER_WARP, a.T, a.K, &Variant<real>::bd);
+    const Variant<real> *v = pick<real>(bit(FAMILY_WARP), a.T, a.K, &Variant<real>::bd);
     return v ? v->bd(a, s) : FAST_NO_MATCH;
 }
 
 template <typename real>
-static int deconv_dispatch(const DeconvArgs<real> &a, cudaStream_t s) {
+static int encode(const Variant<real> &v) { return v.lanes * 1000000 + v.R * 1000 + v.KMAX; }
+
+// Routing of every deconv call (fixed lambda, early stopping, lbda=None, path, masked): group rows, then warp rows,
+// then CTA rows, then (launch_deconv) the generic kernel.  A step is taken when the one before has no variant for
+// (T, K) or its launch returns FAST_NO_MATCH (shared memory or occupancy).  The group rows run early stopping only
+// with a work-queue counter (a.queue).  V == 0 launches nothing and reports the same choice.
+template <typename real>
+static int deconv_dispatch(const DeconvArgs<real> &a, cudaStream_t s, int *id, int *fam_out) {
     // deconv(lbda=None) (nb_outer > 0) takes the same rows through their deconv_auto entry points
     const auto need = a.nb_outer > 0 ? &Variant<real>::deconv_auto : &Variant<real>::deconv;
-    // tier 0 is the group rows only (the CTA rows have no deconv); early stopping runs there only when a
-    // work-queue counter was provided (a.queue)
-    if ((!(a.early_stopping && a.wind >= 2) || a.queue) && !tier0_disabled())
-        if (const Variant<real> *v = pick<real>(TIER_GROUP_CTA, a.T, a.K, need)) {
+    const bool group_ok = (!(a.early_stopping && a.wind >= 2) || a.queue) && !tier0_disabled();
+    for (const int fam : {FAMILY_GROUP, FAMILY_WARP, FAMILY_CTA}) {
+        if (fam == FAMILY_GROUP && !group_ok) continue;
+        if (const Variant<real> *v = pick<real>(bit(fam), a.T, a.K, need)) {
             const int rc = (v->*need)(a, s);
-            if (rc != FAST_NO_MATCH) return rc;
+            if (rc != FAST_NO_MATCH) {
+                if (id) *id = encode(*v);
+                if (fam_out) *fam_out = fam;
+                return rc;
+            }
         }
-    const Variant<real> *v = pick<real>(TIER_WARP, a.T, a.K, need);
-    return v ? (v->*need)(a, s) : FAST_NO_MATCH;
+    }
+    if (id) *id = 0;
+    if (fam_out) *fam_out = FAMILY_GENERIC;
+    return FAST_NO_MATCH;
 }
 
 // the queries describe bd without early stopping and ignore PB_DISABLE_GROUP
 template <typename real>
 static int variant_id(int T, int K) {
-    const Variant<real> *v = pick<real>(TIER_GROUP_CTA, T, K, &Variant<real>::bd);
-    if (!v) v = pick<real>(TIER_WARP, T, K, &Variant<real>::bd);
-    return v ? v->lanes * 1000000 + v->R * 1000 + v->KMAX : 0;
+    const Variant<real> *v = pick<real>(TIER0, T, K, &Variant<real>::bd);
+    if (!v) v = pick<real>(bit(FAMILY_WARP), T, K, &Variant<real>::bd);
+    return v ? encode(*v) : 0;
 }
 
 template <typename real>
 static int bd_wave_voxels(int T, int K, int nb_iter) {
-    const Variant<real> *v = pick<real>(TIER_GROUP_CTA, T, K, &Variant<real>::wave);
+    const Variant<real> *v = pick<real>(TIER0, T, K, &Variant<real>::wave);
     return v ? v->wave(nb_iter) : 0;
 }
 
-int fast_deconv_dispatch(const DeconvArgs<float> &a, cudaStream_t s) { return deconv_dispatch<float>(a, s); }
-int fast_deconv_dispatch(const DeconvArgs<double> &a, cudaStream_t s) { return deconv_dispatch<double>(a, s); }
+int fast_deconv_dispatch(const DeconvArgs<float> &a, cudaStream_t s, int *id, int *fam) {
+    return deconv_dispatch<float>(a, s, id, fam);
+}
+int fast_deconv_dispatch(const DeconvArgs<double> &a, cudaStream_t s, int *id, int *fam) {
+    return deconv_dispatch<double>(a, s, id, fam);
+}
 int fast_bd_dispatch(const BdArgs<float> &a, cudaStream_t s) { return bd_dispatch<float>(a, s); }
 int fast_bd_dispatch(const BdArgs<double> &a, cudaStream_t s) { return bd_dispatch<double>(a, s); }
 

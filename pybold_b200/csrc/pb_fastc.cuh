@@ -1,5 +1,5 @@
-// Register-tiled persistent bd kernel, CTA variant: ONE CTA OF NW WARPS PER VOXEL, for long series
-// (T = 1200 at cfg4).  Thread t of the CTA owns the R contiguous samples [t R, t R + R) in
+// Register-tiled persistent bd and deconv kernels, CTA variant: ONE CTA OF NW WARPS PER VOXEL, for long series
+// (T = 1200 at cfg4) and many taps.  Thread t of the CTA owns the R contiguous samples [t R, t R + R) in
 // registers (32 NW R >= T, R a multiple of 4).
 //
 // Why: with one warp per voxel a 1200-sample voxel needs R = 38-40 samples per lane, i.e. ~255
@@ -15,9 +15,11 @@
 //  * the scans add a cross-warp carry (warp totals through shared memory);
 //  * 4 __syncthreads per iteration (w visible, forward totals, residual visible, reverse totals);
 //  * the Lipschitz constant and the theta solve are run by warp 0 with the code of pb_device.cuh.
-// No early stopping (those calls go to pb_fast.cuh).  Tap 0 of the SPM HRF is identically zero.
+// bd: no early stopping (those calls go to pb_fast.cuh / pb_fastg.cuh); tap 0 of the SPM HRF is identically zero.
+// deconv (fast_deconvc_kernel): every mode of fast_deconv_kernel, including the Q5 early stop and deconv(lbda=None),
+// for the shapes no group or warp variant serves (pb_fast_registry.cu); the caller's taps start at tap 0.
 //
-// Reference code replaced: pybold/bold_signal.py:242-278, :281-382.
+// Reference code replaced: pybold/bold_signal.py:49-97, :99-214, :242-278, :281-382.
 #pragma once
 #include "pb_fast_registry.h"
 #include "pb_generic.cuh"
@@ -73,6 +75,147 @@ struct CtaLayout {
         return (((size_t)nb_iter * sizeof(real) + 15) & ~(size_t)15) +
                ((size_t)pb_scratch_doubles(KMAX) + RED + 2 * NW + 4) * sizeof(double) +
                (size_t)2 * BUF * sizeof(real);
+    }
+    // deconv (fast_deconvc_kernel): beta | doubles: totf [NW], totr [NW], red [NW][2], the window of nwin alphas |
+    // the two buffers | the early-stopping ring of ring_rows past u's.  No theta scratch.
+    __host__ __device__ static constexpr size_t beta_bytes(int nb_iter) {
+        return ((size_t)nb_iter * sizeof(real) + 15) & ~(size_t)15;
+    }
+    __host__ __device__ static constexpr size_t deconv_dbl_bytes(int nwin) {
+        return ((size_t)(4 * NW + nwin) * sizeof(double) + 15) & ~(size_t)15;
+    }
+    __host__ __device__ static constexpr size_t deconv_bytes(int nb_iter, int ring_rows, int nwin) {
+        return beta_bytes(nb_iter) + deconv_dbl_bytes(nwin) + (size_t)2 * BUF * sizeof(real) +
+               (size_t)ring_rows * SLOTS * sizeof(real);
+    }
+};
+
+// Helpers over the register tiles of one CTA-resident deconv problem: the helpers of fast_bdc_kernel, except that
+// the tiles start at tap 0 (the caller's HRF, not the SPM one whose tap 0 is zero) and that a CTA-wide sum uses two
+// doubles per warp (red[2 w], red[2 w + 1]).  fast_bdc_kernel keeps its own copies as lambdas: routed through this
+// struct, its register allocation changed (six SASS lines in the HRF evaluation).  Thread tid owns samples
+// [i0, i0 + R).
+template <typename real, int R, int KMAX, int NW>
+struct CtaTile {
+    static constexpr int JS = 0, RS = 2;
+    using L = CtaLayout<real, R, KMAX, NW>;
+    struct alignas(4 * sizeof(real)) V4 { real t[4]; };
+    static constexpr int NH = (KMAX - 1 + 3) / 4;             // float4 per halo
+    int tid, lane, warp, i0, nvalid;
+    real *totf_r, *totr_r;                                    // [NW] forward / reverse warp totals
+    double *red;
+
+    __device__ __forceinline__ void put(real *dst, const real (&a)[R]) const {
+#pragma unroll
+        for (int r4 = 0; r4 < R / 4; ++r4) {
+            V4 t;
+#pragma unroll
+            for (int e = 0; e < 4; ++e) t.t[e] = a[4 * r4 + e];
+            reinterpret_cast<V4 *>(dst)[r4] = t;
+        }
+    }
+    // hal[m-1] = value at index (i0 - m), m = 1..4 NH
+    __device__ __forceinline__ void halo_before(const real *mine, real (&hal)[4 * NH]) const {
+#pragma unroll
+        for (int c = 0; c < NH; ++c) {
+            const V4 t = L::SKEW ? *reinterpret_cast<const V4 *>(mine - L::pos(i0) + L::pos(i0 - 4 * (c + 1)))
+                                 : reinterpret_cast<const V4 *>(mine)[-1 - c];
+#pragma unroll
+            for (int e = 0; e < 4; ++e) hal[4 * c + (3 - e)] = t.t[e];
+        }
+    }
+    // hal[k] = value at index (i0 + R + k), k = 0..4 NH - 1
+    __device__ __forceinline__ void halo_after(const real *mine, real (&hal)[4 * NH]) const {
+#pragma unroll
+        for (int c = 0; c < NH; ++c) {
+            const V4 t = L::SKEW ? *reinterpret_cast<const V4 *>(mine - L::pos(i0) + L::pos(i0 + R + 4 * c))
+                                 : reinterpret_cast<const V4 *>(mine + R)[c];
+#pragma unroll
+            for (int e = 0; e < 4; ++e) hal[4 * c + e] = t.t[e];
+        }
+    }
+    __device__ __forceinline__ void conv_acc(const real (&h)[KMAX], const real (&a)[R], const real (&hal)[4 * NH],
+                                             real (&acc)[R]) const {
+        tile_conv<real, R, KMAX, 4 * NH, JS, PB_C_CONV_JDESC, PB_C_CONV_RDESC, PB_C_CONV_RB, PB_C_CONV_DS>(h, a, hal, acc);
+    }
+    __device__ __forceinline__ void corr_acc(const real (&h)[KMAX], const real (&a)[R], const real (&hal)[4 * NH],
+                                             real (&acc)[R]) const {
+        tile_corr<real, R, KMAX, 4 * NH, JS, PB_C_CORR_JDESC, PB_C_CORR_RDESC, PB_C_CORR_RB, PB_C_CORR_DS>(h, a, hal, acc);
+    }
+    __device__ __forceinline__ void mask_tail(real (&a)[R]) const {
+#pragma unroll
+        for (int r = 0; r < R; ++r) a[r] = r < nvalid ? a[r] : real(0);
+    }
+    // CTA-wide inclusive prefix of a register tile (one barrier inside)
+    __device__ __forceinline__ void scan_fwd_cta(real (&a)[R]) const {
+#pragma unroll
+        for (int r = 1; r < R; ++r) a[r] += a[r - 1];
+        real inc = a[R - 1];
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            const real t = __shfl_up_sync(PB_FULL, inc, d);
+            if (lane >= d) inc += t;
+        }
+        if (lane == 31) totf_r[warp] = inc;
+        real carry = __shfl_up_sync(PB_FULL, inc, 1);
+        if (lane == 0) carry = real(0);
+        __syncthreads();
+#pragma unroll
+        for (int ww = 0; ww < NW - 1; ++ww)
+            if (ww < warp) carry += totf_r[ww];
+#pragma unroll
+        for (int r = 0; r < R; ++r) a[r] += carry;
+    }
+    __device__ __forceinline__ void scan_rev_cta(real (&a)[R]) const {
+#pragma unroll
+        for (int r = R - 2; r >= 0; --r) a[r] += a[r + 1];
+        real inc = a[0];
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            const real t = __shfl_down_sync(PB_FULL, inc, d);
+            if (lane + d < 32) inc += t;
+        }
+        if (lane == 0) totr_r[warp] = inc;
+        real carry = __shfl_down_sync(PB_FULL, inc, 1);
+        if (lane == 31) carry = real(0);
+        __syncthreads();
+#pragma unroll
+        for (int ww = 1; ww < NW; ++ww)
+            if (ww > warp) carry += totr_r[ww];
+#pragma unroll
+        for (int r = 0; r < R; ++r) a[r] += carry;
+    }
+    // warp sums of a and b into this warp's slots of red (no barrier)
+    __device__ __forceinline__ void publish2(double a, double b) const {
+        a = warp_sum(a);
+        b = warp_sum(b);
+        if (lane == 0) {
+            red[warp * RS] = a;
+            red[warp * RS + 1] = b;
+        }
+    }
+    // the CTA-wide sums of what publish2 wrote, warps added in a fixed order (call after a barrier)
+    __device__ __forceinline__ void gather2(double &a, double &b) const {
+        double sa = 0.0, sb = 0.0;
+#pragma unroll
+        for (int ww = 0; ww < NW; ++ww) {
+            sa += red[ww * RS];
+            sb += red[ww * RS + 1];
+        }
+        a = sa;
+        b = sb;
+    }
+    // CTA-wide sums of two doubles (two barriers; result on every thread)
+    __device__ __forceinline__ void cta_sum2(double &a, double &b) const {
+        a = warp_sum(a);
+        b = warp_sum(b);
+        __syncthreads();
+        if (lane == 0) {
+            red[warp * RS] = a;
+            red[warp * RS + 1] = b;
+        }
+        __syncthreads();
+        gather2(a, b);
     }
 };
 
@@ -412,6 +555,207 @@ fast_bdc_kernel(BdArgs<real> p) {
     }
 }
 
+// ------------------------------------------------------------------------------------------------
+// deconv (pybold/bold_signal.py:49-97), one CTA per problem, with the semantics of fast_deconv_kernel
+// (pb_fast.cuh) line for line: warm start w0, the problem's y row, taps, Lipschitz constant and lambda (the
+// regularisation path's y_mod / lbda_div, per-voxel HRFs), the active mask, the cost trace, the Q5 early stop
+// and the final cost terms.  AUTO: deconv(lbda=None), one inner pass per outer iteration of the noise loop
+// (pb_noise_loop.cuh), each restarting from the iterate of the pass before, then the final pass.
+// Barriers per iteration: the four of fast_bdc_kernel; the cost of the previous iterate rides on B3, the Q5
+// test adds one CTA-wide pair of sums (two barriers), so every thread takes the same break.  With early stopping
+// the problems come from the work queue after the first (their iteration counts differ).
+// ------------------------------------------------------------------------------------------------
+template <typename real, int R, int KMAX, int NW, int MINB, bool AUTO = false>
+__global__ void __launch_bounds__(NW * 32, MINB)
+fast_deconvc_kernel(DeconvArgs<real> p, int ring_rows) {
+    static_assert(R % 4 == 0, "R must be a multiple of 4 (vector halo exchange)");
+    using L = CtaLayout<real, R, KMAX, NW>;
+    using CT = CtaTile<real, R, KMAX, NW>;
+    constexpr int NH = CT::NH;
+    extern __shared__ __align__(16) unsigned char smem[];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    real *beta = reinterpret_cast<real *>(smem);
+    const size_t beta_bytes = L::beta_bytes(p.nb_iter);
+    fill_momentum_table(beta, p.nb_iter);
+    double *totf = reinterpret_cast<double *>(smem + beta_bytes);
+    double *red = totf + 2 * NW;                              // [NW][2], after totf [NW] and totr [NW]
+    double *win = red + 2 * NW;                               // AUTO: the window of alphas [wind]
+    real *bufA = reinterpret_cast<real *>(smem + beta_bytes + L::deconv_dbl_bytes(AUTO ? p.wind : 0));
+    real *bufB = bufA + L::BUF;
+    // ring of the past u's for the early stop (Q5): [slot][r][thread]; a thread only touches its own column
+    real *ring = bufB + L::BUF + tid;
+    for (int i = tid; i < 2 * L::BUF; i += L::NT) bufA[i] = real(0);   // zero pads (and everything else once)
+    real *const myA = bufA + L::PADB + L::pos(tid * R), *const myB = bufB + L::PADB + L::pos(tid * R);
+    const int T = p.T, K = p.K;
+    const int i0 = tid * R;
+    const int nvalid = max(0, min(R, T - i0));
+    const CT ct{tid, lane, warp, i0, nvalid, reinterpret_cast<real *>(totf), reinterpret_cast<real *>(totf + NW),
+                red};
+    const bool es = p.early_stopping && p.wind >= 2;
+    const int sub = p.wind / 2, nring = p.wind - 1;
+    __syncthreads();
+
+    real w[R], dy[R], h[KMAX];
+    auto sumsq = [&](const real (&a)[R]) {
+        real s = 0;
+#pragma unroll
+        for (int r = 0; r < R; ++r) s = fma(a[r], a[r], s);
+        return (double)s;
+    };
+    auto sumabs = [&](const real (&a)[R]) {
+        real s = 0;
+#pragma unroll
+        for (int r = 0; r < R; ++r) s += fabs(a[r]);
+        return (double)s;
+    };
+    // res <- A w - y, zero at and beyond T (B1, B2)
+    auto forward = [&](real (&res)[R]) {
+        real hal[4 * NH];
+        ct.put(myA, w);
+        __syncthreads();                                      // B1: w visible
+        ct.halo_before(myA, hal);
+#pragma unroll
+        for (int r = 0; r < R; ++r) res[r] = -dy[r];
+        ct.conv_acc(h, w, hal, res);
+        ct.scan_fwd_cta(res);                                 // B2 inside
+        ct.mask_tail(res);
+    };
+    // g <- A^T res (B3, B4)
+    auto adjoint = [&](const real (&res)[R], real (&g)[R]) {
+        real hal[4 * NH];
+        ct.put(myB, res);
+        __syncthreads();                                      // B3: residual visible
+        ct.halo_after(myB, hal);
+#pragma unroll
+        for (int r = 0; r < R; ++r) g[r] = real(0);
+        ct.corr_acc(h, res, hal, g);
+        ct.scan_rev_cta(g);                                   // B4 inside
+    };
+
+    __shared__ unsigned int next_task;
+    for (int64_t v = blockIdx.x; v < p.V;) {
+        if (p.is_active(v)) {
+            const real *yv = p.y_row(v);
+            const real *hv = p.h_row(v);
+#pragma unroll
+            for (int r = 0; r < R; ++r) {
+                const int i = i0 + r;
+                const real cur = i < T ? yv[i] : real(0);
+                const real prv = (i > 0 && i - 1 < T) ? yv[i - 1] : real(0);
+                dy[r] = i < T ? cur - prv : real(0);
+                w[r] = (p.w0 && i < T) ? p.w0[v * T + i] : real(0);
+            }
+#pragma unroll
+            for (int j = 0; j < KMAX; ++j) h[j] = j < K ? hv[j] : real(0);
+            const double Lc = p.L_of(v);
+            NoiseLoop nl;
+            if (AUTO) nl.start(win);
+            double lam = AUTO ? nl.lbda : p.lam_of(v);
+            const real step = (real)(1.0 / Lc);
+            real th = (real)(lam / Lc);
+            real *Jv = p.out_J + v * (int64_t)p.nb_iter;
+            const bool trace = !AUTO && p.out_J;
+            int n_done = 0, ring_pos = 0;
+            real res[R];
+            for (;;) {   // one pass (AUTO: one per outer iteration)
+                n_done = 0;
+                ring_pos = 0;
+                for (int k = 0; k < p.nb_iter; ++k) {
+                    forward(res);
+                    // cost of the previous iterate: its residual has just been formed; the warp sums ride on B3
+                    if (trace && k > 0) ct.publish2(sumsq(res), sumabs(w));
+                    real g[R];
+                    adjoint(res, g);
+                    if (trace && k > 0 && tid == 0) {
+                        double s2, s1;
+                        ct.gather2(s2, s1);
+                        Jv[k - 1] = (real)(0.5 * s2 + lam * s1);
+                    }
+                    const real ob = real(1) + beta[k];
+                    real *slot = ring + (size_t)ring_pos * R * L::NT;    // ring_pos = k % nring
+#pragma unroll
+                    for (int r = 0; r < R; ++r) {
+                        const real u = fma(-step, g[r], w[r]);
+                        const real cl = fmin(fmax(u, -th), th);
+                        w[r] = fma(-ob, cl, u);
+                        if (es) slot[r * L::NT] = u;
+                    }
+                    n_done = k + 1;
+                    if (es && k > p.wind) {
+                        // xx = [u_{k-wind+2}, ..., u_k, w_k]; old = mean(first wind-sub), new = mean(last sub)
+                        const real inv_old = real(1) / real(p.wind - sub), inv_new = real(1) / real(sub);
+                        real so[R], sn[R];
+#pragma unroll
+                        for (int r = 0; r < R; ++r) {
+                            so[r] = 0;
+                            sn[r] = w[r];
+                        }
+                        int pos = ring_pos + 1 == nring ? 0 : ring_pos + 1;   // (k - wind + 2) % nring: oldest u
+                        for (int m = 0; m < p.wind - 1; ++m) {
+                            const real *s = ring + (size_t)pos * R * L::NT;
+                            pos = pos + 1 == nring ? 0 : pos + 1;
+                            const bool is_old = m < p.wind - sub;
+#pragma unroll
+                            for (int r = 0; r < R; ++r) {
+                                const real uu = s[r * L::NT];
+                                if (is_old) so[r] += uu; else sn[r] += uu;
+                            }
+                        }
+                        real qn = 0, qd = 0;              // thread partials in `real`, warp sums in double
+#pragma unroll
+                        for (int r = 0; r < R; ++r) {
+                            const real mo = so[r] * inv_old, mn = sn[r] * inv_new;
+                            qn = fma(mn - mo, mn - mo, qn);
+                            qd = fma(mn, mn, qd);
+                        }
+                        double pn = (double)qn, pd = (double)qd;
+                        ct.cta_sum2(pn, pd);
+                        if (sqrt(pn) / (sqrt(pd) + 1.0e-10) < p.tol) break;
+                    }
+                    if (es) ring_pos = ring_pos + 1 == nring ? 0 : ring_pos + 1;
+                }
+                forward(res);
+                double rr = sumsq(res), gg = sumabs(w);
+                ct.cta_sum2(rr, gg);
+                if (AUTO) {
+                    if (!nl.pass_done(p, v, rr, gg, tid == 0, tid, L::NT)) {
+                        lam = nl.lbda;
+                        th = (real)(lam / Lc);
+                        continue;
+                    }
+                } else if (n_done > 0 && tid == 0) {
+                    if (p.out_J) Jv[n_done - 1] = (real)(0.5 * rr + lam * gg);
+                    if (p.out_r) p.out_r[v] = (real)rr;
+                    if (p.out_g) p.out_g[v] = (real)gg;
+                }
+                break;
+            }
+            real z[R];
+#pragma unroll
+            for (int r = 0; r < R; ++r) z[r] = w[r];
+            ct.scan_fwd_cta(z);
+#pragma unroll
+            for (int r = 0; r < R; ++r) {
+                const int i = i0 + r;
+                if (i < T) {
+                    p.out_x[v * T + i] = res[r] + yv[i];      // x = (A w - y) + y
+                    p.out_z[v * T + i] = z[r];
+                    p.out_dz[v * T + i] = w[r];
+                }
+            }
+            if (tid == 0 && !AUTO) p.out_niter[v] = n_done;
+        }
+        if (p.queue) {
+            __syncthreads();
+            if (tid == 0) next_task = atomicAdd(p.queue, 1u);
+            __syncthreads();
+            v = (int64_t)gridDim.x + (int64_t)next_task;
+        } else {
+            v += gridDim.x;
+        }
+    }
+}
+
 template <int R, int KMAX, int NW>
 bool fastc_shape_ok(int T, int K) {
     // the last used thread may be partial, threads beyond it idle; up to half of the threads may idle
@@ -437,10 +781,21 @@ int fast_bdc_wave(int nb_iter) {
     return wave_voxels(fast_bdc_kernel<real, R, KMAX, NW, MINB>, NW * 32, L::bytes(nb_iter), 1);
 }
 
+// FAST_NO_MATCH when the early-stopping ring does not fit: the generic kernel decides
+template <typename real, int R, int KMAX, int NW, int MINB, bool AUTO = false>
+int fast_deconvc_launch(const DeconvArgs<real> &a, cudaStream_t stream) {
+    using L = CtaLayout<real, R, KMAX, NW>;
+    const int ring_rows = a.early_stopping && a.wind >= 2 ? a.wind - 1 : 0;
+    return launch_persistent(fast_deconvc_kernel<real, R, KMAX, NW, MINB, AUTO>, NW * 32,
+                             L::deconv_bytes(a.nb_iter, ring_rows, AUTO ? a.wind : 0), 1, a.V, a.queue, stream, a,
+                             ring_rows);
+}
+
 template <typename real, int R, int KMAX, int NW, int MINB>
 constexpr Variant<real> cta_variant() {
     return {TIER_GROUP_CTA, 32 * NW, R, KMAX, 0, false, fastc_shape_ok<R, KMAX, NW>,
-            fast_bdc_launch<real, R, KMAX, NW, MINB>, nullptr, nullptr, fast_bdc_wave<real, R, KMAX, NW, MINB>};
+            fast_bdc_launch<real, R, KMAX, NW, MINB>, nullptr, fast_deconvc_launch<real, R, KMAX, NW, MINB>,
+            fast_bdc_wave<real, R, KMAX, NW, MINB>, fast_deconvc_launch<real, R, KMAX, NW, MINB, true>};
 }
 
 }  // namespace pb

@@ -58,6 +58,10 @@ int pb_bd_wave_voxels(int T, int K, int is_f64, int nb_iter);
  * Negative PB_ERR_* on bad arguments, shapes beyond the limits, or PB_ERR_NO_DEVICE. */
 int pb_deconv_variant(int T, int K, int is_f64, int nb_iter, int early_stopping, int wind, int is_auto,
                       int *family);
+/* Which kernel a pb_bd_f32 / pb_bd_f64 call with this shape and (nb_iter, early_stopping, wind) runs on the current
+ * device, in the encoding and with the family codes and errors of pb_deconv_variant.  The choice is the launch's
+ * own, shared-memory and occupancy checks included.  With early_stopping = 0 the id is pb_solver_variant's. */
+int pb_bd_variant(int T, int K, int is_f64, int nb_iter, int early_stopping, int wind, int *family);
 
 /* ---- A1: DiscretInteg.op / .adj (pybold/linear.py:15-28, :30-43) -------------------- */
 int pb_integ_op_f32(const float *x, float *out, int64_t V, int T, pb_stream_t stream);

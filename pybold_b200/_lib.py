@@ -84,6 +84,7 @@ _PLAIN = {
     "pb_hrf_len_ex": ([c_double, c_double, c_double], c_int),
     "pb_bd_wave_voxels": ([c_int, c_int, c_int, c_int], c_int),
     "pb_deconv_variant": ([c_int, c_int, c_int, c_int, c_int, c_int, c_int, ctypes.POINTER(c_int)], c_int),
+    "pb_bd_variant": ([c_int, c_int, c_int, c_int, c_int, c_int, ctypes.POINTER(c_int)], c_int),
     "pb_bench_fma_f32": ([_P, c_int, c_int, _P], c_int),
     "pb_copy_async": ([_P, _P, ctypes.c_size_t, _P], c_int),
 }

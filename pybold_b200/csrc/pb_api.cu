@@ -469,6 +469,26 @@ int deconv_variant(int T, int K, int nb_iter, int early_stopping, int wind, int 
     return rc < 0 ? rc : id;
 }
 
+// the register-tiled variant bd_dispatch chooses (pb_fast_registry.cu), else the generic kernel.  V == 0 launches
+// nothing: *id / *family report the kernel a launch would run (pb_bd_variant).
+template <typename real>
+int launch_bd(const pb::BdArgs<real> &a, pb_stream_t stream, int *id = nullptr, int *family = nullptr) {
+    int rc = pb::fast_bd_dispatch(a, (cudaStream_t)stream, id, family);
+    if (rc != pb::FAST_NO_MATCH) return rc;
+    DeviceInfo d = device_info();
+    if (d.err) return d.err;
+    pb::GenLayout lay = pb::GenLayout::make(a.T, a.K, 0, true);
+    const size_t beta_bytes = ((size_t)a.nb_iter * sizeof(real) + 15) & ~(size_t)15;
+    LaunchPlan p = plan_launch(d, beta_bytes, lay.warp_bytes(sizeof(real)), a.V, 8);
+    if (!p.warps) return PB_ERR_UNSUPPORTED;
+    if (a.V == 0) return PB_OK;
+    auto kern = pb::generic_bd_kernel<real>;
+    int e = set_smem(kern, p.smem);
+    if (e) return e;
+    kern<<<p.grid, p.warps * 32, p.smem, (cudaStream_t)stream>>>(a, lay);
+    return last_error();
+}
+
 template <typename real>
 int run_bd(pb::BdArgs<real> a, double t_r, double hrf_dur, pb_stream_t stream) {
     if (a.V == 0) return PB_OK;
@@ -484,19 +504,29 @@ int run_bd(pb::BdArgs<real> a, double t_r, double hrf_dur, pb_stream_t stream) {
     // group / CTA kernels pull their tasks from it (static stride if null; PB_NO_QUEUE=1: developer A/B switch)
     static const bool no_queue = getenv("PB_NO_QUEUE") != nullptr;
     a.queue = no_queue ? nullptr : queue_slot();
-    int rc = pb::fast_bd_dispatch(a, (cudaStream_t)stream);
-    if (rc != pb::FAST_NO_MATCH) return rc;
-    DeviceInfo d = device_info();
-    if (d.err) return d.err;
-    pb::GenLayout lay = pb::GenLayout::make(a.T, a.K, 0, true);
-    const size_t beta_bytes = ((size_t)a.nb_iter * sizeof(real) + 15) & ~(size_t)15;
-    LaunchPlan p = plan_launch(d, beta_bytes, lay.warp_bytes(sizeof(real)), a.V, 8);
-    if (!p.warps) return PB_ERR_UNSUPPORTED;
-    auto kern = pb::generic_bd_kernel<real>;
-    int e = set_smem(kern, p.smem);
-    if (e) return e;
-    kern<<<p.grid, p.warps * 32, p.smem, (cudaStream_t)stream>>>(a, lay);
-    return last_error();
+    return launch_bd(a, stream);
+}
+
+// pb_bd_variant: the routing of a bd call with V = 0 (nothing is launched; the work-queue counter plays no part in
+// the choice)
+template <typename real>
+int bd_variant(int T, int K, int nb_iter, int early_stopping, int wind, int *family) {
+    if (!family || T <= 0 || K <= 0 || nb_iter < 1 || wind < 0) return PB_ERR_INVALID_ARG;
+    if (T > PB_MAX_T || K > PB_MAX_K || nb_iter > PB_MAX_ITER) return PB_ERR_UNSUPPORTED;
+    pb::BdArgs<real> a{};
+    a.T = T;
+    a.K = K;
+    a.nb_iter = nb_iter;
+    a.early_stopping = early_stopping;
+    a.wind = wind;
+    a.V = 0;
+    int id = 0;
+    const int rc = launch_bd(a, nullptr, &id, family);
+    if (rc > 0) {               // a CUDA error
+        cudaGetLastError();
+        return PB_ERR_NO_DEVICE;
+    }
+    return rc < 0 ? rc : id;
 }
 
 template <typename real>
@@ -672,6 +702,11 @@ int pb_deconv_variant(int T, int K, int is_f64, int nb_iter, int early_stopping,
                       int *family) {
     return is_f64 ? deconv_variant<double>(T, K, nb_iter, early_stopping, wind, is_auto, family)
                   : deconv_variant<float>(T, K, nb_iter, early_stopping, wind, is_auto, family);
+}
+
+int pb_bd_variant(int T, int K, int is_f64, int nb_iter, int early_stopping, int wind, int *family) {
+    return is_f64 ? bd_variant<double>(T, K, nb_iter, early_stopping, wind, family)
+                  : bd_variant<float>(T, K, nb_iter, early_stopping, wind, family);
 }
 
 int pb_bd_wave_voxels(int T, int K, int is_f64, int nb_iter) {

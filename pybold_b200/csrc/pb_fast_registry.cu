@@ -57,23 +57,33 @@ static bool tier0_disabled() {
     return disabled;
 }
 
-// The warp tier runs only when the one tier-0 candidate returns FAST_NO_MATCH (its shared memory
-// does not fit); no second tier-0 candidate is tried.
 template <typename real>
-static int bd_dispatch(const BdArgs<real> &a, cudaStream_t s) {
-    // early stopping: only the rows with bd_es (the group variants) are candidates
+static int encode(const Variant<real> &v) { return v.lanes * 1000000 + v.R * 1000 + v.KMAX; }
+
+// The warp tier runs only when the one tier-0 candidate returns FAST_NO_MATCH (its shared memory
+// does not fit); no second tier-0 candidate is tried.  Every tier-0 row (group and CTA) has both bd entry points, so
+// with and without early stopping a call runs on the same row.  V == 0 launches nothing and reports the same choice.
+template <typename real>
+static int bd_dispatch(const BdArgs<real> &a, cudaStream_t s, int *id, int *fam_out) {
     const auto need = a.early_stopping ? &Variant<real>::bd_es : &Variant<real>::bd;
+    auto ran = [&](const Variant<real> &v, int rc) {
+        if (id) *id = encode(v);
+        if (fam_out) *fam_out = family(v);
+        return rc;
+    };
     if (!tier0_disabled())
         if (const Variant<real> *v = pick<real>(TIER0, a.T, a.K, need)) {
             const int rc = (v->*need)(a, s);
-            if (rc != FAST_NO_MATCH) return rc;
+            if (rc != FAST_NO_MATCH) return ran(*v, rc);
         }
-    const Variant<real> *v = pick<real>(bit(FAMILY_WARP), a.T, a.K, &Variant<real>::bd);
-    return v ? v->bd(a, s) : FAST_NO_MATCH;
+    if (const Variant<real> *v = pick<real>(bit(FAMILY_WARP), a.T, a.K, &Variant<real>::bd)) {
+        const int rc = v->bd(a, s);
+        if (rc != FAST_NO_MATCH) return ran(*v, rc);
+    }
+    if (id) *id = 0;
+    if (fam_out) *fam_out = FAMILY_GENERIC;
+    return FAST_NO_MATCH;
 }
-
-template <typename real>
-static int encode(const Variant<real> &v) { return v.lanes * 1000000 + v.R * 1000 + v.KMAX; }
 
 // Routing of every deconv call (fixed lambda, early stopping, lbda=None, path, masked): group rows, then warp rows,
 // then CTA rows, then (launch_deconv) the generic kernel.  A step is taken when the one before has no variant for
@@ -120,8 +130,12 @@ int fast_deconv_dispatch(const DeconvArgs<float> &a, cudaStream_t s, int *id, in
 int fast_deconv_dispatch(const DeconvArgs<double> &a, cudaStream_t s, int *id, int *fam) {
     return deconv_dispatch<double>(a, s, id, fam);
 }
-int fast_bd_dispatch(const BdArgs<float> &a, cudaStream_t s) { return bd_dispatch<float>(a, s); }
-int fast_bd_dispatch(const BdArgs<double> &a, cudaStream_t s) { return bd_dispatch<double>(a, s); }
+int fast_bd_dispatch(const BdArgs<float> &a, cudaStream_t s, int *id, int *fam) {
+    return bd_dispatch<float>(a, s, id, fam);
+}
+int fast_bd_dispatch(const BdArgs<double> &a, cudaStream_t s, int *id, int *fam) {
+    return bd_dispatch<double>(a, s, id, fam);
+}
 
 int fast_bd_wave_voxels(int T, int K, bool is_f64, int nb_iter) {
     return is_f64 ? bd_wave_voxels<double>(T, K, nb_iter) : bd_wave_voxels<float>(T, K, nb_iter);

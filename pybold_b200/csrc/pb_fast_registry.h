@@ -16,8 +16,8 @@ constexpr int FAST_NO_MATCH = -1000;
 // variant are those a launch would have
 int fast_deconv_dispatch(const DeconvArgs<float> &a, cudaStream_t stream, int *id = nullptr, int *family = nullptr);
 int fast_deconv_dispatch(const DeconvArgs<double> &a, cudaStream_t stream, int *id = nullptr, int *family = nullptr);
-int fast_bd_dispatch(const BdArgs<float> &a, cudaStream_t stream);
-int fast_bd_dispatch(const BdArgs<double> &a, cudaStream_t stream);
+int fast_bd_dispatch(const BdArgs<float> &a, cudaStream_t stream, int *id = nullptr, int *family = nullptr);
+int fast_bd_dispatch(const BdArgs<double> &a, cudaStream_t stream, int *id = nullptr, int *family = nullptr);
 // 0 = generic kernel, else lanes per voxel * 1000000 + R * 1000 + KMAX
 int fast_variant_id(int T, int K, bool is_f64);
 // voxels per full wave of the persistent bd grid (0 when unknown): batch sizes that are multiples
@@ -28,7 +28,7 @@ int fast_bd_wave_voxels(int T, int K, bool is_f64, int nb_iter);
 // warp-per-voxel variant only when that launch returns FAST_NO_MATCH (bd_dispatch).  deconv goes through the
 // families in the order group, warp, CTA, then the generic kernel (deconv_dispatch, pb_fast_registry.cu).
 enum VariantTier { TIER_GROUP_CTA = 0, TIER_WARP = 1 };
-// the kernel family a call ran on (the *family of pb_deconv_variant)
+// the kernel family a call ran on (the *family of pb_deconv_variant and pb_bd_variant)
 enum VariantFamily { FAMILY_GENERIC = 0, FAMILY_GROUP = 1, FAMILY_WARP = 2, FAMILY_CTA = 3 };
 
 template <typename real>

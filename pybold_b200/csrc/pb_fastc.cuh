@@ -15,7 +15,7 @@
 //  * the scans add a cross-warp carry (warp totals through shared memory);
 //  * 4 __syncthreads per iteration (w visible, forward totals, residual visible, reverse totals);
 //  * the Lipschitz constant and the theta solve are run by warp 0 with the code of pb_device.cuh.
-// bd: no early stopping (those calls go to pb_fast.cuh / pb_fastg.cuh); tap 0 of the SPM HRF is identically zero.
+// bd: tap 0 of the SPM HRF is identically zero.  ES = true runs the reference's early stopping (Q6 / Q7, below).
 // deconv (fast_deconvc_kernel): every mode of fast_deconv_kernel, including the Q5 early stop and deconv(lbda=None),
 // for the shapes no group or warp variant serves (pb_fast_registry.cu); the caller's taps start at tap 0.
 //
@@ -219,7 +219,15 @@ struct CtaTile {
     }
 };
 
-template <typename real, int R, int KMAX, int NW, int MINB>
+// ES = true: bd(early_stopping=True).  Q6 -- the inner loop stops at iteration j > 2 once
+// ||w_j - u_j|| / (||w_j|| + 1e-10) < tol, with ||w_j - u_j|| = (1 + beta_j) ||clamp(u_j)|| -- takes its two sums on
+// the barriers already there: the warp sums of iteration j go to red[2], red[3] of the warp's row before B1 of
+// iteration j + 1, and every thread reads them after it and takes the same break (iteration j + 1 has then only
+// stored w).  Q7 -- the signed window test on J (bd_outer_stop) after pass idx > wind -- is run by thread 0, which
+// wrote J, while warp 0 forms the Lipschitz constant of the next pass; the decision reaches every thread on the
+// barrier after it and makes that pass the last one.  out_ntrace = idx + 3 for a stop after pass idx.  With
+// ES = false none of this is compiled in.
+template <typename real, int R, int KMAX, int NW, int MINB, bool ES = false>
 __global__ void __launch_bounds__(NW * 32, MINB)
 fast_bdc_kernel(BdArgs<real> p) {
     static_assert(R % 4 == 0, "R must be a multiple of 4 (vector halo exchange)");
@@ -237,7 +245,7 @@ fast_bdc_kernel(BdArgs<real> p) {
     double *red = dbl + pb_scratch_doubles(KMAX);             // [NW][2 KMAX + 4]
     double *totf = red + L::RED;                              // [NW] forward warp totals
     double *totr = totf + NW;                                 // [NW] reverse warp totals
-    double *bcast = totr + NW;                                // [4]  theta, Lipschitz, ...
+    double *bcast = totr + NW;                                // [4]  theta, Lipschitz, Q7 stop, -
     real *bufA = reinterpret_cast<real *>(bcast + 4);         // w / z with zero pads
     real *bufB = bufA + L::BUF;                               // residual with zero pads
     for (int i = tid; i < 2 * L::BUF; i += L::NT) bufA[i] = real(0);   // zero pads (and everything else once)
@@ -416,20 +424,38 @@ fast_bdc_kernel(BdArgs<real> p) {
             rv[0] = real(1);
             gv[0] = (real)g0;
         }
+        int n_tr = ntr;                                           // ES: trace entries written
+        double sumJ = 1.0;                                        // ES: sum of the J entries (as stored)
         for (int idx = 0; idx <= p.nb_iter; ++idx) {
-            const bool last = idx == p.nb_iter;                   // final deconvolution, :365-376
+            bool last = idx == p.nb_iter;                         // final deconvolution, :365-376
             __syncthreads();
             if (warp == 0) {
                 const double Lw = frob_lipschitz_warp(sc, K, T, lane);
                 if (lane == 0) bcast[1] = Lw;
+                if constexpr (ES)                                 // Q7 (:350-362) after pass idx - 1: J[0 .. idx]
+                    if (lane == 0)
+                        bcast[2] = idx - 1 > p.wind && bd_outer_stop(Jv, idx + 1, sumJ, p.wind / 2, p.tol) ? 1.0 : 0.0;
             }
             __syncthreads();
+            if constexpr (ES) last = last || bcast[2] != 0.0;     // (:350-362: the pass after the stop is the last)
             const double Lc = bcast[1];
             const real step = (real)(1.0 / Lc), th = (real)(lam / Lc);
             for (int j = 0; j < p.nb_iter; ++j) {                 // _loops_deconv, :259-276
                 real hal[4 * NH], res[R], g[R];
                 put(myA, w);
                 __syncthreads();                                  // B1: w visible
+                if constexpr (ES) {
+                    if (j > 3) {                                  // Q6 (:267-273) on iteration j - 1
+                        double sc2 = 0.0, sw2 = 0.0;
+#pragma unroll
+                        for (int ww = 0; ww < NW; ++ww) {
+                            sc2 += red[ww * (2 * KMAX + 4) + 2];
+                            sw2 += red[ww * (2 * KMAX + 4) + 3];
+                        }
+                        const double num = (1.0 + (double)beta[j - 1]) * sqrt(sc2);   // ||w - u||
+                        if (num / (sqrt(sw2) + 1.0e-10) < p.tol) break;
+                    }
+                }
                 halo_before(myA, hal);
 #pragma unroll
                 for (int r = 0; r < R; ++r) res[r] = -dy[r];
@@ -444,11 +470,30 @@ fast_bdc_kernel(BdArgs<real> p) {
                 corr_acc(res, hal, g);
                 scan_rev_cta(g);                                  // B4 inside
                 const real ob = real(1) + beta[j];
+                if constexpr (!ES) {
 #pragma unroll
-                for (int r = 0; r < R; ++r) {
-                    const real u = fma(-step, g[r], w[r]);
-                    const real cl = fmin(fmax(u, -th), th);
-                    w[r] = fma(-ob, cl, u);
+                    for (int r = 0; r < R; ++r) {
+                        const real u = fma(-step, g[r], w[r]);
+                        const real cl = fmin(fmax(u, -th), th);
+                        w[r] = fma(-ob, cl, u);
+                    }
+                } else {
+                    real pc = 0, pw = 0;
+#pragma unroll
+                    for (int r = 0; r < R; ++r) {
+                        const real u = fma(-step, g[r], w[r]);
+                        const real cl = fmin(fmax(u, -th), th);
+                        w[r] = fma(-ob, cl, u);
+                        pc = fma(cl, cl, pc);
+                        pw = fma(w[r], w[r], pw);
+                    }
+                    if (j > 2) {                                  // read after the next B1
+                        const double sc2 = warp_sum((double)pc), sw2 = warp_sum((double)pw);
+                        if (lane == 0) {
+                            red[warp * (2 * KMAX + 4) + 2] = sc2;
+                            red[warp * (2 * KMAX + 4) + 3] = sw2;
+                        }
+                    }
                 }
             }
             real z[R], hal[4 * NH];
@@ -531,6 +576,7 @@ fast_bdc_kernel(BdArgs<real> p) {
                 rv[idx + 1] = (real)(rr / r0 + eps);
                 gv[idx + 1] = (real)gg;
             }
+            if constexpr (ES) sumJ += (double)(real)((rr + lam * gg) / j0 + eps);
             if (last) {
 #pragma unroll
                 for (int r = 0; r < R; ++r) {
@@ -541,13 +587,17 @@ fast_bdc_kernel(BdArgs<real> p) {
                         p.out_dz[v * T + i] = w[r];
                     }
                 }
+                if constexpr (ES) {
+                    n_tr = idx + 2;
+                    break;
+                }
             }
         }
         __syncthreads();
         for (int a = tid; a < K; a += L::NT) p.out_h[v * K + a] = (real)sc.hs[a];
         if (tid == 0) {
             p.out_theta[v] = (real)theta;
-            p.out_ntrace[v] = ntr;
+            p.out_ntrace[v] = n_tr;
             if (p.queue) next_task = atomicAdd(p.queue, 1u);
         }
         __syncthreads();
@@ -768,10 +818,11 @@ bool fastc_shape_ok(int T, int K) {
            (T > NW * 16 * R - R || (NW == 1 && R == 4)) && T >= 1;
 }
 
-template <typename real, int R, int KMAX, int NW, int MINB>
+// ES: bd(early_stopping=True), which needs no shared memory beyond the kernel without it
+template <typename real, int R, int KMAX, int NW, int MINB, bool ES = false>
 int fast_bdc_launch(const BdArgs<real> &a, cudaStream_t stream) {
     using L = CtaLayout<real, R, KMAX, NW>;
-    return launch_persistent(fast_bdc_kernel<real, R, KMAX, NW, MINB>, NW * 32, L::bytes(a.nb_iter), 1, a.V,
+    return launch_persistent(fast_bdc_kernel<real, R, KMAX, NW, MINB, ES>, NW * 32, L::bytes(a.nb_iter), 1, a.V,
                              a.queue, stream, a);
 }
 
@@ -794,7 +845,8 @@ int fast_deconvc_launch(const DeconvArgs<real> &a, cudaStream_t stream) {
 template <typename real, int R, int KMAX, int NW, int MINB>
 constexpr Variant<real> cta_variant() {
     return {TIER_GROUP_CTA, 32 * NW, R, KMAX, 0, false, fastc_shape_ok<R, KMAX, NW>,
-            fast_bdc_launch<real, R, KMAX, NW, MINB>, nullptr, fast_deconvc_launch<real, R, KMAX, NW, MINB>,
+            fast_bdc_launch<real, R, KMAX, NW, MINB>, fast_bdc_launch<real, R, KMAX, NW, MINB, true>,
+            fast_deconvc_launch<real, R, KMAX, NW, MINB>,
             fast_bdc_wave<real, R, KMAX, NW, MINB>, fast_deconvc_launch<real, R, KMAX, NW, MINB, true>};
 }
 

@@ -17,7 +17,8 @@
 //    the bd kernel starts its tap loops at j = 1;
 //  * the Lipschitz / theta phases (double, O(K^2)) run for all groups of the warp in lock step
 //    (pb_theta_group.cuh): measured, running them group after group cost 14 % of the kernel.
-// Early stopping (Q6/Q7) makes groups diverge; those calls are served by pb_fast.cuh (G = 32).
+// Early stopping (Q6/Q7) makes groups diverge: fast_bdg_kernel<..., ES = true> (below) lets a group that has
+// stopped wait for its neighbour.
 //
 // Reference code replaced: pybold/bold_signal.py:242-278, :281-382.
 #pragma once

@@ -242,6 +242,70 @@ int pb_deconv_lbda_path_ex_f64(const double *y, const double *h, int64_t h_strid
                                double *out_r, double *out_g, int32_t *out_niter, int64_t V, int T, int K,
                                pb_stream_t stream);
 
+/* ---- Scan censoring for deconv, deconv(lbda=None) and the lambda path (no reference counterpart).
+ * Volumes flagged for head motion ("scrubbing") stay on the model's time grid and leave the data term:
+ *   min_w 1/2 ||M (A w - y)||^2 + lbda ||w||_1,   M = diag(1 - censor)
+ *   censor[v*censor_stride + i] != 0   scan i of voxel v is left out (uint8; censor_stride 0: one [T] mask for the
+ *                                      batch, T: one row per voxel; for the path, per voxel of y, not per problem)
+ *   y                                  read as 0 on censored scans: NaN or Inf there are ignored
+ *   out_x                              A w on EVERY scan (the model's prediction at the gaps); z, diff_z likewise
+ *   out_J, out_r / out_R               with the masked residual M (A w - y)
+ *   L                                  the caller's Lipschitz constant; the censored operator's is 0.9 x
+ *                                      pb_lipschitz_power_censored_* from the same start
+ *   deconv(lbda=None)                  alpha += 1e-4 (||M (x - y)||^2 - n_kept sigma^2), n_kept = the voxel's kept scans
+ * Precondition: every voxel keeps at least one scan (an all-censored voxel has a zero operator and no Lipschitz
+ * constant).  Otherwise each entry point takes the arguments of its uncensored twin and behaves like it; calls run
+ * on the register-tiled CTA kernels wherever one fits (pb_deconv_censored_variant), else on the generic kernel. */
+int pb_deconv_censored_f32(const float *y, const float *h, int64_t h_stride, const float *L, int64_t L_stride,
+                           const float *lbda, int64_t lbda_stride, const float *w0, const unsigned char *censor,
+                           int64_t censor_stride, int nb_iter, int early_stopping, int wind, double tol, float *out_x,
+                           float *out_z, float *out_dz, float *out_J, int32_t *out_niter, int64_t V, int T, int K,
+                           pb_stream_t stream);
+int pb_deconv_censored_f64(const double *y, const double *h, int64_t h_stride, const double *L, int64_t L_stride,
+                           const double *lbda, int64_t lbda_stride, const double *w0, const unsigned char *censor,
+                           int64_t censor_stride, int nb_iter, int early_stopping, int wind, double tol,
+                           double *out_x, double *out_z, double *out_dz, double *out_J, int32_t *out_niter,
+                           int64_t V, int T, int K, pb_stream_t stream);
+int pb_deconv_auto_censored_f32(const float *y, const float *h, int64_t h_stride, const float *L, int64_t L_stride,
+                                const float *sigma, int64_t sigma_stride, const unsigned char *censor,
+                                int64_t censor_stride, int nb_iter, int nb_sub_iter, int early_stopping, int wind,
+                                double tol, float *out_x, float *out_z, float *out_dz, float *out_J, float *out_R,
+                                float *out_G, float *out_lbda, int32_t *out_nouter, int64_t V, int T, int K,
+                                pb_stream_t stream);
+int pb_deconv_auto_censored_f64(const double *y, const double *h, int64_t h_stride, const double *L,
+                                int64_t L_stride, const double *sigma, int64_t sigma_stride,
+                                const unsigned char *censor, int64_t censor_stride, int nb_iter, int nb_sub_iter,
+                                int early_stopping, int wind, double tol, double *out_x, double *out_z,
+                                double *out_dz, double *out_J, double *out_R, double *out_G, double *out_lbda,
+                                int32_t *out_nouter, int64_t V, int T, int K, pb_stream_t stream);
+int pb_deconv_lbda_path_censored_f32(const float *y, const float *h, int64_t h_stride, const float *L,
+                                     int64_t L_stride, const float *lbdas, int n_lbda, const unsigned char *censor,
+                                     int64_t censor_stride, int nb_iter, int early_stopping, int wind, double tol,
+                                     float *out_x, float *out_z, float *out_dz, float *out_J, float *out_r,
+                                     float *out_g, int32_t *out_niter, int64_t V, int T, int K, pb_stream_t stream);
+int pb_deconv_lbda_path_censored_f64(const double *y, const double *h, int64_t h_stride, const double *L,
+                                     int64_t L_stride, const double *lbdas, int n_lbda, const unsigned char *censor,
+                                     int64_t censor_stride, int nb_iter, int early_stopping, int wind, double tol,
+                                     double *out_x, double *out_z, double *out_dz, double *out_J, double *out_r,
+                                     double *out_g, int32_t *out_niter, int64_t V, int T, int K, pb_stream_t stream);
+/* Power iteration on A^T M A, M applied between op and adj (arguments of pb_lipschitz_power_*, mask as above). */
+int pb_lipschitz_power_censored_f32(const float *h, int64_t h_stride, const float *x0, int64_t x0_stride,
+                                    const unsigned char *censor, int64_t censor_stride, int nb_iter, double tol,
+                                    float *out_L, int64_t V, int T, int K, pb_stream_t stream);
+int pb_lipschitz_power_censored_f64(const double *h, int64_t h_stride, const double *x0, int64_t x0_stride,
+                                    const unsigned char *censor, int64_t censor_stride, int nb_iter, double tol,
+                                    double *out_L, int64_t V, int T, int K, pb_stream_t stream);
+/* pb_mad_daub_noise_est over the level-1 db3 detail coefficients that touch no censored scan (a coefficient reads
+ * six samples, after the symmetric extension; T < 10: the kept samples).  NaN for a voxel with none left. */
+int pb_mad_daub_noise_est_censored_f32(const float *y, const unsigned char *censor, int64_t censor_stride, double c,
+                                       float *out_sigma, int64_t V, int T, pb_stream_t stream);
+int pb_mad_daub_noise_est_censored_f64(const double *y, const unsigned char *censor, int64_t censor_stride,
+                                       double c, double *out_sigma, int64_t V, int T, pb_stream_t stream);
+/* The kernel a censored deconv call of this shape runs on, in the encoding, family codes and V = 0 routing of
+ * pb_deconv_variant (3 = CTA, 0 = generic). */
+int pb_deconv_censored_variant(int T, int K, int is_f64, int nb_iter, int early_stopping, int wind, int is_auto,
+                               int *family);
+
 /* ---- A10: the theta step alone / hrf_estim (pybold/bold_signal.py:217-239, :329-334) --
  * theta[v] <- bounded local minimiser of 0.5||y_v - h(theta)*z_v||^2 from theta0;
  * out_h [V,K] = non-normalised taps at the minimiser; out_cost [V] = the cost there. */

@@ -58,6 +58,15 @@ _OPS = {
     "pb_deconv_lbda_path": [_P, _P, _P, _P, c_int, c_int, _P, _P, _P, _P, _P, c_int64, c_int, c_int, _P],
     "pb_deconv_lbda_path_ex": [_P, _P, c_int64, _P, c_int64, _P, c_int, c_int, c_int, c_int, c_double,
                                _P, _P, _P, _P, _P, _P, _P, c_int64, c_int, c_int, _P],
+    "pb_deconv_censored": [_P, _P, c_int64, _P, c_int64, _P, c_int64, _P, _P, c_int64, c_int, c_int, c_int,
+                           c_double, _P, _P, _P, _P, _P, c_int64, c_int, c_int, _P],
+    "pb_deconv_auto_censored": [_P, _P, c_int64, _P, c_int64, _P, c_int64, _P, c_int64, c_int, c_int, c_int, c_int,
+                                c_double, _P, _P, _P, _P, _P, _P, _P, _P, c_int64, c_int, c_int, _P],
+    "pb_deconv_lbda_path_censored": [_P, _P, c_int64, _P, c_int64, _P, c_int, _P, c_int64, c_int, c_int, c_int,
+                                     c_double, _P, _P, _P, _P, _P, _P, _P, c_int64, c_int, c_int, _P],
+    "pb_lipschitz_power_censored": [_P, c_int64, _P, c_int64, _P, c_int64, c_int, c_double, _P, c_int64, c_int,
+                                    c_int, _P],
+    "pb_mad_daub_noise_est_censored": [_P, _P, c_int64, c_double, _P, c_int64, c_int, _P],
     "pb_bd": [_P, c_double, c_double, _P, c_int64, _P, c_int64, _P, c_double, c_double,
               c_int, c_int, c_int, c_double, _P, _P, _P, _P, _P, _P, _P, _P, _P,
               c_int64, c_int, c_int, _P],
@@ -84,6 +93,8 @@ _PLAIN = {
     "pb_hrf_len_ex": ([c_double, c_double, c_double], c_int),
     "pb_bd_wave_voxels": ([c_int, c_int, c_int, c_int], c_int),
     "pb_deconv_variant": ([c_int, c_int, c_int, c_int, c_int, c_int, c_int, ctypes.POINTER(c_int)], c_int),
+    "pb_deconv_censored_variant": ([c_int, c_int, c_int, c_int, c_int, c_int, c_int, ctypes.POINTER(c_int)],
+                                   c_int),
     "pb_bd_variant": ([c_int, c_int, c_int, c_int, c_int, c_int, ctypes.POINTER(c_int)], c_int),
     "pb_bench_fma_f32": ([_P, c_int, c_int, _P], c_int),
     "pb_copy_async": ([_P, _P, ctypes.c_size_t, _P], c_int),

@@ -35,7 +35,7 @@ def _as_batch(y, dtype):
 
 
 def deconv_batch(y, hrf, lbda, lipschitz, w0=None, early_stopping=True, tol=1.0e-6, wind=6,
-                 nb_iter=1000, events=None, active=None, out=None, trace=True):
+                 nb_iter=1000, events=None, active=None, out=None, trace=True, censor=None):
     """Device entry point: tensors in, tensors out.  Returns (x, z, diff_z, J_raw, n_iter).
 
     ``J_raw[v, k]`` is the un-normalised cost of iteration k (NaN past ``n_iter[v]``);
@@ -43,6 +43,9 @@ def deconv_batch(y, hrf, lbda, lipschitz, w0=None, early_stopping=True, tol=1.0e
     ``events=(e0, e1)``: CUDA events recorded immediately around the solver launch (benchmarks).
     ``active`` (uint8 ``[V]``): voxels with 0 are skipped, their rows of the outputs stay as they are;
     ``out=(x, z, diff_z, n_iter)`` reuses output tensors; ``trace=False`` skips the cost trace (J is None).
+    ``censor`` (``[T]`` or ``[V, T]``, non-zero = scan left out of the data term, :mod:`pybold_b200.censor`): J is
+    the cost of the masked residual and ``lipschitz`` should be the censored operator's; it does not combine with
+    ``active``.  A device mask is not checked for all-censored voxels (that would wait on the device).
     """
     V, T = y.shape
     dtype, dev = y.dtype, y.device
@@ -72,10 +75,22 @@ def deconv_batch(y, hrf, lbda, lipschitz, w0=None, early_stopping=True, tol=1.0e
     J = torch.full((V, nb_iter), float("nan"), dtype=dtype, device=dev) if trace else None
     if active is not None and (active.dtype != torch.uint8 or active.numel() != V or active.device != dev):
         raise ValueError("active must be a uint8 tensor with one entry per voxel on %s" % dev)
+    if censor is not None:
+        from .censor import censor_mask
+        if active is not None:
+            raise ValueError("censor does not combine with active")
+        cm, c_stride = censor_mask(censor, V, T, dev, check=False)
+        if J is None:                   # the censored entry always writes a trace
+            J_buf = torch.empty((V, nb_iter), dtype=dtype, device=dev)
     with torch.cuda.device(dev):        # the C side sizes its grid for, and launches on, the current device
         if events is not None:
             events[0].record()
-        if active is None and trace:
+        if censor is not None:
+            rc = _lib.fn("pb_deconv_censored", dtype)(
+                ptr(y), ptr(hrf), h_stride, ptr(Lc), L_stride, ptr(lb), lb_stride, ptr(w0), ptr(cm), c_stride,
+                int(nb_iter), int(bool(early_stopping)), int(wind), float(tol),
+                ptr(x), ptr(z), ptr(dz), ptr(J if J is not None else J_buf), ptr(n_iter), V, T, K, stream_ptr())
+        elif active is None and trace:
             rc = _lib.fn("pb_deconv", dtype)(
                 ptr(y), ptr(hrf), h_stride, ptr(Lc), L_stride, ptr(lb), lb_stride, ptr(w0),
                 int(nb_iter), int(bool(early_stopping)), int(wind), float(tol),
@@ -92,7 +107,7 @@ def deconv_batch(y, hrf, lbda, lipschitz, w0=None, early_stopping=True, tol=1.0e
 
 
 def deconv_auto_batch(y, hrf, sigma, lipschitz, nb_iter=1000, nb_sub_iter=1000, early_stopping=True, tol=1.0e-6,
-                      wind=6):
+                      wind=6, censor=None):
     """Device entry point of ``deconv(lbda=None)`` (pybold/bold_signal.py:99-214): tensors in, dict of tensors out.
 
     ``y`` is ``[V, T]`` on the device, ``hrf`` ``[K]`` (shared) or ``[V, K]``, ``sigma`` (noise level) and
@@ -103,6 +118,10 @@ def deconv_auto_batch(y, hrf, sigma, lipschitz, nb_iter=1000, nb_sub_iter=1000, 
     Returns ``{x, z, diff_z}`` (``[V, T]``, final pass), ``{J, R, G}`` (``[V, nb_iter]``, one entry per outer
     iteration, NaN past the voxel's outer count), ``lbda`` (``[V]``, the lambda of the final pass) and
     ``n_outer`` (``[V]`` int32, outer iterations done).
+
+    ``censor`` (``[T]`` or ``[V, T]``, :mod:`pybold_b200.censor`): R is ``||M (x - y)||^2`` and the noise target
+    ``n_kept sigma^2``; a device mask keeps the call free of host synchronisation (it is then not checked for
+    all-censored voxels).
     """
     V, T = y.shape
     dtype, dev = y.dtype, y.device
@@ -119,6 +138,17 @@ def deconv_auto_batch(y, hrf, sigma, lipschitz, nb_iter=1000, nb_sub_iter=1000, 
     out.update({k: torch.empty((V, nb_iter), dtype=dtype, device=dev) for k in ("J", "R", "G")})
     out["lbda"] = torch.empty(V, dtype=dtype, device=dev)
     out["n_outer"] = torch.empty(V, dtype=torch.int32, device=dev)
+    if censor is not None:
+        from .censor import censor_mask
+        cm, c_stride = censor_mask(censor, V, T, dev, check=False)
+        with torch.cuda.device(dev):
+            rc = _lib.fn("pb_deconv_auto_censored", dtype)(
+                ptr(y), ptr(hrf), h_stride, ptr(Lc), L_stride, ptr(sg), sg_stride, ptr(cm), c_stride, int(nb_iter),
+                int(nb_sub_iter), int(bool(early_stopping)), int(wind), float(tol), ptr(out["x"]), ptr(out["z"]),
+                ptr(out["diff_z"]), ptr(out["J"]), ptr(out["R"]), ptr(out["G"]), ptr(out["lbda"]),
+                ptr(out["n_outer"]), V, T, K, stream_ptr())
+        _lib.check(rc, "pb_deconv_auto_censored")
+        return out
     with torch.cuda.device(dev):
         rc = _lib.fn("pb_deconv_auto", dtype)(
             ptr(y), ptr(hrf), h_stride, ptr(Lc), L_stride, ptr(sg), sg_stride, int(nb_iter), int(nb_sub_iter),
@@ -139,15 +169,20 @@ def _lipschitz_cst(est, dtype):
 
 
 def deconv(y, t_r, hrf, lbda=None, early_stopping=True, tol=1.0e-6,  # noqa
-           wind=6, nb_iter=1000, nb_sub_iter=1000, verbose=0, x0=None, sigma=None, dtype=None):
+           wind=6, nb_iter=1000, nb_sub_iter=1000, verbose=0, x0=None, sigma=None, dtype=None, censor=None):
     """Sparse deconvolution with a known HRF (pybold/bold_signal.py:13-214).
 
     Returns ``(x, z, diff_z, J, R, G)`` like the reference: with a float ``lbda`` J is the cost
     trace normalised by its first entry and R, G are None (bold_signal.py:97).  ``lbda=None``
     (noise-constrained lambda, bold_signal.py:99-214) estimates the noise level like the reference
     (db3 MAD, utils.py:16-25, on the device) unless ``sigma=`` is given.
-    Extra keyword arguments: ``x0`` (power-iteration start), ``sigma``, ``dtype``.  float64 input
+    Extra keyword arguments: ``x0`` (power-iteration start), ``sigma``, ``dtype``, ``censor``.  float64 input
     (the reference's type) selects the FP64 build, float32 input or ``dtype=np.float32`` the FP32 one.
+
+    ``censor`` (``[T]`` or ``[V, T]`` 0/1 mask, NumPy or torch; :mod:`pybold_b200.censor`) leaves the flagged scans
+    out of the data term: ``J = 1/2 ||M (A w - y)||^2 + lbda ||w||_1``, y may hold NaN there, x = A w on every scan,
+    the Lipschitz constant is the censored operator's, and ``lbda=None`` targets ``n_kept sigma^2`` with sigma from
+    the detail coefficients that touch no censored scan.  ``ValueError`` for a voxel with every scan censored.
     """
     dtype = pick_dtype(y, hrf, dtype=dtype)
     yb, one_d = _as_batch(y, dtype)
@@ -157,16 +192,22 @@ def deconv(y, t_r, hrf, lbda=None, early_stopping=True, tol=1.0e-6,  # noqa
     # bold_signal.py:52 -- 0.9 x power-iteration estimate, start vector from the global RNG
     if x0 is None:
         x0 = np.random.randn(T)
-    est = spectral_radius_est(H, (T,), x0=to_device(x0, dtype))
-    lipschitz = _lipschitz_cst(est, dtype)
+    cm = None
+    if censor is not None:
+        from .censor import censor_mask, lipschitz_censored
+        cm, c_stride = censor_mask(censor, V, T, yb.device)
+        lipschitz, _ = lipschitz_censored(hd, x0, cm, c_stride, dtype, T)
+    else:
+        est = spectral_radius_est(H, (T,), x0=to_device(x0, dtype))
+        lipschitz = _lipschitz_cst(est, dtype)
 
     if lbda is None:
         from .noise import deconv_auto_lbda
         return deconv_auto_lbda(y, yb, one_d, hd, lipschitz, sigma, early_stopping, tol, wind,
-                                nb_iter, nb_sub_iter)
+                                nb_iter, nb_sub_iter, censor=cm)
 
     x, z, dz, J, n_iter = deconv_batch(yb, hd, lbda, lipschitz, None, early_stopping, tol, wind,
-                                       nb_iter)
+                                       nb_iter, censor=cm)
     Jn = J / (J[:, :1] + 1.0e-30)                                  # bold_signal.py:97
     if one_d:
         n = int(n_iter[0])
@@ -183,10 +224,11 @@ def deconv(y, t_r, hrf, lbda=None, early_stopping=True, tol=1.0e-6,  # noqa
 FIT_SCRATCH_BYTES = 4 << 30
 
 
-def _path_problem(y, hrf, lbdas, x0, dtype):
+def _path_problem(y, hrf, lbdas, x0, dtype, censor=None):
     """Device inputs of the regularisation path: the rows of ``y``, the taps (``[K]`` shared or ``[V, K]``), the
     Lipschitz constants ``0.9 x spectral_radius_est`` from ``x0`` -- per voxel with ``[V, K]`` taps, the constants
-    ``deconv(y, t_r, hrf, x0=x0)`` uses -- and the lambdas, with the element strides of the C ABI."""
+    ``deconv(y, t_r, hrf, x0=x0)`` uses -- and the lambdas, with the element strides of the C ABI.  With ``censor``
+    also the mask and its stride, and the constants of the censored operators."""
     dtype = pick_dtype(y, hrf, dtype=dtype)
     yb, _ = _as_batch(y, dtype)
     yb = yb.contiguous()
@@ -202,16 +244,31 @@ def _path_problem(y, hrf, lbdas, x0, dtype):
     lb = upload(np.asarray(lbdas, dtype=np.float64).reshape(-1), dtype, yb.device)
     if x0 is None:
         x0 = np.random.randn(T)
+    if censor is not None:
+        from .censor import censor_mask, lipschitz_censored
+        cm, c_stride = censor_mask(censor, V, T, yb.device)
+        Lc, L_stride = lipschitz_censored(hd, x0, cm, c_stride, dtype, T)
+        return yb, hd, h_stride, Lc, L_stride, lb, (cm, c_stride)
     est = spectral_radius_est(ConvAndLinear(DiscretInteg(), hd, dim_in=T), (T,), x0=to_device(x0, dtype))
     Lc, L_stride = per_voxel(_lipschitz_cst(est, dtype), V, dtype, yb.device, "lipschitz")
-    return yb, hd, h_stride, Lc, L_stride, lb
+    return yb, hd, h_stride, Lc, L_stride, lb, None
 
 
-def _path_launch(yb, hd, h_stride, Lc, L_stride, lb, nb_iter, early_stopping, wind, tol, sol, J, r, g, n_iter):
+def _path_launch(yb, hd, h_stride, Lc, L_stride, lb, nb_iter, early_stopping, wind, tol, sol, J, r, g, n_iter,
+                 censor=None):
     """One ``pb_deconv_lbda_path_ex`` launch: every lambda of ``lb`` x every row of ``yb``, problem (l, v) at
     flat index l * V + v of the outputs.  ``sol`` = (x, z, diff_z) buffers of n_lbda * V * T elements; ``J``
-    (n_lbda * V * nb_iter), ``r`` and ``g`` may be None; ``n_iter`` holds n_lbda * V int32."""
+    (n_lbda * V * nb_iter), ``r`` and ``g`` may be None; ``n_iter`` holds n_lbda * V int32.  ``censor`` = (mask,
+    stride) of the rows of ``yb``: ``pb_deconv_lbda_path_censored`` instead."""
     V, T = yb.shape
+    if censor is not None:
+        with torch.cuda.device(yb.device):
+            rc = _lib.fn("pb_deconv_lbda_path_censored", yb.dtype)(
+                ptr(yb), ptr(hd), h_stride, ptr(Lc), L_stride, ptr(lb), lb.numel(), ptr(censor[0]), censor[1],
+                int(nb_iter), int(bool(early_stopping)), int(wind), float(tol), ptr(sol[0]), ptr(sol[1]),
+                ptr(sol[2]), ptr(J), ptr(r), ptr(g), ptr(n_iter), V, T, hd.shape[-1], stream_ptr())
+        _lib.check(rc, "pb_deconv_lbda_path_censored")
+        return
     with torch.cuda.device(yb.device):
         rc = _lib.fn("pb_deconv_lbda_path_ex", yb.dtype)(
             ptr(yb), ptr(hd), h_stride, ptr(Lc), L_stride, ptr(lb), lb.numel(), int(nb_iter),
@@ -221,7 +278,7 @@ def _path_launch(yb, hd, h_stride, Lc, L_stride, lb, nb_iter, early_stopping, wi
 
 
 def deconv_lbda_path(y, t_r, hrf, lbdas, nb_iter=200, x0=None, dtype=None, max_problems=1 << 21,
-                     early_stopping=False, tol=1.0e-6, wind=6):
+                     early_stopping=False, tol=1.0e-6, wind=6, censor=None):
     """Regularisation path: ``deconv(y, t_r, hrf, lbda=l, nb_iter=nb_iter, x0=x0, early_stopping=...,
     tol=..., wind=...)`` for every lambda of ``lbdas`` and every voxel of ``y[V, T]`` -- the grid search of
     examples/icassp_2019/validation.py batched over (lambda, voxel) instead of looping (BASELINE.json configs[4]).
@@ -237,8 +294,10 @@ def deconv_lbda_path(y, t_r, hrf, lbdas, nb_iter=200, x0=None, dtype=None, max_p
     and writes straight into the results; more than ``max_problems`` pairs are cut into launches of whole
     lambdas.  The solutions take ``3 n_lbda V T`` elements on the device: to choose lambda at whole-brain size,
     use :func:`deconv_lbda_path_fit`.
+
+    ``censor`` (``[T]`` or ``[V, T]``): every problem is the censored ``deconv(..., censor=censor)`` of its voxel.
     """
-    yb, hd, h_stride, Lc, L_stride, lb = _path_problem(y, hrf, lbdas, x0, dtype)
+    yb, hd, h_stride, Lc, L_stride, lb, cz = _path_problem(y, hrf, lbdas, x0, dtype, censor)
     V, T = yb.shape
     n_l = lb.numel()
     outs = [torch.empty((n_l, V, T), dtype=yb.dtype, device=yb.device) for _ in range(3)]
@@ -251,13 +310,13 @@ def deconv_lbda_path(y, t_r, hrf, lbdas, nb_iter=200, x0=None, dtype=None, max_p
     for l0 in range(0, n_l, per):
         l1 = min(l0 + per, n_l)
         _path_launch(yb, hd, h_stride, Lc, L_stride, lb[l0:l1], nb_iter, early_stopping, wind, tol,
-                     [o[l0:l1] for o in outs], J[l0:l1], None, None, n_iter[l0:l1])
+                     [o[l0:l1] for o in outs], J[l0:l1], None, None, n_iter[l0:l1], cz)
     J /= (J[:, :, :1] + 1.0e-30)                                   # bold_signal.py:97, in place
     return tuple(like_input(t, y) for t in outs) + (like_input(J, y),)
 
 
 def deconv_lbda_path_fit(y, t_r, hrf, lbdas, nb_iter=200, early_stopping=False, tol=1.0e-6, wind=6, x0=None,
-                         dtype=None):
+                         dtype=None, censor=None):
     """Data-fit and penalty terms of every (lambda, voxel) problem of :func:`deconv_lbda_path`, without
     keeping the solutions: what choosing lambda needs, at any number of voxels.
 
@@ -277,8 +336,16 @@ def deconv_lbda_path_fit(y, t_r, hrf, lbdas, nb_iter=200, early_stopping=False, 
         sigma = mad_daub_noise_est(y)                              # [V]
         lbda_v = np.asarray(lbdas)[np.argmin(np.abs(R - y.shape[1] * sigma ** 2), axis=0)]
         x, z, diff_z, J, _, _ = deconv(y, t_r, h, lbda=lbda_v, nb_iter=200, early_stopping=True, x0=x0)
+
+    With ``censor`` (``[T]`` or ``[V, T]``), ``R = ||M (x - y)||^2`` counts the kept scans only, so the target is
+    ``n_kept * sigma ** 2`` with ``n_kept = (censor == 0).sum(-1)`` and sigma from the kept detail coefficients::
+
+        R, G, n_iter = deconv_lbda_path_fit(y, t_r, h, lbdas, early_stopping=True, x0=x0, censor=censor)
+        sigma = mad_daub_noise_est_censored(yb, cm, stride)        # pybold_b200.censor
+        lbda_v = np.asarray(lbdas)[np.argmin(np.abs(R - n_kept * sigma ** 2), axis=0)]
+        x, z, diff_z, J, _, _ = deconv(y, t_r, h, lbda=lbda_v, early_stopping=True, x0=x0, censor=censor)
     """
-    yb, hd, h_stride, Lc, L_stride, lb = _path_problem(y, hrf, lbdas, x0, dtype)
+    yb, hd, h_stride, Lc, L_stride, lb, cz = _path_problem(y, hrf, lbdas, x0, dtype, censor)
     V, T = yb.shape
     n_l = lb.numel()
     dev = yb.device
@@ -296,8 +363,9 @@ def deconv_lbda_path_fit(y, t_r, hrf, lbdas, nb_iter=200, early_stopping=False, 
     for v0 in range(0, V, vc):
         v1 = min(v0 + vc, V)
         n = v1 - v0
+        czr = None if cz is None else (cz[0][v0:v1] if cz[1] else cz[0], cz[1])
         _path_launch(yb[v0:v1], hd[v0:v1] if h_stride else hd, h_stride, Lc[v0:v1] if L_stride else Lc,
-                     L_stride, lb, nb_iter, early_stopping, wind, tol, scratch, None, r, g, n_it)
+                     L_stride, lb, nb_iter, early_stopping, wind, tol, scratch, None, r, g, n_it, czr)
         R[:, v0:v1] = r[:n_l * n].view(n_l, n)
         G[:, v0:v1] = g[:n_l * n].view(n_l, n)
         n_iter[:, v0:v1] = n_it[:n_l * n].view(n_l, n)

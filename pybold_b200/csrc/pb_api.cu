@@ -301,12 +301,14 @@ int run_spm_hrf_ex(const real *theta, double t_r, double dur, int normalized, co
     return last_error();
 }
 
+// censor != null: the power iteration of the censored operator A^T M A (censor_stride 0: one mask for the batch)
 template <typename real>
 int run_lipschitz_power(const real *h, int64_t h_stride, const real *x0, int64_t x0_stride,
                         int nb_iter, double tol, real *out_L, int64_t V, int T, int K,
-                        pb_stream_t stream) {
+                        pb_stream_t stream, const unsigned char *censor = nullptr, int64_t censor_stride = 0) {
     if (V == 0) return PB_OK;
-    if (!h || !x0 || !out_L || V < 0 || T <= 0 || K <= 0 || nb_iter < 1) return PB_ERR_INVALID_ARG;
+    if (!h || !x0 || !out_L || V < 0 || T <= 0 || K <= 0 || nb_iter < 1 || censor_stride < 0)
+        return PB_ERR_INVALID_ARG;
     if (T > PB_MAX_T || K > PB_MAX_OP_K) return PB_ERR_UNSUPPORTED;
     if (V == 0) return PB_OK;
     DeviceInfo d = device_info();
@@ -314,12 +316,15 @@ int run_lipschitz_power(const real *h, int64_t h_stride, const real *x0, int64_t
     pb::GenLayout lay = pb::GenLayout::make(T, K, 0, false);
     LaunchPlan p = plan_launch(d, 0, lay.warp_bytes(sizeof(real)), V, 8);
     if (!p.warps) return PB_ERR_UNSUPPORTED;
-    auto kern = pb::lipschitz_power_kernel<real>;
-    int e = set_smem(kern, p.smem);
-    if (e) return e;
-    kern<<<p.grid, p.warps * 32, p.smem, (cudaStream_t)stream>>>(h, h_stride, x0, x0_stride, nb_iter,
-                                                                 tol, out_L, V, T, K, lay);
-    return last_error();
+    auto go = [&](auto kern) {
+        int e = set_smem(kern, p.smem);
+        if (e) return e;
+        kern<<<p.grid, p.warps * 32, p.smem, (cudaStream_t)stream>>>(h, h_stride, x0, x0_stride, nb_iter,
+                                                                     tol, out_L, V, T, K, lay,
+                                                                     pb::Censor{censor, censor_stride});
+        return last_error();
+    };
+    return censor ? go(pb::lipschitz_power_kernel<real, true>) : go(pb::lipschitz_power_kernel<real, false>);
 }
 
 template <typename real>
@@ -375,11 +380,13 @@ int run_toeplitz(const real *k, int klen, real *out, int64_t dim_out, int64_t di
 }
 
 // the register-tiled variant the dispatch chooses (pb_fast_registry.cu), else the generic kernel; a.nb_outer > 0
-// selects the deconv(lbda=None) instances.  V == 0 launches nothing: *id / *family report the kernel a launch
-// would run (pb_deconv_variant).
+// selects the deconv(lbda=None) instances, cz (scan censoring) the censored ones.  V == 0 launches nothing: *id /
+// *family report the kernel a launch would run (pb_deconv_variant, pb_deconv_censored_variant).
 template <typename real>
-int launch_deconv(const pb::DeconvArgs<real> &a, pb_stream_t stream, int *id = nullptr, int *family = nullptr) {
-    int rc = pb::fast_deconv_dispatch(a, (cudaStream_t)stream, id, family);
+int launch_deconv(const pb::DeconvArgs<real> &a, pb_stream_t stream, int *id = nullptr, int *family = nullptr,
+                  const pb::Censor *cz = nullptr) {
+    int rc = cz ? pb::fast_deconv_censored_dispatch(a, *cz, (cudaStream_t)stream, id, family)
+                : pb::fast_deconv_dispatch(a, (cudaStream_t)stream, id, family);
     if (rc != pb::FAST_NO_MATCH) return rc;
     DeviceInfo d = device_info();
     if (d.err) return d.err;
@@ -396,9 +403,12 @@ int launch_deconv(const pb::DeconvArgs<real> &a, pb_stream_t stream, int *id = n
     auto go = [&](auto kern) {
         int e = set_smem(kern, p.smem);
         if (e) return e;
-        kern<<<p.grid, p.warps * 32, p.smem, (cudaStream_t)stream>>>(a, lay);
+        kern<<<p.grid, p.warps * 32, p.smem, (cudaStream_t)stream>>>(a, lay, cz ? *cz : pb::Censor{});
         return last_error();
     };
+    if (cz)
+        return a.nb_outer > 0 ? go(pb::generic_deconv_kernel<real, true, true>)
+                              : go(pb::generic_deconv_kernel<real, false, true>);
     return a.nb_outer > 0 ? go(pb::generic_deconv_kernel<real, true>) : go(pb::generic_deconv_kernel<real, false>);
 }
 
@@ -416,34 +426,37 @@ void set_routing(pb::DeconvArgs<real> &a, unsigned int *(*queue)()) {
 }
 
 template <typename real>
-int run_deconv(pb::DeconvArgs<real> a, pb_stream_t stream) {
+int run_deconv(pb::DeconvArgs<real> a, pb_stream_t stream, const pb::Censor *cz = nullptr) {
     if (a.V == 0) return PB_OK;
+    if (cz && (!cz->m || cz->stride < 0)) return PB_ERR_INVALID_ARG;
     if (!a.y || !a.h || !a.L || !a.lbda || !a.out_x || !a.out_z || !a.out_dz ||
         !a.out_niter || a.V < 0 || a.T <= 0 || a.K <= 0 || a.nb_iter < 1 || a.wind < 0)
         return PB_ERR_INVALID_ARG;
     if (a.T > PB_MAX_T || a.K > PB_MAX_K || a.nb_iter > PB_MAX_ITER) return PB_ERR_UNSUPPORTED;
     if (a.V == 0) return PB_OK;
     set_routing(a, queue_slot);
-    return launch_deconv(a, stream);
+    return launch_deconv(a, stream, nullptr, nullptr, cz);
 }
 
 // deconv(lbda=None): the noise loop runs inside the kernel, nb_outer outer iterations at most, nb_iter inner
 // ones per pass
 template <typename real>
-int run_deconv_auto(pb::DeconvArgs<real> a, pb_stream_t stream) {
+int run_deconv_auto(pb::DeconvArgs<real> a, pb_stream_t stream, const pb::Censor *cz = nullptr) {
     if (a.V == 0) return PB_OK;
+    if (cz && (!cz->m || cz->stride < 0)) return PB_ERR_INVALID_ARG;
     if (!a.y || !a.h || !a.L || !a.sigma || !a.out_x || !a.out_z || !a.out_dz || a.V < 0 || a.T <= 0 ||
         a.K <= 0 || a.nb_iter < 1 || a.nb_outer < 1 || a.wind < 0 || a.h_stride < 0 || a.L_stride < 0 ||
         a.sigma_stride < 0)
         return PB_ERR_INVALID_ARG;
     if (a.T > PB_MAX_T || a.K > PB_MAX_K || a.nb_iter > PB_MAX_ITER) return PB_ERR_UNSUPPORTED;
     set_routing(a, queue_slot);
-    return launch_deconv(a, stream);
+    return launch_deconv(a, stream, nullptr, nullptr, cz);
 }
 
-// pb_deconv_variant: the routing of a deconv call with V = 0 (nothing is launched)
+// pb_deconv_variant / pb_deconv_censored_variant: the routing of a deconv call with V = 0 (nothing is launched)
 template <typename real>
-int deconv_variant(int T, int K, int nb_iter, int early_stopping, int wind, int is_auto, int *family) {
+int deconv_variant(int T, int K, int nb_iter, int early_stopping, int wind, int is_auto, int *family,
+                   bool censored = false) {
     if (!family || T <= 0 || K <= 0 || nb_iter < 1 || wind < 0) return PB_ERR_INVALID_ARG;
     if (T > PB_MAX_T || K > PB_MAX_K || nb_iter > PB_MAX_ITER) return PB_ERR_UNSUPPORTED;
     pb::DeconvArgs<real> a{};
@@ -461,7 +474,9 @@ int deconv_variant(int T, int K, int nb_iter, int early_stopping, int wind, int 
         return &placeholder;
     });
     int id = 0;
-    const int rc = launch_deconv(a, nullptr, &id, family);
+    static const unsigned char placeholder_mask = 0;
+    const pb::Censor cz{&placeholder_mask, 0};
+    const int rc = launch_deconv(a, nullptr, &id, family, censored ? &cz : nullptr);
     if (rc > 0) {               // a CUDA error
         cudaGetLastError();
         return PB_ERR_NO_DEVICE;
@@ -642,6 +657,28 @@ int run_mad(const real *x, double c, real *out, int64_t V, int T, pb_stream_t st
     return last_error();
 }
 
+template <typename real>
+int run_mad_censored(const real *y, const unsigned char *censor, int64_t censor_stride, double c, real *out,
+                     int64_t V, int T, pb_stream_t stream) {
+    if (V == 0) return PB_OK;
+    if (!y || !censor || !out || V < 0 || T <= 0 || censor_stride < 0 || !(c > 0.0)) return PB_ERR_INVALID_ARG;
+    DeviceInfo d = device_info();
+    if (d.err) return d.err;
+    const int nmax = pb::noise_detail_len(T);
+    const size_t warp_bytes = (size_t)nmax * sizeof(double);
+    if (warp_bytes > (size_t)d.max_smem_optin) return PB_ERR_UNSUPPORTED;
+    int warps = (int)((size_t)d.max_smem_optin / 2 / warp_bytes);
+    warps = warps < 1 ? 1 : (warps > 8 ? 8 : warps);
+    const size_t smem = (size_t)warps * warp_bytes;
+    auto kern = pb::mad_daub_censored_kernel<real>;
+    int e = set_smem(kern, smem);
+    if (e) return e;
+    const int64_t need = (V + warps - 1) / warps, cap = (int64_t)d.sm_count * 2;
+    kern<<<(int)(need < cap ? need : cap), warps * 32, smem, (cudaStream_t)stream>>>(
+        y, c, out, V, T, nmax, pb::Censor{censor, censor_stride});
+    return last_error();
+}
+
 // FP32 FMA-pipe ceiling: 16 independent chains a = a * m + c per thread (one register read per FFMA, the
 // multiplier and the addend sit in the operand-reuse cache); launch with 4 CTAs of 256 threads per SM.
 // Best of the variants in tools/exp_fma.cu (profiles/r01_fma_microbench.txt: 70.7 Tflop/s of 74.4 nominal).
@@ -704,6 +741,12 @@ int pb_deconv_variant(int T, int K, int is_f64, int nb_iter, int early_stopping,
                   : deconv_variant<float>(T, K, nb_iter, early_stopping, wind, is_auto, family);
 }
 
+int pb_deconv_censored_variant(int T, int K, int is_f64, int nb_iter, int early_stopping, int wind, int is_auto,
+                               int *family) {
+    return is_f64 ? deconv_variant<double>(T, K, nb_iter, early_stopping, wind, is_auto, family, true)
+                  : deconv_variant<float>(T, K, nb_iter, early_stopping, wind, is_auto, family, true);
+}
+
 int pb_bd_variant(int T, int K, int is_f64, int nb_iter, int early_stopping, int wind, int *family) {
     return is_f64 ? bd_variant<double>(T, K, nb_iter, early_stopping, wind, family)
                   : bd_variant<float>(T, K, nb_iter, early_stopping, wind, family);
@@ -759,6 +802,14 @@ int pb_hrf_len_ex(double t_r, double dur, double dt) {
                                  double tol, REAL *out_L, int64_t V, int T, int K, pb_stream_t s) {    \
         return run_lipschitz_power<REAL>(h, hs, x0, xs, nb_iter, tol, out_L, V, T, K, s);              \
     }                                                                                                  \
+    int pb_lipschitz_power_censored_##SUF(const REAL *h, int64_t hs, const REAL *x0, int64_t xs,       \
+                                          const unsigned char *censor, int64_t censor_stride,          \
+                                          int nb_iter, double tol, REAL *out_L, int64_t V, int T,      \
+                                          int K, pb_stream_t s) {                                      \
+        if (!censor && V != 0) return PB_ERR_INVALID_ARG;                                              \
+        return run_lipschitz_power<REAL>(h, hs, x0, xs, nb_iter, tol, out_L, V, T, K, s, censor,       \
+                                         censor_stride);                                               \
+    }                                                                                                  \
     int pb_lipschitz_frob_##SUF(const REAL *h, int64_t hs, REAL *out_L, int64_t V, int T, int K,       \
                                 pb_stream_t s) {                                                       \
         return run_lipschitz_frob<REAL>(h, hs, out_L, V, T, K, s);                                     \
@@ -776,6 +827,22 @@ int pb_hrf_len_ex(double t_r, double dur, double dt) {
         a.T = T; a.K = K;                                                                              \
         if (!out_J && V != 0) return PB_ERR_INVALID_ARG;                                               \
         return run_deconv<REAL>(a, s);                                                                 \
+    }                                                                                                  \
+    int pb_deconv_censored_##SUF(const REAL *y, const REAL *h, int64_t h_stride, const REAL *L,        \
+                                 int64_t L_stride, const REAL *lbda, int64_t lbda_stride, const REAL *w0,\
+                                 const unsigned char *censor, int64_t censor_stride, int nb_iter,      \
+                                 int early_stopping, int wind, double tol, REAL *out_x, REAL *out_z,   \
+                                 REAL *out_dz, REAL *out_J, int32_t *out_niter, int64_t V, int T,      \
+                                 int K, pb_stream_t s) {                                               \
+        pb::DeconvArgs<REAL> a;                                                                        \
+        a.y = y; a.h = h; a.h_stride = h_stride; a.L = L; a.L_stride = L_stride; a.lbda = lbda;        \
+        a.lbda_stride = lbda_stride; a.w0 = w0; a.nb_iter = nb_iter;                                   \
+        a.early_stopping = early_stopping; a.wind = wind; a.tol = tol; a.out_x = out_x;                \
+        a.out_z = out_z; a.out_dz = out_dz; a.out_J = out_J; a.out_niter = out_niter; a.V = V;         \
+        a.T = T; a.K = K;                                                                              \
+        if (!out_J && V != 0) return PB_ERR_INVALID_ARG;                                               \
+        const pb::Censor cz{censor, censor_stride};                                                    \
+        return run_deconv<REAL>(a, s, &cz);                                                            \
     }                                                                                                  \
     int pb_deconv_masked_##SUF(const REAL *y, const REAL *h, int64_t h_stride, const REAL *L,          \
                                int64_t L_stride, const REAL *lbda, int64_t lbda_stride, const REAL *w0, \
@@ -804,6 +871,42 @@ int pb_hrf_len_ex(double t_r, double dur, double dt) {
         a.sigma = sigma; a.sigma_stride = sigma_stride; a.nb_outer = nb_iter; a.out_R = out_R;         \
         a.out_G = out_G; a.out_lbda = out_lbda; a.out_nouter = out_nouter;                             \
         return run_deconv_auto<REAL>(a, s);                                                            \
+    }                                                                                                  \
+    int pb_deconv_auto_censored_##SUF(const REAL *y, const REAL *h, int64_t h_stride, const REAL *L,   \
+                                      int64_t L_stride, const REAL *sigma, int64_t sigma_stride,       \
+                                      const unsigned char *censor, int64_t censor_stride, int nb_iter, \
+                                      int nb_sub_iter, int early_stopping, int wind, double tol,       \
+                                      REAL *out_x, REAL *out_z, REAL *out_dz, REAL *out_J,             \
+                                      REAL *out_R, REAL *out_G, REAL *out_lbda, int32_t *out_nouter,   \
+                                      int64_t V, int T, int K, pb_stream_t s) {                        \
+        pb::DeconvArgs<REAL> a;                                                                        \
+        a.y = y; a.h = h; a.h_stride = h_stride; a.L = L; a.L_stride = L_stride; a.lbda = nullptr;     \
+        a.lbda_stride = 0; a.w0 = nullptr; a.nb_iter = nb_sub_iter; a.early_stopping = early_stopping; \
+        a.wind = wind; a.tol = tol; a.out_x = out_x; a.out_z = out_z; a.out_dz = out_dz;               \
+        a.out_J = out_J; a.out_niter = nullptr; a.V = V; a.T = T; a.K = K;                             \
+        a.sigma = sigma; a.sigma_stride = sigma_stride; a.nb_outer = nb_iter; a.out_R = out_R;         \
+        a.out_G = out_G; a.out_lbda = out_lbda; a.out_nouter = out_nouter;                             \
+        const pb::Censor cz{censor, censor_stride};                                                    \
+        return run_deconv_auto<REAL>(a, s, &cz);                                                       \
+    }                                                                                                  \
+    int pb_deconv_lbda_path_censored_##SUF(const REAL *y, const REAL *h, int64_t h_stride,             \
+                                           const REAL *L, int64_t L_stride, const REAL *lbdas,         \
+                                           int n_lbda, const unsigned char *censor,                    \
+                                           int64_t censor_stride, int nb_iter, int early_stopping,     \
+                                           int wind, double tol, REAL *out_x, REAL *out_z,             \
+                                           REAL *out_dz, REAL *out_J, REAL *out_r, REAL *out_g,        \
+                                           int32_t *out_niter, int64_t V, int T, int K,                \
+                                           pb_stream_t s) {                                            \
+        if (n_lbda < 0 || V < 0 || h_stride < 0 || L_stride < 0) return PB_ERR_INVALID_ARG;          \
+        pb::DeconvArgs<REAL> a;                                                                        \
+        a.y = y; a.h = h; a.h_stride = h_stride; a.L = L; a.L_stride = L_stride; a.lbda = lbdas;       \
+        a.lbda_stride = 0; a.w0 = nullptr; a.nb_iter = nb_iter; a.early_stopping = early_stopping;     \
+        a.wind = wind; a.tol = tol; a.out_x = out_x; a.out_z = out_z; a.out_dz = out_dz;               \
+        a.out_J = out_J; a.out_r = out_r; a.out_g = out_g; a.out_niter = out_niter;                    \
+        a.V = (int64_t)n_lbda * V; a.T = T; a.K = K;                                                   \
+        a.y_mod = V; a.lbda_div = V;                                                                   \
+        const pb::Censor cz{censor, censor_stride};                                                    \
+        return run_deconv<REAL>(a, s, &cz);                                                            \
     }                                                                                                  \
     int pb_deconv_lbda_path_ex_##SUF(const REAL *y, const REAL *h, int64_t h_stride, const REAL *L,    \
                                      int64_t L_stride, const REAL *lbdas, int n_lbda, int nb_iter,     \
@@ -878,6 +981,11 @@ int pb_hrf_len_ex(double t_r, double dur, double dt) {
     int pb_mad_daub_noise_est_##SUF(const REAL *y, double c, REAL *out_sigma, int64_t V, int T,        \
                                     pb_stream_t s) {                                                   \
         return run_mad<REAL, 1>(y, c, out_sigma, V, T, s);                                             \
+    }                                                                                                  \
+    int pb_mad_daub_noise_est_censored_##SUF(const REAL *y, const unsigned char *censor,              \
+                                             int64_t censor_stride, double c, REAL *out_sigma,         \
+                                             int64_t V, int T, pb_stream_t s) {                        \
+        return run_mad_censored<REAL>(y, censor, censor_stride, c, out_sigma, V, T, s);                \
     }                                                                                                  \
     int pb_hrf_estim_##SUF(const REAL *z, const REAL *y, double t_r, double hrf_dur,                   \
                            const REAL *theta0, int64_t theta0_stride, double lo, double hi,            \

@@ -110,6 +110,34 @@ static int deconv_dispatch(const DeconvArgs<real> &a, cudaStream_t s, int *id, i
     return FAST_NO_MATCH;
 }
 
+// Routing of a censored deconv call: the cheapest CTA row whose ok_censored takes (T, K), then (launch_deconv) the
+// generic kernel.  The group and warp kernels have no censored mode.
+template <typename real>
+static int deconv_censored_dispatch(const DeconvArgs<real> &a, const Censor &cz, cudaStream_t s, int *id, int *fam_out) {
+    const auto need = a.nb_outer > 0 ? &Variant<real>::deconv_auto_censored : &Variant<real>::deconv_censored;
+    const Variant<real> *best = nullptr;
+    long best_cost = 0;
+    for (const Variant<real> *v : variants(real())) {
+        if (!(v->*need) || !v->ok_censored(a.T, a.K)) continue;
+        const long c = cost(*v);
+        if (!best || c < best_cost) {
+            best = v;
+            best_cost = c;
+        }
+    }
+    if (best) {
+        const int rc = (best->*need)(a, cz, s);
+        if (rc != FAST_NO_MATCH) {
+            if (id) *id = encode(*best);
+            if (fam_out) *fam_out = family(*best);
+            return rc;
+        }
+    }
+    if (id) *id = 0;
+    if (fam_out) *fam_out = FAMILY_GENERIC;
+    return FAST_NO_MATCH;
+}
+
 // the queries describe bd without early stopping and ignore PB_DISABLE_GROUP
 template <typename real>
 static int variant_id(int T, int K) {
@@ -129,6 +157,12 @@ int fast_deconv_dispatch(const DeconvArgs<float> &a, cudaStream_t s, int *id, in
 }
 int fast_deconv_dispatch(const DeconvArgs<double> &a, cudaStream_t s, int *id, int *fam) {
     return deconv_dispatch<double>(a, s, id, fam);
+}
+int fast_deconv_censored_dispatch(const DeconvArgs<float> &a, const Censor &cz, cudaStream_t s, int *id, int *fam) {
+    return deconv_censored_dispatch<float>(a, cz, s, id, fam);
+}
+int fast_deconv_censored_dispatch(const DeconvArgs<double> &a, const Censor &cz, cudaStream_t s, int *id, int *fam) {
+    return deconv_censored_dispatch<double>(a, cz, s, id, fam);
 }
 int fast_bd_dispatch(const BdArgs<float> &a, cudaStream_t s, int *id, int *fam) {
     return bd_dispatch<float>(a, s, id, fam);

@@ -16,6 +16,12 @@ constexpr int FAST_NO_MATCH = -1000;
 // variant are those a launch would have
 int fast_deconv_dispatch(const DeconvArgs<float> &a, cudaStream_t stream, int *id = nullptr, int *family = nullptr);
 int fast_deconv_dispatch(const DeconvArgs<double> &a, cudaStream_t stream, int *id = nullptr, int *family = nullptr);
+// censored deconv (Censor, pb_generic.cuh): the cheapest CTA row with a censored entry point that serves (T, K); the
+// generic kernel is the caller's step after FAST_NO_MATCH
+int fast_deconv_censored_dispatch(const DeconvArgs<float> &a, const Censor &cz, cudaStream_t stream, int *id = nullptr,
+                                  int *family = nullptr);
+int fast_deconv_censored_dispatch(const DeconvArgs<double> &a, const Censor &cz, cudaStream_t stream, int *id = nullptr,
+                                  int *family = nullptr);
 int fast_bd_dispatch(const BdArgs<float> &a, cudaStream_t stream, int *id = nullptr, int *family = nullptr);
 int fast_bd_dispatch(const BdArgs<double> &a, cudaStream_t stream, int *id = nullptr, int *family = nullptr);
 // 0 = generic kernel, else lanes per voxel * 1000000 + R * 1000 + KMAX
@@ -45,6 +51,10 @@ struct Variant {
     int (*wave)(int nb_iter);
     // deconv(lbda=None): DeconvArgs::nb_outer > 0, the noise loop inside the kernel (pb_noise_loop.cuh)
     int (*deconv_auto)(const DeconvArgs<real> &, cudaStream_t);
+    // scan censoring (CTA rows only): the shapes a censored call may take, deconv and deconv(lbda=None)
+    bool (*ok_censored)(int T, int K);
+    int (*deconv_censored)(const DeconvArgs<real> &, const Censor &, cudaStream_t);
+    int (*deconv_auto_censored)(const DeconvArgs<real> &, const Censor &, cudaStream_t);
 };
 
 // Whether a kernel of `threads` threads and `smem` bytes of dynamic shared memory per CTA can run:

@@ -614,10 +614,14 @@ fast_bdc_kernel(BdArgs<real> p) {
 // Barriers per iteration: the four of fast_bdc_kernel; the cost of the previous iterate rides on B3, the Q5
 // test adds one CTA-wide pair of sums (two barriers), so every thread takes the same break.  With early stopping
 // the problems come from the work queue after the first (their iteration counts differ).
+// CENSOR: scan censoring (Censor, pb_generic.cuh).  A thread keeps the keep-bits of its R samples in one register;
+// censored y entries are zeroed at load, a select masks the residual after forward() (before the adjoint and the cost
+// sums), x = (A w - y) + y is formed from the unmasked final residual and the zeroed y, and the noise loop's target is
+// n_kept sigma^2 with n_kept one CTA-wide sum at voxel start.
 // ------------------------------------------------------------------------------------------------
-template <typename real, int R, int KMAX, int NW, int MINB, bool AUTO = false>
+template <typename real, int R, int KMAX, int NW, int MINB, bool AUTO = false, bool CENSOR = false>
 __global__ void __launch_bounds__(NW * 32, MINB)
-fast_deconvc_kernel(DeconvArgs<real> p, int ring_rows) {
+fast_deconvc_kernel(DeconvArgs<real> p, int ring_rows, Censor cz) {
     static_assert(R % 4 == 0, "R must be a multiple of 4 (vector halo exchange)");
     using L = CtaLayout<real, R, KMAX, NW>;
     using CT = CtaTile<real, R, KMAX, NW>;
@@ -687,19 +691,52 @@ fast_deconvc_kernel(DeconvArgs<real> p, int ring_rows) {
         if (p.is_active(v)) {
             const real *yv = p.y_row(v);
             const real *hv = p.h_row(v);
+            unsigned keep = 0;                                // CENSOR: bit r set when sample i0 + r is kept
+            if constexpr (CENSOR) {
+                const unsigned char *cm = cz.row(p.voxel_of(v));
 #pragma unroll
-            for (int r = 0; r < R; ++r) {
-                const int i = i0 + r;
-                const real cur = i < T ? yv[i] : real(0);
-                const real prv = (i > 0 && i - 1 < T) ? yv[i - 1] : real(0);
-                dy[r] = i < T ? cur - prv : real(0);
-                w[r] = (p.w0 && i < T) ? p.w0[v * T + i] : real(0);
+                for (int r = 0; r < R; ++r) {
+                    const int i = i0 + r;
+                    const bool kept = i < T && cm[i] == 0;
+                    const real cur = kept ? yv[i] : real(0);
+                    const real prv = (i > 0 && i - 1 < T && cm[i - 1] == 0) ? yv[i - 1] : real(0);
+                    dy[r] = i < T ? cur - prv : real(0);
+                    w[r] = (p.w0 && i < T) ? p.w0[v * T + i] : real(0);
+                    keep |= (unsigned)kept << r;
+                }
+            } else {
+#pragma unroll
+                for (int r = 0; r < R; ++r) {
+                    const int i = i0 + r;
+                    const real cur = i < T ? yv[i] : real(0);
+                    const real prv = (i > 0 && i - 1 < T) ? yv[i - 1] : real(0);
+                    dy[r] = i < T ? cur - prv : real(0);
+                    w[r] = (p.w0 && i < T) ? p.w0[v * T + i] : real(0);
+                }
             }
+            // res <- M res
+            auto censor_res = [&](real (&res)[R]) {
+#pragma unroll
+                for (int r = 0; r < R; ++r) res[r] = (keep >> r) & 1u ? res[r] : real(0);
+            };
+            // ||M res||^2, res itself unchanged (the final residual gives x)
+            auto sumsq_kept = [&](const real (&res)[R]) {
+                real rm[R];
+#pragma unroll
+                for (int r = 0; r < R; ++r) rm[r] = res[r];
+                censor_res(rm);
+                return sumsq(rm);
+            };
 #pragma unroll
             for (int j = 0; j < KMAX; ++j) h[j] = j < K ? hv[j] : real(0);
             const double Lc = p.L_of(v);
             NoiseLoop nl;
             if (AUTO) nl.start(win);
+            double n_kept = (double)T, zero = 0.0;
+            if (AUTO && CENSOR) {
+                n_kept = (double)__popc(keep);
+                ct.cta_sum2(n_kept, zero);
+            }
             double lam = AUTO ? nl.lbda : p.lam_of(v);
             const real step = (real)(1.0 / Lc);
             real th = (real)(lam / Lc);
@@ -712,6 +749,7 @@ fast_deconvc_kernel(DeconvArgs<real> p, int ring_rows) {
                 ring_pos = 0;
                 for (int k = 0; k < p.nb_iter; ++k) {
                     forward(res);
+                    if constexpr (CENSOR) censor_res(res);
                     // cost of the previous iterate: its residual has just been formed; the warp sums ride on B3
                     if (trace && k > 0) ct.publish2(sumsq(res), sumabs(w));
                     real g[R];
@@ -765,10 +803,10 @@ fast_deconvc_kernel(DeconvArgs<real> p, int ring_rows) {
                     if (es) ring_pos = ring_pos + 1 == nring ? 0 : ring_pos + 1;
                 }
                 forward(res);
-                double rr = sumsq(res), gg = sumabs(w);
+                double rr = CENSOR ? sumsq_kept(res) : sumsq(res), gg = sumabs(w);
                 ct.cta_sum2(rr, gg);
                 if (AUTO) {
-                    if (!nl.pass_done(p, v, rr, gg, tid == 0, tid, L::NT)) {
+                    if (!nl.pass_done<CENSOR>(p, v, rr, gg, tid == 0, tid, L::NT, n_kept)) {
                         lam = nl.lbda;
                         th = (real)(lam / Lc);
                         continue;
@@ -788,7 +826,10 @@ fast_deconvc_kernel(DeconvArgs<real> p, int ring_rows) {
             for (int r = 0; r < R; ++r) {
                 const int i = i0 + r;
                 if (i < T) {
-                    p.out_x[v * T + i] = res[r] + yv[i];      // x = (A w - y) + y
+                    if constexpr (CENSOR)                     // x = A w - y0 + y0, y0 = y zeroed on censored scans
+                        p.out_x[v * T + i] = res[r] + ((keep >> r) & 1u ? yv[i] : real(0));
+                    else
+                        p.out_x[v * T + i] = res[r] + yv[i];  // x = (A w - y) + y
                     p.out_z[v * T + i] = z[r];
                     p.out_dz[v * T + i] = w[r];
                 }
@@ -833,13 +874,25 @@ int fast_bdc_wave(int nb_iter) {
 }
 
 // FAST_NO_MATCH when the early-stopping ring does not fit: the generic kernel decides
-template <typename real, int R, int KMAX, int NW, int MINB, bool AUTO = false>
-int fast_deconvc_launch(const DeconvArgs<real> &a, cudaStream_t stream) {
+template <typename real, int R, int KMAX, int NW, int MINB, bool AUTO = false, bool CENSOR = false>
+int fast_deconvc_launch_c(const DeconvArgs<real> &a, const Censor &cz, cudaStream_t stream) {
     using L = CtaLayout<real, R, KMAX, NW>;
     const int ring_rows = a.early_stopping && a.wind >= 2 ? a.wind - 1 : 0;
-    return launch_persistent(fast_deconvc_kernel<real, R, KMAX, NW, MINB, AUTO>, NW * 32,
+    return launch_persistent(fast_deconvc_kernel<real, R, KMAX, NW, MINB, AUTO, CENSOR>, NW * 32,
                              L::deconv_bytes(a.nb_iter, ring_rows, AUTO ? a.wind : 0), 1, a.V, a.queue, stream, a,
-                             ring_rows);
+                             ring_rows, cz);
+}
+
+template <typename real, int R, int KMAX, int NW, int MINB, bool AUTO = false>
+int fast_deconvc_launch(const DeconvArgs<real> &a, cudaStream_t stream) {
+    return fast_deconvc_launch_c<real, R, KMAX, NW, MINB, AUTO>(a, Censor{}, stream);
+}
+
+// censored calls run on the CTA rows only; below T = 181 no row of at most 32 taps serves a series, and the many-tap
+// rows take K <= 28 there too, with zero-padded taps (pb_fast_registry.cu: pick_censored)
+template <int R, int KMAX, int NW>
+bool fastc_censored_ok(int T, int K) {
+    return fastc_shape_ok<R, KMAX, NW>(T, K) || (KMAX > 32 && K <= 28 && T <= 180 && fastc_shape_ok<R, KMAX, NW>(T, 29));
 }
 
 template <typename real, int R, int KMAX, int NW, int MINB>
@@ -847,7 +900,9 @@ constexpr Variant<real> cta_variant() {
     return {TIER_GROUP_CTA, 32 * NW, R, KMAX, 0, false, fastc_shape_ok<R, KMAX, NW>,
             fast_bdc_launch<real, R, KMAX, NW, MINB>, fast_bdc_launch<real, R, KMAX, NW, MINB, true>,
             fast_deconvc_launch<real, R, KMAX, NW, MINB>,
-            fast_bdc_wave<real, R, KMAX, NW, MINB>, fast_deconvc_launch<real, R, KMAX, NW, MINB, true>};
+            fast_bdc_wave<real, R, KMAX, NW, MINB>, fast_deconvc_launch<real, R, KMAX, NW, MINB, true>,
+            fastc_censored_ok<R, KMAX, NW>, fast_deconvc_launch_c<real, R, KMAX, NW, MINB, false, true>,
+            fast_deconvc_launch_c<real, R, KMAX, NW, MINB, true, true>};
 }
 
 }  // namespace pb

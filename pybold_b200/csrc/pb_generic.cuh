@@ -253,10 +253,21 @@ struct DeconvArgs {
     }
 };
 
+// Scan censoring (pb_deconv_censored_*): m[voxel * stride + i] != 0 leaves scan i of the voxel out of the data term,
+// min 1/2 ||M (A w - y)||^2 + lbda ||w||_1 with M = diag(1 - censor).  y reads as 0 on censored scans (NaN there is
+// ignored); x = A w is still written on every scan.  Kernels take it as their last parameter and read it only in
+// their CENSOR instances.
+struct Censor {
+    const unsigned char *m = nullptr;
+    int64_t stride = 0;       // 0: one mask shared by the batch
+    __device__ __forceinline__ const unsigned char *row(int64_t voxel) const { return m + voxel * stride; }
+};
+
 // AUTO: deconv(lbda=None), one inner pass per outer iteration of the noise loop, then the final pass; the
-// window of alphas lives in the warp's scratch doubles
-template <typename real, bool AUTO = false>
-__global__ void generic_deconv_kernel(DeconvArgs<real> p, GenLayout lay) {
+// window of alphas lives in the warp's scratch doubles.  CENSOR: the residual is masked with cz before the adjoint
+// and the cost terms, and the noise target is n_kept sigma^2.
+template <typename real, bool AUTO = false, bool CENSOR = false>
+__global__ void generic_deconv_kernel(DeconvArgs<real> p, GenLayout lay, Censor cz) {
     extern __shared__ __align__(16) unsigned char smem[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = blockDim.x >> 5;
     real *beta = reinterpret_cast<real *>(smem);
@@ -273,10 +284,31 @@ __global__ void generic_deconv_kernel(DeconvArgs<real> p, GenLayout lay) {
         if (!p.is_active(v)) continue;
         const real *yv = p.y_row(v);
         const real *hv = p.h_row(v);
-        for (int i = lane; i < T; i += 32) {
-            g.ys[i] = yv[i];
-            g.ws[i] = p.w0 ? p.w0[v * T + i] : real(0);
+        const unsigned char *cm = CENSOR ? cz.row(p.voxel_of(v)) : nullptr;
+        double n_kept = (double)T;
+        if constexpr (CENSOR) {
+            int nk = 0;
+            for (int i = lane; i < T; i += 32) {
+                const bool kept = cm[i] == 0;
+                g.ys[i] = kept ? yv[i] : real(0);
+                g.ws[i] = p.w0 ? p.w0[v * T + i] : real(0);
+                nk += kept;
+            }
+            n_kept = warp_sum((double)nk);
+        } else {
+            for (int i = lane; i < T; i += 32) {
+                g.ys[i] = yv[i];
+                g.ws[i] = p.w0 ? p.w0[v * T + i] : real(0);
+            }
         }
+        // bs <- M bs (CENSOR), after forward() and before the adjoint and the cost sums
+        auto censor_res = [&]() {
+            if constexpr (CENSOR) {
+                for (int i = lane; i < T; i += 32)
+                    if (cm[i]) g.bs[i] = real(0);
+                __syncwarp();
+            }
+        };
         for (int a = lane; a < K; a += 32) g.hr[a] = hv[a];
         __syncwarp();
         const double Lc = p.L_of(v);
@@ -298,6 +330,7 @@ __global__ void generic_deconv_kernel(DeconvArgs<real> p, GenLayout lay) {
             n_done = 0;
             for (int k = 0; k < p.nb_iter; ++k) {
                 g.forward();
+                censor_res();
                 if (!AUTO && k > 0) {
                     const double J = 0.5 * g.sumsq(g.bs) + lam * g.sumabs(g.ws);
                     if (lane == 0 && p.out_J) Jv[k - 1] = (real)J;
@@ -329,14 +362,25 @@ __global__ void generic_deconv_kernel(DeconvArgs<real> p, GenLayout lay) {
                 }
             }
             g.forward();
+            // the final residual stays unmasked in bs: x = bs + ys = A w on every scan
+            auto res_sumsq = [&]() -> double {
+                if constexpr (CENSOR) {
+                    double q = 0.0;
+                    for (int i = lane; i < T; i += 32)
+                        if (!cm[i]) q += (double)g.bs[i] * (double)g.bs[i];
+                    return warp_sum(q);
+                } else {
+                    return g.sumsq(g.bs);
+                }
+            };
             if (AUTO) {
-                if (!nl.pass_done(p, v, g.sumsq(g.bs), g.sumabs(g.ws), lane == 0, lane, 32)) {
+                if (!nl.pass_done<CENSOR>(p, v, res_sumsq(), g.sumabs(g.ws), lane == 0, lane, 32, n_kept)) {
                     lam = nl.lbda;
                     th = (real)(lam / Lc);
                     continue;
                 }
             } else if (n_done > 0) {
-                const double rr = g.sumsq(g.bs), gg = g.sumabs(g.ws);
+                const double rr = res_sumsq(), gg = g.sumabs(g.ws);
                 const double J = 0.5 * rr + lam * gg;
                 if (lane == 0) {
                     if (p.out_J) Jv[n_done - 1] = (real)J;

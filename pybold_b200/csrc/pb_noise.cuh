@@ -13,8 +13,10 @@
 // `except ValueError` branch then takes `wavedec(level=0)`, i.e. the series itself.
 #pragma once
 #include <cstdint>
+#include <math_constants.h>
 
 #include "pb_device.cuh"
+#include "pb_generic.cuh"
 
 namespace pb {
 
@@ -92,6 +94,59 @@ __global__ void mad_rows_kernel(const real *x, double c, real *out, int64_t V, i
         for (int i = lane; i < n; i += 32) d[i] = fabs(d[i] - med);
         __syncwarp();
         const double dev = warp_median(d, n, lane);
+        if (lane == 0) out[v] = (real)(dev / c);
+        __syncwarp();
+    }
+}
+
+// pb_mad_daub_noise_est_censored: the db3 MAD over the level-1 detail coefficients that touch no censored scan (a
+// coefficient reads six samples, after the symmetric extension; T < 10 takes the kept samples themselves).  The left-out
+// coefficients are parked at +inf, above every kept one, so both medians are order statistics among the first n_kept.
+// A voxel with no coefficient left gets NaN.
+template <typename real>
+__global__ void mad_daub_censored_kernel(const real *x, double c, real *out, int64_t V, int T, int nmax, Censor cz) {
+    extern __shared__ __align__(16) unsigned char smem[];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = blockDim.x >> 5;
+    double *d = reinterpret_cast<double *>(smem) + (size_t)warp * nmax;
+    const int n = noise_detail_len(T);
+    auto median_of_kept = [&](int nk) {
+        const double lo = warp_select(d, n, (nk - 1) / 2, lane);
+        return (nk & 1) ? lo : 0.5 * (lo + warp_select(d, n, nk / 2, lane));
+    };
+    for (int64_t v = (int64_t)blockIdx.x * nwarp + warp; v < V; v += (int64_t)gridDim.x * nwarp) {
+        const real *row = x + v * T;
+        const unsigned char *cm = cz.row(v);
+        int nk = 0;
+        for (int o = lane; o < n; o += 32) {
+            double acc = 0.0;
+            bool kept = true;
+            if (T >= 10) {
+#pragma unroll
+                for (int j = 0; j < 6; ++j) {
+                    int i = 2 * o + 1 - j;
+                    i = i < 0 ? -i - 1 : (i >= T ? 2 * T - 1 - i : i);
+                    kept = kept && cm[i] == 0;
+                    acc += kDb3DecHi[j] * (double)row[i];
+                }
+            } else {
+                kept = cm[o] == 0;
+                acc = (double)row[o];
+            }
+            d[o] = kept ? acc : CUDART_INF;
+            nk += kept;
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) nk += __shfl_xor_sync(PB_FULL, nk, o);
+        __syncwarp();
+        if (nk == 0) {
+            if (lane == 0) out[v] = (real)CUDART_NAN;
+            continue;
+        }
+        const double med = median_of_kept(nk);
+        __syncwarp();
+        for (int i = lane; i < n; i += 32) d[i] = d[i] == CUDART_INF ? d[i] : fabs(d[i] - med);
+        __syncwarp();
+        const double dev = median_of_kept(nk);
         if (lane == 0) out[v] = (real)(dev / c);
         __syncwarp();
     }

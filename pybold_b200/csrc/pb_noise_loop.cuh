@@ -4,7 +4,7 @@
 //   alpha = 1, lbda = 1 / (2 alpha), w = 0
 //   for i < nb_outer:   inner pass with lbda (momentum from beta_0, empty Q5 window, w warm in registers)
 //                       r = ||A w - y||^2, g = ||w||_1
-//                       alpha += 1e-4 (r - T sigma^2), lbda = 1 / (2 alpha)
+//                       alpha += 1e-4 (r - T sigma^2), lbda = 1 / (2 alpha)   (censored: n_kept, not T)
 //                       J[i] = 0.5 r + lbda g, R[i] = r, G[i] = g
 //                       early stop: i > wind, |mean(new) - mean(old)| / |mean(new)| < tol over the last
 //                       wind alphas (old: the first wind - wind/2, new: the last wind/2)
@@ -42,9 +42,10 @@ struct NoiseLoop {
     // An inner pass with `lbda` has ended with r = ||A w - y||^2, g = ||w||_1.  Returns true when it was the
     // final pass (the caller stores x, z, diff_z), else the next pass runs with the updated `lbda`.
     // `writer`: the one lane that stores the scalars; lane q of the nq lanes of the voxel fills the row tails.
-    template <typename real>
+    // KEPT (scan censoring): n_kept scans in the data term, r = ||M (A w - y)||^2 is steered toward n_kept sigma^2.
+    template <bool KEPT = false, typename real>
     __device__ __forceinline__ bool pass_done(const DeconvArgs<real> &p, int64_t v, double r, double g,
-                                              bool writer, int q, int nq) {
+                                              bool writer, int q, int nq, double n_kept = 0.0) {
         const int64_t row = v * (int64_t)p.nb_outer;
         if (last) {
             // complete rows for a C caller: NaN past the voxel's outer count
@@ -59,7 +60,10 @@ struct NoiseLoop {
             return true;
         }
         const double s = (double)p.sigma[p.voxel_of(v) * p.sigma_stride];
-        alpha += 1.0e-4 * (r - (double)p.T * (s * s));     // bold_signal.py:139-145
+        if constexpr (KEPT)
+            alpha += 1.0e-4 * (r - n_kept * (s * s));
+        else
+            alpha += 1.0e-4 * (r - (double)p.T * (s * s));     // bold_signal.py:139-145
         lbda = 1.0 / (2.0 * alpha);
         if (writer) {
             if (p.out_J) p.out_J[row + i] = (real)(0.5 * r + lbda * g);

@@ -221,11 +221,12 @@ __global__ void spm_hrf_ex_kernel(const real *theta, HrfGrid grid, HrfShape sh, 
     }
 }
 
-// spectral_radius_est (pybold/utils.py:94-109) with the start vector supplied.
-template <typename real>
+// spectral_radius_est (pybold/utils.py:94-109) with the start vector supplied.  CENSOR: the power iteration of the
+// censored operator A^T M A (M applied between op and adj), the mask of voxel v at cz.row(v).
+template <typename real, bool CENSOR = false>
 __global__ void lipschitz_power_kernel(const real *h, int64_t h_stride, const real *x0,
                                        int64_t x0_stride, int nb_iter, double tol, real *out_L,
-                                       int64_t V, int T, int K, GenLayout lay) {
+                                       int64_t V, int T, int K, GenLayout lay, Censor cz) {
     extern __shared__ __align__(16) unsigned char smem[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = blockDim.x >> 5;
     double *scratch;
@@ -242,6 +243,12 @@ __global__ void lipschitz_power_kernel(const real *h, int64_t h_stride, const re
             __syncwarp();
             g.scan_fwd(g.as);
             g.conv(g.as, nullptr, g.bs);
+            if constexpr (CENSOR) {
+                const unsigned char *cm = cz.row(v);
+                for (int i = lane; i < T; i += 32)
+                    if (cm[i]) g.bs[i] = real(0);
+                __syncwarp();
+            }
             g.adjoint();
             const real inv = (real)(1.0 / n_old);
             for (int i = lane; i < T; i += 32) g.as[i] *= inv;

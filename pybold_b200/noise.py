@@ -64,13 +64,14 @@ def mad_daub_noise_est(x, c=0.6744):
 
 
 def deconv_auto_lbda(y_in, yb, one_d, hrf, lipschitz, sigma, early_stopping, tol, wind,
-                     nb_iter, nb_sub_iter):
+                     nb_iter, nb_sub_iter, censor=None):
     """``deconv(lbda=None)`` (pybold/bold_signal.py:99-214) for a batch: the noise level (given, or estimated
     like the reference does), then the whole noise-constrained loop of every voxel in ONE persistent kernel
     launch (:func:`~pybold_b200.bold_signal.deconv_auto_batch`): outer iterations, alpha / lambda updates, the
     alpha-window stop and the final inner pass all run on the device, nothing goes through the host between
     outer iterations.  Returns the reference's tuple (x, z, diff_z, J, R, G): lists for one voxel, rows cut at
-    the largest outer count (NaN past each voxel's own) for a batch.
+    the largest outer count (NaN past each voxel's own) for a batch.  ``censor``: a uint8 device mask from
+    :func:`~pybold_b200.censor.censor_mask`; sigma then comes from the detail coefficients that touch no censored scan.
     """
     from .bold_signal import deconv_auto_batch
     if sigma is None:
@@ -83,8 +84,13 @@ def deconv_auto_lbda(y_in, yb, one_d, hrf, lipschitz, sigma, early_stopping, tol
                           "boundary convention is pinned on PyWavelets' documented examples only; pass sigma= for "
                           "a run that does not depend on it", UserWarning, stacklevel=3)
             _warned_sigma = True
-        sigma = mad_daub_noise_est(yb)
-    out = deconv_auto_batch(yb, hrf, sigma, lipschitz, nb_iter, nb_sub_iter, early_stopping, tol, wind)
+        if censor is None:
+            sigma = mad_daub_noise_est(yb)
+        else:
+            from .censor import mad_daub_noise_est_censored
+            sigma = mad_daub_noise_est_censored(yb, censor, 0 if censor.dim() == 1 else yb.shape[1])
+    out = deconv_auto_batch(yb, hrf, sigma, lipschitz, nb_iter, nb_sub_iter, early_stopping, tol, wind,
+                            censor=censor)
     x, z, w, J, R, G = (out[k] for k in ("x", "z", "diff_z", "J", "R", "G"))
     if one_d:
         n = int(out["n_outer"][0])

@@ -199,7 +199,10 @@ int pb_deconv_masked_f64(const double *y, const double *h, int64_t h_stride, con
  *   out_J, out_R, out_G     [V, nb_iter]: 0.5 R + lbda G (with the updated lbda), ||x - y||^2, ||diff_z||_1 of every
  *                           outer iteration, NaN past the voxel's outer count
  *   out_lbda [V]            the lambda of the final pass;  out_nouter [V]  outer iterations done
- * out_J, out_R, out_G, out_lbda and out_nouter may be NULL (not written). */
+ * out_J, out_R, out_G, out_lbda and out_nouter may be NULL (not written).
+ * A voxel whose sigma is NaN gets the reference's result: out_x, out_z, out_dz, out_J and out_lbda NaN, out_R and
+ * out_G NaN from the second outer iteration on, out_nouter = nb_iter.  Other voxels are not affected.  The censored
+ * entry points below do the same. */
 int pb_deconv_auto_f32(const float *y, const float *h, int64_t h_stride, const float *L, int64_t L_stride,
                        const float *sigma, int64_t sigma_stride, int nb_iter, int nb_sub_iter, int early_stopping,
                        int wind, double tol, float *out_x, float *out_z, float *out_dz, float *out_J, float *out_R,
@@ -296,7 +299,8 @@ int pb_lipschitz_power_censored_f64(const double *h, int64_t h_stride, const dou
                                     const unsigned char *censor, int64_t censor_stride, int nb_iter, double tol,
                                     double *out_L, int64_t V, int T, int K, pb_stream_t stream);
 /* pb_mad_daub_noise_est over the level-1 db3 detail coefficients that touch no censored scan (a coefficient reads
- * six samples, after the symmetric extension; T < 10: the kept samples).  NaN for a voxel with none left. */
+ * six samples, after the symmetric extension; T < 10: the kept samples).  NaN for a voxel with none left, and, as for
+ * pb_mad_daub_noise_est, for one with a NaN or an infinite median among its kept coefficients. */
 int pb_mad_daub_noise_est_censored_f32(const float *y, const unsigned char *censor, int64_t censor_stride, double c,
                                        float *out_sigma, int64_t V, int T, pb_stream_t stream);
 int pb_mad_daub_noise_est_censored_f64(const double *y, const unsigned char *censor, int64_t censor_stride,
@@ -352,7 +356,8 @@ int pb_rel_l2_err_f64(const double *est, const double *ref, int64_t ref_stride, 
  * x[V, n] (`mad`, utils.py:10-13).  pb_mad_daub_noise_est: the same statistic of the level-1 db3
  * detail coefficients of y[V, T] (PyWavelets "symmetric" extension, floor((T + 5) / 2)
  * coefficients; T < 10 has no level-1 decomposition and takes the series itself, the reference's
- * `except ValueError` branch, utils.py:23-24).  Medians are exact order statistics. */
+ * `except ValueError` branch, utils.py:23-24).  Medians are exact order statistics.  A row holding a NaN gives NaN,
+ * like NumPy's median, and so does a row whose median is +-inf (its deviation there is inf - inf). */
 int pb_mad_f32(const float *x, double c, float *out, int64_t V, int n, pb_stream_t stream);
 int pb_mad_f64(const double *x, double c, double *out, int64_t V, int n, pb_stream_t stream);
 int pb_mad_daub_noise_est_f32(const float *y, double c, float *out_sigma, int64_t V, int T,

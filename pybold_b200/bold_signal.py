@@ -122,6 +122,10 @@ def deconv_auto_batch(y, hrf, sigma, lipschitz, nb_iter=1000, nb_sub_iter=1000, 
     ``censor`` (``[T]`` or ``[V, T]``, :mod:`pybold_b200.censor`): R is ``||M (x - y)||^2`` and the noise target
     ``n_kept sigma^2``; a device mask keeps the call free of host synchronisation (it is then not checked for
     all-censored voxels).
+
+    A voxel whose sigma is NaN (the estimate is NaN when a NaN is among the kept scans, like NumPy's median) gets the
+    reference's result: x, z, diff_z, J and lbda NaN, R and G NaN after the first outer iteration, and all
+    ``nb_iter`` outer iterations.  The other voxels are not affected.
     """
     V, T = y.shape
     dtype, dev = y.dtype, y.device

@@ -71,14 +71,19 @@ def lipschitz_censored(h, x0, cm, c_stride, dtype, T):
 
 def mad_daub_noise_est_censored(yb, cm, c_stride, c=0.6744):
     """db3 MAD noise level of every row of ``yb`` ``[V, T]`` over the level-1 detail coefficients that touch no
-    censored scan.  Raises ``ValueError`` when a voxel has no such coefficient: pass ``sigma=`` then."""
+    censored scan.  Raises ``ValueError`` when a voxel has no such coefficient: pass ``sigma=`` then.  A voxel with a
+    NaN or an Inf among its kept scans may get a NaN sigma, like NumPy's median gives; that is not an error, and such
+    a voxel gets NaN without the error even when it has no clean coefficient either (its fit is NaN whatever sigma
+    is)."""
     V, T = yb.shape
     out = torch.empty(V, dtype=yb.dtype, device=yb.device)
     with torch.cuda.device(yb.device):
         rc = _lib.fn("pb_mad_daub_noise_est_censored", yb.dtype)(ptr(yb), ptr(cm), c_stride, float(c), ptr(out), V, T,
                                                                   stream_ptr())
     _lib.check(rc, "pb_mad_daub_noise_est_censored")
-    if bool(torch.isnan(out).any()):
+    # with finite kept scans every kept coefficient is finite: a NaN sigma then means that none was left
+    finite_kept = (torch.isfinite(yb) | (cm != 0)).all(dim=1)
+    if bool((torch.isnan(out) & finite_kept).any()):
         raise ValueError("censor leaves no db3 detail coefficient free of censored scans in some voxel, so the "
                          "noise level cannot be estimated: pass sigma=")
     return out

@@ -439,7 +439,7 @@ int run_deconv(pb::DeconvArgs<real> a, pb_stream_t stream, const pb::Censor *cz 
 }
 
 // deconv(lbda=None): the noise loop runs inside the kernel, nb_outer outer iterations at most, nb_iter inner
-// ones per pass
+// ones per pass; then the voxels with a NaN sigma get the reference's NaN outputs (pb_noise.cuh)
 template <typename real>
 int run_deconv_auto(pb::DeconvArgs<real> a, pb_stream_t stream, const pb::Censor *cz = nullptr) {
     if (a.V == 0) return PB_OK;
@@ -450,7 +450,13 @@ int run_deconv_auto(pb::DeconvArgs<real> a, pb_stream_t stream, const pb::Censor
         return PB_ERR_INVALID_ARG;
     if (a.T > PB_MAX_T || a.K > PB_MAX_K || a.nb_iter > PB_MAX_ITER) return PB_ERR_UNSUPPORTED;
     set_routing(a, queue_slot);
-    return launch_deconv(a, stream, nullptr, nullptr, cz);
+    const int rc = launch_deconv(a, stream, nullptr, nullptr, cz);
+    if (rc) return rc;
+    DeviceInfo d = device_info();
+    if (d.err) return d.err;
+    const int64_t cap = (int64_t)d.sm_count * 8;
+    pb::nan_sigma_rows_kernel<real><<<(int)(a.V < cap ? a.V : cap), 128, 0, (cudaStream_t)stream>>>(a);
+    return last_error();
 }
 
 // pb_deconv_variant / pb_deconv_censored_variant: the routing of a deconv call with V = 0 (nothing is launched)

@@ -57,6 +57,14 @@ __device__ inline double warp_select(const double *d, int n, int k, int lane) {
     return key_value(prefix);
 }
 
+// NumPy's median of a row holding a NaN is NaN, whatever the NaN's sign bit; ordered_key would rank it past +-inf
+// instead, so the kernels test for one before they select
+__device__ inline bool warp_any_nan(const double *d, int n, int lane) {
+    bool nan = false;
+    for (int i = lane; i < n; i += 32) nan = nan || isnan(d[i]);
+    return __any_sync(PB_FULL, nan);
+}
+
 // NumPy's median: the middle order statistic, or the mean of the two middle ones
 __device__ inline double warp_median(const double *d, int n, int lane) {
     const double lo = warp_select(d, n, (n - 1) / 2, lane);
@@ -66,6 +74,9 @@ __device__ inline double warp_median(const double *d, int n, int lane) {
 }
 
 // MODE 0: mad of the rows of x[V, n].  MODE 1: mad of the db3 detail coefficients of y[V, T].
+// Non-finite values: a row holding a NaN gives NaN.  So does a row whose median is +-inf: that median is one of the
+// row's values, and its deviation inf - inf is NaN in NumPy too.  Otherwise every deviation is finite or +inf and
+// both selections are exact.
 template <typename real, int MODE>
 __global__ void mad_rows_kernel(const real *x, double c, real *out, int64_t V, int T, int nmax) {
     extern __shared__ __align__(16) unsigned char smem[];
@@ -89,8 +100,12 @@ __global__ void mad_rows_kernel(const real *x, double c, real *out, int64_t V, i
             for (int i = lane; i < n; i += 32) d[i] = (double)row[i];
         }
         __syncwarp();
-        const double med = warp_median(d, n, lane);
+        const double med = warp_any_nan(d, n, lane) ? CUDART_NAN : warp_median(d, n, lane);
         __syncwarp();
+        if (!isfinite(med)) {
+            if (lane == 0) out[v] = (real)CUDART_NAN;
+            continue;
+        }
         for (int i = lane; i < n; i += 32) d[i] = fabs(d[i] - med);
         __syncwarp();
         const double dev = warp_median(d, n, lane);
@@ -102,7 +117,8 @@ __global__ void mad_rows_kernel(const real *x, double c, real *out, int64_t V, i
 // pb_mad_daub_noise_est_censored: the db3 MAD over the level-1 detail coefficients that touch no censored scan (a
 // coefficient reads six samples, after the symmetric extension; T < 10 takes the kept samples themselves).  The left-out
 // coefficients are parked at +inf, above every kept one, so both medians are order statistics among the first n_kept.
-// A voxel with no coefficient left gets NaN.
+// A voxel with no coefficient left gets NaN, and so does one with a NaN or an infinite median among its kept
+// coefficients (as in mad_rows_kernel); a NaN at a censored scan reaches left-out coefficients only.
 template <typename real>
 __global__ void mad_daub_censored_kernel(const real *x, double c, real *out, int64_t V, int T, int nmax, Censor cz) {
     extern __shared__ __align__(16) unsigned char smem[];
@@ -138,17 +154,41 @@ __global__ void mad_daub_censored_kernel(const real *x, double c, real *out, int
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) nk += __shfl_xor_sync(PB_FULL, nk, o);
         __syncwarp();
-        if (nk == 0) {
+        const double med = nk == 0 || warp_any_nan(d, n, lane) ? CUDART_NAN : median_of_kept(nk);
+        __syncwarp();
+        if (!isfinite(med)) {
             if (lane == 0) out[v] = (real)CUDART_NAN;
             continue;
         }
-        const double med = median_of_kept(nk);
-        __syncwarp();
+        // a finite median: a kept +inf and a parked coefficient both deviate by +inf
         for (int i = lane; i < n; i += 32) d[i] = d[i] == CUDART_INF ? d[i] : fabs(d[i] - med);
         __syncwarp();
         const double dev = median_of_kept(nk);
         if (lane == 0) out[v] = (real)(dev / c);
         __syncwarp();
+    }
+}
+
+// deconv(lbda=None) for a voxel whose noise level is NaN (a NaN among its kept samples, or a NaN sigma from the
+// caller).  In the reference alpha and lambda turn NaN after the first pass, and its soft threshold then makes every
+// later iterate NaN; the kernels' clamp fmin(fmax(u, -th), th) passes u through on a NaN th and would leave a finite,
+// meaningless fit.  Launched after the solve on the same stream, this gives such a voxel the reference's outputs:
+// x, z, diff_z NaN, and R, G NaN from the second outer iteration on.  J and lambda are NaN already, and the outer
+// count is nb_outer, because the window test never passes on a NaN alpha.  Other voxels are not touched.
+template <typename real>
+__global__ void nan_sigma_rows_kernel(DeconvArgs<real> a) {
+    const real nan = (real)CUDART_NAN;
+    for (int64_t v = blockIdx.x; v < a.V; v += gridDim.x) {
+        if (!isnan((double)a.sigma[a.voxel_of(v) * a.sigma_stride])) continue;
+        for (int t = threadIdx.x; t < a.T; t += blockDim.x) {
+            a.out_x[v * a.T + t] = nan;
+            a.out_z[v * a.T + t] = nan;
+            a.out_dz[v * a.T + t] = nan;
+        }
+        for (int j = 1 + threadIdx.x; j < a.nb_outer; j += blockDim.x) {
+            if (a.out_R) a.out_R[v * a.nb_outer + j] = nan;
+            if (a.out_G) a.out_G[v * a.nb_outer + j] = nan;
+        }
     }
 }
 
